@@ -9,18 +9,22 @@ Weak scaling: every GPU processes its own batch.
   python bench.py [--gpus N] [--steps K] [--warmup W]               # our arm (torchrun for N > 1)
   python bench.py --impl reference [--steps K] [--warmup W]         # CPU reference arm (oracle port, host threads)
   python bench.py --config {c1,c2,c3,c4,c5} ...                     # the other BASELINE configs, same JSON schema
+  python bench.py --dump-outputs DIR ...                            # also write the last timed step's results to DIR
 
 --config: c2 (default) conformer streaming b32x10s greedy; c1 deepspeech2 non-streaming 1x5s greedy (CPU arm: one core);
 c3 conformer non-streaming b64x30s ctc_beam_search beam 10; c4 squeezeformer streaming b32x10s per GPU greedy; c5
 efficient_conformer streaming chunk 16, b64x5s per GPU, ctc_beam_search beam 20 + 4-gram LM.
 
-Timing: W >= 3 warm-up steps; the timed region is R repetitions of exactly K steps, each repetition bracketed by CUDA events on
-the launching streams (barrier + synchronize on both sides, max over ranks); R is chosen so that the repetitions cover >= 1 s.
-`ms_per_step` / `value` are the MEDIAN repetition; p10 / p90 are reported beside it.
+Timing: W >= 3 warm-up steps; the timed region is exactly K steps, bracketed by CUDA events on the launching streams (barrier +
+synchronize on both sides, max over ranks). `ms_per_step` / `value` are its mean; pick K so that the region lasts about a
+second or more. The single-stream, CUDA-graph, e2e and kernel-profile figures beside it also time K steps each.
+
+--dump-outputs DIR: after the timed steps, the results of the last one as a caller of the timed path receives them (decoded
+ids, their lengths and scores; with N > 1 the gathered results of all ranks) go to DIR/<name>.npy as float64. Weights and
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
-import math
 import os
 import statistics
 import sys
@@ -215,6 +219,16 @@ class ClockSampler(threading.Thread):
                 "reasons": sorted(self.reasons), "samples": len(self.samples)}
 
 
+def dump_outputs(path, ids, out_lens, scores):
+    """path/{ids,out_lens,scores}.npy in float64 (exact for the int32 ids and lengths). Only the first out_lens[b] ids of an
+    utterance are defined; the rest of its row is written as -1 so that dumps of two builds compare element for element."""
+    ids, out_lens, scores = (t.cpu().numpy() if hasattr(t, "cpu") else np.asarray(t) for t in (ids, out_lens, scores))
+    ids = np.where(np.arange(ids.shape[1])[None, :] < out_lens[:, None], ids, -1)
+    os.makedirs(path, exist_ok=True)
+    for name, a in (("ids", ids), ("out_lens", out_lens), ("scores", scores)):
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def quantiles(xs):
     xs = sorted(xs)
     n = len(xs)
@@ -308,15 +322,7 @@ def run_reference(args, conf):
     threads, probe = ref.choose_threads(feats, lens)
     W = max(1, args.warmup)
     K = max(1, args.steps)
-    # keep the whole run within a few minutes: one step of the full C2 batch is ~1.5-3 s on 16 cores
-    t0 = time.perf_counter()
-    ref.step(feats, lens)
-    one = time.perf_counter() - t0
-    budget_s = 240.0
-    if one * (W + K) > budget_s:
-        K = max(1, int(budget_s / one) - min(W, 2))
-        W = min(W, 2)
-    for _ in range(max(0, W - 1)):
+    for _ in range(W):
         ref.step(feats, lens)
     times = []
     for _ in range(K):
@@ -431,7 +437,11 @@ def main():
     ap.add_argument("--config", default=None, choices=sorted(CONFIGS),
                     help="BASELINE config to run (default c2 = configs[1], the config the headline metric is quoted on)")
     ap.add_argument("--model", default=None, choices=["conformer", "squeezeformer"], help="deprecated alias: squeezeformer = --config c4")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step (ids, lens, scores) to DIR/<name>.npy as float64")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU path's results; the reference arm has none")
     cname = args.config or ("c4" if args.model == "squeezeformer" else "c2")
     conf = CONFIGS[cname]
     if args.impl == "reference":
@@ -479,16 +489,15 @@ def main():
     for _ in range(W):
         step()
     torch.cuda.synchronize()
-    ks = max(5, min(K, 20))
-    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(ks)]
-    for k in range(ks):
+    ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
+    for k in range(K):
         flush.zero_()  # L2 flush between timed iterations (not inside the timed events)
         ev[k][0].record()
         step()
         ev[k][1].record()
     torch.cuda.synchronize()
     single = [a.elapsed_time(b) for a, b in ev]
-    single_ms = sum(single) / ks
+    single_ms = sum(single) / K
 
     # ---- (a') the same single-batch step captured once as a CUDA graph and replayed (one graph launch per step) ----
     graph_info = None
@@ -513,16 +522,16 @@ def main():
                 eng.graph_launch(gs)
             gs.synchronize()
             same = bool(torch.equal(gi, want[0]) and torch.equal(gl, want[1]))
-            gev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(ks)]
+            gev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
             with torch.cuda.stream(gs):
-                for k in range(ks):
+                for k in range(K):
                     flush.zero_()
                     gev[k][0].record(gs)
                     eng.graph_launch(gs)
                     gev[k][1].record(gs)
             gs.synchronize()
             gms = [a.elapsed_time(b) for a, b in gev]
-            graph_info = {"ms_per_step": sum(gms) / ks, "quantiles": quantiles(gms), "kernels_per_replay": nk,
+            graph_info = {"ms_per_step": sum(gms) / K, "quantiles": quantiles(gms), "kernels_per_replay": nk,
                           "replay_matches_direct_run": same}
         except Exception as e:  # a driver / runtime without capture support for some launch attribute: report, do not fail
             graph_info = {"error": str(e)[:300]}
@@ -551,20 +560,25 @@ def main():
 
     def finish(ticket):
         if world > 1:
-            gather_slot(ticket)
+            return gather_slot(ticket)
+        return pipe.device_result(ticket)
 
     def run_steps(n):
+        """Runs n steps and returns what the last one gives its caller: (ids, out_lens, scores) device tensors, or the
+        gathered records of all ranks when the pipeline runs with N > 1."""
+        last = None
         if pipe is None:
             for i in range(n):
-                gather(wl.step_device(pool[i % len(pool)]))
-            return
+                last = gather(wl.step_device(pool[i % len(pool)]))
+            return last
         pending = []
         for i in range(n):
             pending.append(pipe.submit(pool[i % len(pool)], to_host=False))
             if len(pending) == depth:
-                finish(pending.pop(0))
+                last = finish(pending.pop(0))
         while pending:
-            finish(pending.pop(0))
+            last = finish(pending.pop(0))
+        return last
 
     def timed_rep(n):
         e0 = torch.cuda.Event(enable_timing=True)
@@ -576,7 +590,7 @@ def main():
         if pipe is not None:
             for sl in pipe.slots:
                 sl["stream"].wait_event(e0)
-        run_steps(n)
+        last = run_steps(n)
         if pipe is not None:
             for sl in pipe.slots:
                 torch.cuda.current_stream().wait_stream(sl["stream"])
@@ -585,25 +599,22 @@ def main():
         t = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)  # max over ranks
-        return float(t.item())
+        return float(t.item()), last
 
     run_steps(max(W, 4))
     torch.cuda.synchronize()
-    probe_ms = timed_rep(K)
-    reps = int(min(200, max(5, math.ceil(1000.0 / max(probe_ms, 1e-3)))))  # >= 1 s of timed region in total
-    if world > 1:
-        rt = torch.tensor([reps], device=dev)
-        dist.broadcast(rt, 0)
-        reps = int(rt.item())
     sampler = ClockSampler(local_rank)
     sampler.start()
     launches0 = lib.ppasr_b200_launch_count()
-    rep_ms = [timed_rep(K) for _ in range(reps)]
+    timed_ms, last = timed_rep(K)
     launches1 = lib.ppasr_b200_launch_count()
     sampler.stop_flag = True
-    ms = statistics.median(rep_ms) / K
+    ms = timed_ms / K
     value = total_utts / (ms * 1e-3)
-    q_ms = quantiles([r / K for r in rep_ms])
+    if args.dump_outputs and rank == 0:
+        if pipe is not None and world > 1:
+            last = unpack_records(last.cpu().numpy(), total_utts, world, lmax)
+        dump_outputs(args.dump_outputs, *last)
     if pipe is not None:
         pipe.close()
 
@@ -669,30 +680,18 @@ def main():
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
-    ke = max(10, min(K, 40)) if ms < 20 else max(3, min(K, 10))
-    ereps = int(min(50, max(3, math.ceil(500.0 / max(ms * ke, 1e-3)))))
-    if world > 1:
-        rt = torch.tensor([ereps], device=dev)
-        dist.broadcast(rt, 0)
-        ereps = int(rt.item())
     for k in brk:
         brk[k] = 0.0
-    e2e_reps = []
-    texts = None
-    for _ in range(ereps):
-        if world > 1:
-            dist.barrier()
-        t0 = time.perf_counter()
-        texts = e2e_run(ke)
-        torch.cuda.synchronize()
-        t = torch.tensor([(time.perf_counter() - t0) / ke * 1e3], device=dev)
-        if world > 1:
-            dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        e2e_reps.append(float(t.item()))
-    e2e_ms = statistics.median(e2e_reps)
+    t0 = time.perf_counter()
+    texts = e2e_run(K)
+    torch.cuda.synchronize()
+    t = torch.tensor([(time.perf_counter() - t0) / K * 1e3], device=dev)
+    if world > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    e2e_ms = float(t.item())
     if pipe is not None:
         pipe.close()
-    brk = {k: v / (ereps * ke) for k, v in brk.items()}
+    brk = {k: v / K for k, v in brk.items()}
 
     # ---- roofline of the dominant kernel, measured live with CUDA events ----
     pk = peaks()
@@ -733,8 +732,7 @@ def main():
             # like the `value` measurement: inputs cycle over the pool of distinct device-resident batches (larger than L2), no
             # explicit flush -- a 256 MiB flush would also evict the 70 MB of weights a serving process keeps L2 resident
             eng.profile_enable(True)
-            reps_p = 6
-            for i in range(reps_p):
+            for i in range(K):
                 eng.encode(wl.pool[i % len(wl.pool)])
                 eng.ctc_greedy(to_host=False)
             prof = eng.profile_read()
@@ -753,14 +751,14 @@ def main():
                 "conv_front": 2.0 * (B * Tp * 19) * D * 9 * D,
             }
             total = sum(v[1] for v in prof.values())
-            prof_table = {k: {"launches_per_step": v[0] // reps_p, "us_per_launch": v[1] / v[0] * 1e3,
+            prof_table = {k: {"launches_per_step": v[0] // K, "us_per_launch": v[1] / v[0] * 1e3,
                               "share": v[1] / total} for k, v in sorted(prof.items(), key=lambda kv: -kv[1][1])}
             top = max((k for k in prof if k in flops), key=lambda k: prof[k][1])
             us_all = prof[top][1] / prof[top][0] * 1e3
             # second pass: event pairs around the dominant class ONLY, so the other ~70 launches of the step stay back to back
             # and the CPU-side event records do not open gaps in front of the timed kernel
             eng.profile_enable(True, only=top)
-            for i in range(reps_p):
+            for i in range(K):
                 eng.encode(wl.pool[i % len(wl.pool)])
                 eng.ctc_greedy(to_host=False)
             prof1 = eng.profile_read()
@@ -772,7 +770,7 @@ def main():
                     "us_per_launch": us, "us_per_launch_all_classes_timed": us_all, "share_of_step": prof[top][1] / total,
                     "algorithmic_flops_per_launch": flops[top],
                     "step_tensor_frac_sustained": (conf["gflop_per_utt"] * B / ms) / pk["bf16_tflops_sustained"],
-                    "note": "us_per_launch: CUDA-event pairs around the launches of this kernel class only, 6 single-batch steps "
+                    "note": f"us_per_launch: CUDA-event pairs around the launches of this kernel class only, {K} single-batch steps "
                             "over distinct input batches (pool larger than L2, no flush; average over the plain and the "
                             "chained launches); shares: a first pass with pairs around every launch"}
             try:
@@ -815,8 +813,7 @@ def main():
                                 if wl.pipelined else "one batch at a time on one stream"),
                        "l2": f"inputs larger than L2: {len(pool)} distinct device-resident batches ({wl.pool_bytes / 1e6:.0f} MB) "
                              "cycled; no explicit flush",
-                       "timed_region": {"repetitions_of_k_steps": reps, "total_s": sum(rep_ms) / 1e3,
-                                        "ms_per_step_quantiles": q_ms, "statistic": "median repetition"},
+                       "timed_region": {"steps": K, "total_s": timed_ms / 1e3},
                        "single_stream_ms_per_step": single_ms,
                        "single_stream_quantiles": quantiles(single),
                        "single_stream_note": "one batch at a time, 256 MiB memset L2 flush between steps (outside the events)",
@@ -827,12 +824,11 @@ def main():
                        "numa_pinned_cpus": numa_cpus},
             "clocks": sampler.result(),
             "e2e": {"value": total_utts / (e2e_ms * 1e-3), "unit": "utt/s", "ms_per_step": e2e_ms,
-                    "ms_per_step_quantiles": quantiles(e2e_reps),
                     "h2d_bytes_per_step": wl.h2d_bytes(), "d2h_bytes_per_step": wl.d2h_bytes(),
                     "host_ms_per_step_rank0": brk,
                     "api": (f"InferencePredictor.pipeline(depth={depth}).submit(host fbank)/result() + host detokenisation"
                             if wl.pipelined else "engine.encode/encode_chunk(host fbank) + decoder + D2H of the best ids + host detokenisation")},
-            "gpu_launches": int((launches1 - launches0) // max(1, reps)),
+            "gpu_launches": int(launches1 - launches0),
             "roofline": roof, "cpu_baseline": cpu, "kernel_profile": prof_table,
             "sample_text_len": len(texts[0]) if texts else 0,
         }

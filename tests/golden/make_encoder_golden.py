@@ -154,7 +154,10 @@ def make_squeezeformer(path, streaming=True, seed=1000, lens=LENS, chunk_T=211, 
     return out
 
 
-def make_efficient_conformer(path, streaming=False, seed=1000, norm="batch_norm", lens=LENS, chunk_T=211, vocab=40, **kw):
+def make_efficient_conformer(path, streaming=False, seed=1000, norm="batch_norm", lens=LENS, chunk_T=211, vocab=40,
+                             att_cache_step=1, **kw):
+    """att_cache_step > 1 stores every att_cache_step-th channel of the final attention cache (all blocks, heads and frames)
+    together with its full shape, to keep a large fixture under 1 MB."""
     from ppasr.model_utils.efficient_conformer.encoder import EfficientConformerEncoder
     from ppasr.model_utils.loss.ctc import CTCLoss
     from ppasr.model_utils.utils.cmvn import GlobalCMVN
@@ -179,6 +182,11 @@ def make_efficient_conformer(path, streaming=False, seed=1000, norm="batch_norm"
     load_into(ctc, weights, "ctc.")
     feats, lens, chunk_feats = inputs(lens, chunk_T if streaming else 0, seed)
     out = run_former(enc, ctc, feats, lens, chunk_feats)
+    if att_cache_step > 1:
+        att = out["chunk_att_cache"]
+        out["chunk_att_cache_shape"] = np.array(att.shape)
+        out["chunk_att_cache_step"] = np.array(att_cache_step)
+        out["chunk_att_cache"] = np.ascontiguousarray(att[..., ::att_cache_step])
     np.savez_compressed(path, cfg=np.array(repr(cfg.to_dict())), seed=seed, feats=feats.astype(np.float32), lens=lens,
                         chunk_feats=(chunk_feats if chunk_feats is not None else np.zeros((0, 80), np.float32)), **out)
     return out
@@ -285,7 +293,7 @@ if __name__ == "__main__":
                                  seed=1005)
         make_efficient_conformer(G("efficient_conformer_gpu_stream12"), streaming=True, norm="layer_norm", lens=(99,),
                                  chunk_T=67 + 64 * 5, vocab=120, num_blocks=12, group_layer_idx=(0, 1, 2, 3), stride_layer_idx=3,
-                                 seed=1006)
+                                 seed=1006, att_cache_step=4)
         make_deepspeech2(G("deepspeech2_gpu_stream_lstm"), True, False, lens=(203, 150, 99), chunk_T=67 + 64 * 2, chunk_B=2,
                          vocab=120, nl=2, H=256)
         make_deepspeech2(G("deepspeech2_gpu_offline_gru"), False, True, lens=(203, 150, 99), vocab=120, nl=2, H=256)

@@ -95,8 +95,11 @@ def test_chunk_chain_matches_reference_code(fname):
             x, att, cnn = o.get_encoder_out_chunk(torch.from_numpy(cf[None, a:b]), off, required, att, cnn, return_logits=True)
             off += x.shape[1]
             outs.append(x[0].numpy())
-        assert tuple(att.shape) == g["chunk_att_cache"].shape and tuple(cnn.shape) == g["chunk_cnn_cache"].shape
-        np.testing.assert_allclose(att.numpy(), g["chunk_att_cache"], rtol=0, atol=1e-5)
+        # the largest fixture stores every step-th channel of the attention cache (make_encoder_golden.py, att_cache_step)
+        step = int(g["chunk_att_cache_step"]) if "chunk_att_cache_step" in g.files else 1
+        att_shape = tuple(g["chunk_att_cache_shape"]) if step > 1 else g["chunk_att_cache"].shape
+        assert tuple(att.shape) == att_shape and tuple(cnn.shape) == g["chunk_cnn_cache"].shape
+        np.testing.assert_allclose(att.numpy()[..., ::step], g["chunk_att_cache"], rtol=0, atol=1e-5)
         np.testing.assert_allclose(cnn.numpy(), g["chunk_cnn_cache"], rtol=0, atol=1e-5)
     outs = np.concatenate(outs, 1 if outs[0].ndim == 3 else 0)
     assert outs.shape == g["chunk_logits"].shape
