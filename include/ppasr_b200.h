@@ -63,10 +63,11 @@ int ppasr_b200_set_pdl(int32_t enable);
 
 /* Process-wide: fused feed-forward kernel variant (env PPASR_B200_FFN_SPLIT). 1 (default) = each 128-row tile is
  * computed by a 2-CTA thread-block cluster, the 2048-wide hidden dimension split over the pair and the two partial
- * outputs reduced through distributed shared memory (2 x ceil(M/128) CTAs per launch: lowest latency of one launch);
- * 2 = the same two-team Swish pipeline on one CTA per tile (least SM time: used when several batches are in flight);
- * 0 = the round-1 kernel. Replaces nothing in the reference (a tuning switch of positionwise.py:30-39's kernel);
- * results agree to fp32 summation order. */
+ * outputs reduced through distributed shared memory (2 x ceil(M/128) CTAs per launch: lowest latency of one launch;
+ * a hidden dimension of fewer than 4 or an odd number of 128-wide chunks runs as 2);
+ * 2 = the same two-team Swish pipeline on one CTA per tile (least SM time: used when several batches are in flight).
+ * Any other mode returns PPASR_ERR_INVALID and keeps the current one. Replaces nothing in the reference (a tuning
+ * switch of positionwise.py:30-39's kernel); results agree to fp32 summation order. */
 int ppasr_b200_set_ffn_split(int32_t mode);
 int ppasr_b200_get_ffn_split(void);
 
@@ -233,11 +234,11 @@ int ppasr_b200_fbank(const float* audio, int32_t B, int64_t stride, int32_t N, c
                      int32_t sample_rate, int32_t db_normalize, float target_db, float* gain_ws, float* out, int32_t Tmax,
                      void* stream);
 
-/* Switches: "fused_ffn" / "fused_attn_out" (default 1) select the fused row-tile kernels, "fused_dwconv" (default 0; causal
- * models) computes the conv module's depthwise stage in the chained FFN kernel's prologue (measured slower, kept for A/B), "fused_conv" (default 2) the
+/* Switches: "fused_ffn" / "fused_attn_out" (default 1) select the fused row-tile kernels, "fused_conv" (default 2) the
  * subsampling front end: 2 = conv1 (split-tf32 GEMM) as the A-operand producer of the conv2 GEMM in one kernel, 0 = conv1 kernel + conv2 GEMM
- * through the stride-phase images (bit-identical to 2 with conv1_tc = 1), 1 = the CUDA-core fused producer (slower; kept for A/B); "conv1_tc" (default 1) the first
- * subsampling conv on the tensor cores (split-tf32, conv1_tc.cu; 0 = the CUDA-core kernel); "host_sync" (default 1): ppasr_b200_ctc_greedy with host outputs synchronises the stream before
+ * through the stride-phase images (bit-identical to 2 with conv1_tc = 1; the only front end for feat_dim > 96); "conv1_tc" (default 1) the first
+ * subsampling conv on the tensor cores (split-tf32, conv1_tc.cu; 0 = the CUDA-core kernel); "ffn_split" (1 or 2) = ppasr_b200_set_ffn_split;
+ * "host_sync" (default 1): ppasr_b200_ctc_greedy with host outputs synchronises the stream before
  * returning -- 0 leaves the copies in flight (pinned host buffers; the caller synchronises), used by the
  * double-buffered serving pipeline. */
 int ppasr_b200_set_option(ppasr_b200_ctx* ctx, const char* name, int32_t value);

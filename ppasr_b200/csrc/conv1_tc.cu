@@ -319,7 +319,7 @@ conv1_tc_kernel(const __grid_constant__ CUtensorMap tmap_phase, const Conv1TcPar
 //   warps 12-15 : A1 producers (thread = row), inputs of the next two taps in flight
 //   warps 16-23 : epilogue-1: conv1 accumulator -> ReLU -> bf16 -> the 128B-swizzled K-major A2 tile the conv2 MMA reads
 // Arithmetic is identical to conv1_tc_kernel + the CONV GEMM (same MMAs in the same order, same roundings): the two paths
-// agree bit for bit (tests/test_gpu_parity.py::test_fused_conv_front_bit_identical).
+// agree bit for bit (tests/test_gpu_parity.py::test_conv_front_tc_bit_identical).
 // ------------------------------------------------------------------------------------------------
 constexpr int CF2_THREADS = 768;
 constexpr int CF2_A1_BYTES = 128 * 128;   // [128 rows][32 tf32]

@@ -5,18 +5,18 @@
 //                                                                  convolution.py:104-106)
 //   g_out = GLU(Wpw1 . y + bpw1)                                  (pointwise_conv1 + glu, convolution.py:119-123)
 //
-// Same row-tile skeleton as fused_ffn.cu: the fp32 residual tile is preloaded into the TMEM accumulator
-// (O, columns [256,512)), the out-projection MMAs accumulate on top of it, the row owners normalise straight
-// from TMEM and write the bf16 LayerNorm output into the (reused) A tiles in shared memory -- y never goes
-// to HBM -- then the 512-wide pointwise_conv1 runs as two 128x256x16 MMA groups (gate/value rows are
-// interleaved so GLU is thread-local) and g is written with coalesced stores through an smem staging tile.
+// Same row-tile skeleton as fused_ffn.cu. The out-projection starts from zero in the TMEM accumulator (O, columns
+// [256,512)) as soon as the att tile has landed; the row owners add the old residual (prefetched into registers with
+// coalesced loads while the TMA / MMA run) and bo in the same slab pass that writes x back: v = O + x_old + bo ->
+// statistics, x_new -> TMEM O and -> global. They then normalise straight from TMEM and write the bf16 LayerNorm output
+// into the (reused) A tiles in shared memory -- y never goes to HBM -- then the 512-wide pointwise_conv1 runs as two
+// 128x256x16 MMA groups (gate/value rows are interleaved so GLU is thread-local) and g is written with coalesced stores
+// through an smem staging tile.
 #include "kernels.h"
 #include "launch.h"
 #include "ptx.cuh"
 #include "row_tile.cuh"
 
-#include <atomic>
-#include <cstdlib>
 #include <mutex>
 
 namespace ppasr {
@@ -46,10 +46,6 @@ struct AttnOutParams {
   float eps;
 };
 
-// V2 = no serial residual preload: the out-projection starts from zero as soon as the att tile has landed, and the row
-// owners add the old residual (prefetched into registers with coalesced loads while the TMA / MMA run) in the same slab pass
-// that writes x back: v = O + x_old + bo -> statistics, x_new -> TMEM O (for the LayerNorm pass) and -> global.
-template <bool V2>
 __global__ void __launch_bounds__(AO_THREADS, 1)
 fused_attn_out_kernel(const __grid_constant__ CUtensorMap tm_att, const __grid_constant__ CUtensorMap tm_wo,
                       const __grid_constant__ CUtensorMap tm_wpw1, const AttnOutParams p) {
@@ -62,11 +58,10 @@ fused_attn_out_kernel(const __grid_constant__ CUtensorMap tm_att, const __grid_c
   uint64_t* a_full = bars;        // TMA att tile
   uint64_t* w_full = bars + 1;    // [3]
   uint64_t* w_empty = bars + 4;   // [3]
-  uint64_t* x_loaded = bars + 7;  // 256
-  uint64_t* pre_full = bars + 8;  // out-projection accumulated
-  uint64_t* a_ready = bars + 9;   // 256: y in A tiles, O drained
-  uint64_t* g_full = bars + 10;   // [2] halves of pointwise_conv1
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 12);
+  uint64_t* pre_full = bars + 7;  // out-projection accumulated
+  uint64_t* a_ready = bars + 8;   // 256: y in A tiles, O drained
+  uint64_t* g_full = bars + 9;    // [2] halves of pointwise_conv1
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 11);
 
   const int warp_idx = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -83,7 +78,6 @@ fused_attn_out_kernel(const __grid_constant__ CUtensorMap tm_att, const __grid_c
       mbar_init(&w_full[i], 1);
       mbar_init(&w_empty[i], 1);
     }
-    mbar_init(x_loaded, 256);
     mbar_init(pre_full, 1);
     mbar_init(a_ready, 256);
     mbar_init(&g_full[0], 1);
@@ -124,7 +118,7 @@ fused_attn_out_kernel(const __grid_constant__ CUtensorMap tm_att, const __grid_c
       int slot = 0;
       uint32_t phase = 0;
       const uint32_t a_addr = smem_u32(s_a);
-      auto gemm256 = [&](uint32_t tmem_d, bool accumulate_first) {
+      auto gemm256 = [&](uint32_t tmem_d) {
         for (int kb = 0; kb < 4; ++kb) {
           mbar_wait(&w_full[slot], phase);
           tc_fence_after();
@@ -132,21 +126,20 @@ fused_attn_out_kernel(const __grid_constant__ CUtensorMap tm_att, const __grid_c
 #pragma unroll
           for (int k = 0; k < 4; ++k)
             umma_bf16(tmem_d, umma_desc_k_sw128(a_addr + kb * AO_TILE + k * 32), umma_desc_k_sw128(w_addr + k * 32), idesc,
-                      (accumulate_first || (kb | k) != 0) ? 1u : 0u);
+                      (kb | k) != 0 ? 1u : 0u);
           umma_commit(&w_empty[slot]);
           if (++slot == AO_RING) slot = 0, phase ^= 1;
         }
       };
       mbar_wait(a_full, 0);
-      if (!V2) mbar_wait(x_loaded, 0);
       tc_fence_after();
-      gemm256(tmem_o, !V2);  // O (= x + bo, preloaded; V2: from zero) += att . Wo^T
+      gemm256(tmem_o);  // O = att . Wo^T (the row owners add the residual)
       umma_commit(pre_full);
       mbar_wait(a_ready, 0);  // y replaced att in the A tiles; O has been drained
       tc_fence_after();
-      gemm256(tmem_base, false);  // G[:, 0:256]
+      gemm256(tmem_base);  // G[:, 0:256]
       umma_commit(&g_full[0]);
-      gemm256(tmem_o, false);     // G[:, 256:512]
+      gemm256(tmem_o);     // G[:, 256:512]
       umma_commit(&g_full[1]);
     }
   } else if (warp_idx >= 4) {
@@ -164,152 +157,25 @@ fused_attn_out_kernel(const __grid_constant__ CUtensorMap tm_att, const __grid_c
       pad = (row_g - b * p.T) >= __ldg(p.lens + b);
     }
     float* slab = reinterpret_cast<float*>(s_h);
-    if (V2) {
-      const int cq = ct & 15;
-      float4 pre[8];  // this thread's share of the next residual slab (16 rows apart, 16 B per row segment)
-      auto prefetch = [&](int s) {
+    const int cq = ct & 15;
+    float4 pre[8];  // this thread's share of the next residual slab (16 rows apart, 16 B per row segment)
+    auto prefetch = [&](int s) {
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int rr = (ct >> 4) + 16 * i;
-          pre[i] = ((m0 + rr) < p.M) ? __ldcg(reinterpret_cast<const float4*>(p.x + (size_t)(m0 + rr) * 256 + s * 64) + cq)
-                                     : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-      };
-      prefetch(0);
-      mbar_wait(pre_full, 0);
-      tc_fence_after();
-      FfnStat st{0.f, 0.f, 0.f};
-      for (int s = 0; s < 4; ++s) {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) *reinterpret_cast<float4*>(slab + ((ct >> 4) + 16 * i) * AO_SLAB_PITCH + cq * 4) = pre[i];
-        if (s + 1 < 4) prefetch(s + 1);
-        named_bar_sync(1, 256);
-        if (half == (s >> 1)) {
-#pragma unroll
-          for (int c = 0; c < 2; ++c) {
-            const int cc = s * 64 + c * 32;
-            uint32_t ro[32];
-            tmem_ld_32x32b_x32(tmem_o + lane_base + cc, ro);
-            tmem_ld_wait();
-            float v[32];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              const float4 xo = *reinterpret_cast<const float4*>(slab + r * AO_SLAB_PITCH + c * 32 + 4 * j);
-              const float4 bb = __ldg(reinterpret_cast<const float4*>(p.bo + cc) + j);
-              v[4 * j + 0] = __uint_as_float(ro[4 * j + 0]) + xo.x + bb.x;
-              v[4 * j + 1] = __uint_as_float(ro[4 * j + 1]) + xo.y + bb.y;
-              v[4 * j + 2] = __uint_as_float(ro[4 * j + 2]) + xo.z + bb.z;
-              v[4 * j + 3] = __uint_as_float(ro[4 * j + 3]) + xo.w + bb.w;
-              *reinterpret_cast<float4*>(slab + r * AO_SLAB_PITCH + c * 32 + 4 * j) =
-                  make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-              ro[4 * j + 0] = __float_as_uint(v[4 * j + 0]), ro[4 * j + 1] = __float_as_uint(v[4 * j + 1]);
-              ro[4 * j + 2] = __float_as_uint(v[4 * j + 2]), ro[4 * j + 3] = __float_as_uint(v[4 * j + 3]);
-            }
-            tmem_st_32x32b_x32(tmem_o + lane_base + cc, ro);  // x_new stays in O for the LayerNorm pass
-            ffn_add_chunk(st, v);
-          }
-        }
-        named_bar_sync(1, 256);
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int rr = (ct >> 4) + 16 * i;
-          if ((m0 + rr) < p.M)
-            *(reinterpret_cast<float4*>(p.x + (size_t)(m0 + rr) * 256 + s * 64) + cq) =
-                *reinterpret_cast<const float4*>(slab + rr * AO_SLAB_PITCH + cq * 4);
-        }
-        named_bar_sync(1, 256);
-      }
-      tmem_st_wait();
-      float4* sc = reinterpret_cast<float4*>(s_h + 128 * AO_SLAB_PITCH * 4);
-      ffn_exchange(st, sc, r, half, 2);
-      const float mean = st.mean;
-      const float rstd = rsqrtf(st.m2 * (1.0f / 256.0f) + p.eps);
-      // y = LN(x_new) -> A tiles (this thread's 128 columns, read back from O)
-#pragma unroll 1
-      for (int c = 0; c < 4; ++c) {
-        const int cc = half * 128 + c * 32;
-        uint32_t ro[32];
-        tmem_ld_32x32b_x32(tmem_o + lane_base + cc, ro);
-        tmem_ld_wait();
-        uint32_t pk[16];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const float4 gg = __ldg(reinterpret_cast<const float4*>(p.ln_g + cc) + j);
-          const float4 bb = __ldg(reinterpret_cast<const float4*>(p.ln_b + cc) + j);
-          const float y0 = (__uint_as_float(ro[4 * j + 0]) - mean) * rstd * gg.x + bb.x;
-          const float y1 = (__uint_as_float(ro[4 * j + 1]) - mean) * rstd * gg.y + bb.y;
-          const float y2 = (__uint_as_float(ro[4 * j + 2]) - mean) * rstd * gg.z + bb.z;
-          const float y3 = (__uint_as_float(ro[4 * j + 3]) - mean) * rstd * gg.w + bb.w;
-          pk[2 * j] = pad ? 0u : pack_bf16x2(y0, y1);
-          pk[2 * j + 1] = pad ? 0u : pack_bf16x2(y2, y3);
-        }
-        uint8_t* atile = s_a + (cc >> 6) * AO_TILE + r * 128;
-        const int ch0 = (cc & 63) >> 3;
-#pragma unroll
-        for (int q4 = 0; q4 < 4; ++q4)
-          *reinterpret_cast<uint4*>(atile + (((ch0 + q4) ^ (r & 7)) << 4)) =
-              make_uint4(pk[4 * q4], pk[4 * q4 + 1], pk[4 * q4 + 2], pk[4 * q4 + 3]);
-      }
-    } else {
-    // ---- residual (+ bo) -> TMEM O through coalesced 64-column slabs ----
-    for (int s = 0; s < 4; ++s) {
-      {
-        const int cq = ct & 15;
-        float4 v[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int rr = (ct >> 4) + 16 * i;
-          v[i] = ((m0 + rr) < p.M) ? __ldcg(reinterpret_cast<const float4*>(p.x + (size_t)(m0 + rr) * 256 + s * 64) + cq)
+      for (int i = 0; i < 8; ++i) {
+        const int rr = (ct >> 4) + 16 * i;
+        pre[i] = ((m0 + rr) < p.M) ? __ldcg(reinterpret_cast<const float4*>(p.x + (size_t)(m0 + rr) * 256 + s * 64) + cq)
                                    : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-#pragma unroll
-        for (int i = 0; i < 8; ++i) *reinterpret_cast<float4*>(slab + ((ct >> 4) + 16 * i) * AO_SLAB_PITCH + cq * 4) = v[i];
       }
-      named_bar_sync(1, 256);
-      if (half == (s >> 1)) {
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          uint32_t v[32];
-          const int col0 = s * 64 + c * 32;
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {
-            float4 t = *reinterpret_cast<const float4*>(slab + r * AO_SLAB_PITCH + c * 32 + 4 * j);
-            const float4 bb = __ldg(reinterpret_cast<const float4*>(p.bo + col0) + j);
-            v[4 * j] = __float_as_uint(t.x + bb.x), v[4 * j + 1] = __float_as_uint(t.y + bb.y);
-            v[4 * j + 2] = __float_as_uint(t.z + bb.z), v[4 * j + 3] = __float_as_uint(t.w + bb.w);
-          }
-          tmem_st_32x32b_x32(tmem_o + lane_base + col0, v);
-        }
-        tmem_st_wait();
-      }
-      named_bar_sync(1, 256);
-    }
-    tc_fence_before();
-    mbar_arrive(x_loaded);
-    // ---- x_new = O : statistics, y -> A tiles, x_new -> global through the slabs ----
+    };
+    prefetch(0);
     mbar_wait(pre_full, 0);
     tc_fence_after();
-    float4* sc = reinterpret_cast<float4*>(s_h + 128 * AO_SLAB_PITCH * 4);  // exchange slots behind the slab
     FfnStat st{0.f, 0.f, 0.f};
-#pragma unroll 1
-    for (int c = 0; c < 4; c += 2) {
-      uint32_t ro[2][32];
-      tmem_ld_32x32b_x32(tmem_o + lane_base + half * 128 + c * 32, ro[0]);
-      tmem_ld_32x32b_x32(tmem_o + lane_base + half * 128 + c * 32 + 32, ro[1]);
-      tmem_ld_wait();
-#pragma unroll
-      for (int u = 0; u < 2; ++u) {
-        float v[32];
-#pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(ro[u][j]);
-        ffn_add_chunk(st, v);
-      }
-    }
-    ffn_exchange(st, sc, r, half, 2);
-    const float mean = st.mean;
-    const float rstd = rsqrtf(st.m2 * (1.0f / 256.0f) + p.eps);
-    // x write-out: slab s holds columns [64s, 64s+64); owners (half == s/2) fill it, everyone stores it coalesced
     for (int s = 0; s < 4; ++s) {
+#pragma unroll
+      for (int i = 0; i < 8; ++i) *reinterpret_cast<float4*>(slab + ((ct >> 4) + 16 * i) * AO_SLAB_PITCH + cq * 4) = pre[i];
+      if (s + 1 < 4) prefetch(s + 1);
+      named_bar_sync(1, 256);
       if (half == (s >> 1)) {
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
@@ -317,42 +183,64 @@ fused_attn_out_kernel(const __grid_constant__ CUtensorMap tm_att, const __grid_c
           uint32_t ro[32];
           tmem_ld_32x32b_x32(tmem_o + lane_base + cc, ro);
           tmem_ld_wait();
-          uint32_t pk[16];
+          float v[32];
 #pragma unroll
           for (int j = 0; j < 8; ++j) {
+            const float4 xo = *reinterpret_cast<const float4*>(slab + r * AO_SLAB_PITCH + c * 32 + 4 * j);
+            const float4 bb = __ldg(reinterpret_cast<const float4*>(p.bo + cc) + j);
+            v[4 * j + 0] = __uint_as_float(ro[4 * j + 0]) + xo.x + bb.x;
+            v[4 * j + 1] = __uint_as_float(ro[4 * j + 1]) + xo.y + bb.y;
+            v[4 * j + 2] = __uint_as_float(ro[4 * j + 2]) + xo.z + bb.z;
+            v[4 * j + 3] = __uint_as_float(ro[4 * j + 3]) + xo.w + bb.w;
             *reinterpret_cast<float4*>(slab + r * AO_SLAB_PITCH + c * 32 + 4 * j) =
-                make_float4(__uint_as_float(ro[4 * j]), __uint_as_float(ro[4 * j + 1]), __uint_as_float(ro[4 * j + 2]),
-                            __uint_as_float(ro[4 * j + 3]));
-            const float4 gg = __ldg(reinterpret_cast<const float4*>(p.ln_g + cc) + j);
-            const float4 bb = __ldg(reinterpret_cast<const float4*>(p.ln_b + cc) + j);
-            const float y0 = (__uint_as_float(ro[4 * j + 0]) - mean) * rstd * gg.x + bb.x;
-            const float y1 = (__uint_as_float(ro[4 * j + 1]) - mean) * rstd * gg.y + bb.y;
-            const float y2 = (__uint_as_float(ro[4 * j + 2]) - mean) * rstd * gg.z + bb.z;
-            const float y3 = (__uint_as_float(ro[4 * j + 3]) - mean) * rstd * gg.w + bb.w;
-            pk[2 * j] = pad ? 0u : pack_bf16x2(y0, y1);
-            pk[2 * j + 1] = pad ? 0u : pack_bf16x2(y2, y3);
+                make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
+            ro[4 * j + 0] = __float_as_uint(v[4 * j + 0]), ro[4 * j + 1] = __float_as_uint(v[4 * j + 1]);
+            ro[4 * j + 2] = __float_as_uint(v[4 * j + 2]), ro[4 * j + 3] = __float_as_uint(v[4 * j + 3]);
           }
-          uint8_t* atile = s_a + (cc >> 6) * AO_TILE + r * 128;
-          const int ch0 = (cc & 63) >> 3;
-#pragma unroll
-          for (int q4 = 0; q4 < 4; ++q4)
-            *reinterpret_cast<uint4*>(atile + (((ch0 + q4) ^ (r & 7)) << 4)) =
-                make_uint4(pk[4 * q4], pk[4 * q4 + 1], pk[4 * q4 + 2], pk[4 * q4 + 3]);
+          tmem_st_32x32b_x32(tmem_o + lane_base + cc, ro);  // x_new stays in O for the LayerNorm pass
+          ffn_add_chunk(st, v);
         }
       }
       named_bar_sync(1, 256);
-      {
-        const int cq = ct & 15;
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int rr = (ct >> 4) + 16 * i;
-          if ((m0 + rr) < p.M)
-            *(reinterpret_cast<float4*>(p.x + (size_t)(m0 + rr) * 256 + s * 64) + cq) =
-                *reinterpret_cast<const float4*>(slab + rr * AO_SLAB_PITCH + cq * 4);
-        }
+      for (int i = 0; i < 8; ++i) {
+        const int rr = (ct >> 4) + 16 * i;
+        if ((m0 + rr) < p.M)
+          *(reinterpret_cast<float4*>(p.x + (size_t)(m0 + rr) * 256 + s * 64) + cq) =
+              *reinterpret_cast<const float4*>(slab + rr * AO_SLAB_PITCH + cq * 4);
       }
       named_bar_sync(1, 256);
     }
+    tmem_st_wait();
+    float4* sc = reinterpret_cast<float4*>(s_h + 128 * AO_SLAB_PITCH * 4);
+    ffn_exchange(st, sc, r, half, 2);
+    const float mean = st.mean;
+    const float rstd = rsqrtf(st.m2 * (1.0f / 256.0f) + p.eps);
+    // y = LN(x_new) -> A tiles (this thread's 128 columns, read back from O)
+#pragma unroll 1
+    for (int c = 0; c < 4; ++c) {
+      const int cc = half * 128 + c * 32;
+      uint32_t ro[32];
+      tmem_ld_32x32b_x32(tmem_o + lane_base + cc, ro);
+      tmem_ld_wait();
+      uint32_t pk[16];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const float4 gg = __ldg(reinterpret_cast<const float4*>(p.ln_g + cc) + j);
+        const float4 bb = __ldg(reinterpret_cast<const float4*>(p.ln_b + cc) + j);
+        const float y0 = (__uint_as_float(ro[4 * j + 0]) - mean) * rstd * gg.x + bb.x;
+        const float y1 = (__uint_as_float(ro[4 * j + 1]) - mean) * rstd * gg.y + bb.y;
+        const float y2 = (__uint_as_float(ro[4 * j + 2]) - mean) * rstd * gg.z + bb.z;
+        const float y3 = (__uint_as_float(ro[4 * j + 3]) - mean) * rstd * gg.w + bb.w;
+        pk[2 * j] = pad ? 0u : pack_bf16x2(y0, y1);
+        pk[2 * j + 1] = pad ? 0u : pack_bf16x2(y2, y3);
+      }
+      uint8_t* atile = s_a + (cc >> 6) * AO_TILE + r * 128;
+      const int ch0 = (cc & 63) >> 3;
+#pragma unroll
+      for (int q4 = 0; q4 < 4; ++q4)
+        *reinterpret_cast<uint4*>(atile + (((ch0 + q4) ^ (r & 7)) << 4)) =
+            make_uint4(pk[4 * q4], pk[4 * q4 + 1], pk[4 * q4 + 2], pk[4 * q4 + 3]);
     }
     tc_fence_before();
     fence_proxy_async_smem();
@@ -407,18 +295,6 @@ fused_attn_out_kernel(const __grid_constant__ CUtensorMap tm_att, const __grid_c
   }
 }
 
-static std::atomic<int> g_attn_out_v2{-1};
-int attn_out_variant() {
-  int v = g_attn_out_v2.load(std::memory_order_relaxed);
-  if (v < 0) {
-    const char* e = getenv("PPASR_B200_ATTN_OUT_V2");  // 0 = the round-1 variant with the serial residual preload (A/B runs)
-    v = (e != nullptr && e[0] == '0') ? 0 : 1;
-    g_attn_out_v2.store(v, std::memory_order_relaxed);
-  }
-  return v;
-}
-void set_attn_out_variant(int v) { g_attn_out_v2.store(v ? 1 : 0, std::memory_order_relaxed); }
-
 cudaError_t launch_fused_attn_out(const CUtensorMap& tm_att, const CUtensorMap& tm_wo, const CUtensorMap& tm_wpw1, int M,
                                   float* x, __nv_bfloat16* g, const float* bo, const float* ln_g, const float* ln_b,
                                   const float* bpw1, const int* lens, int T, float eps, cudaStream_t st) {
@@ -426,18 +302,13 @@ cudaError_t launch_fused_attn_out(const CUtensorMap& tm_att, const CUtensorMap& 
   static std::once_flag once;
   static cudaError_t cfg_err = cudaSuccess;
   std::call_once(once, [] {
-    cfg_err = cudaFuncSetAttribute(fused_attn_out_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, AO_SMEM_TOTAL);
-    if (cfg_err == cudaSuccess)
-      cfg_err = cudaFuncSetAttribute(fused_attn_out_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, AO_SMEM_TOTAL);
+    cfg_err = cudaFuncSetAttribute(fused_attn_out_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, AO_SMEM_TOTAL);
   });
   if (cfg_err != cudaSuccess) return cfg_err;
-  const int v2 = attn_out_variant();
   AttnOutParams p;
   p.M = M, p.x = x, p.g = g, p.bo = bo, p.ln_g = ln_g, p.ln_b = ln_b, p.bpw1 = bpw1, p.lens = lens, p.T = T, p.eps = eps;
-  cudaError_t le = v2 ? launch_pdl(fused_attn_out_kernel<true>, dim3((M + 127) / 128), dim3(AO_THREADS), (size_t)AO_SMEM_TOTAL, st,
-                                   tm_att, tm_wo, tm_wpw1, p)
-                      : launch_pdl(fused_attn_out_kernel<false>, dim3((M + 127) / 128), dim3(AO_THREADS), (size_t)AO_SMEM_TOTAL, st,
-                                   tm_att, tm_wo, tm_wpw1, p);
+  cudaError_t le = launch_pdl(fused_attn_out_kernel, dim3((M + 127) / 128), dim3(AO_THREADS), (size_t)AO_SMEM_TOTAL, st, tm_att,
+                              tm_wo, tm_wpw1, p);
   count_launch();
   return le != cudaSuccess ? le : cudaGetLastError();
 }

@@ -1,4 +1,4 @@
-// Fused position-wise feed-forward block for sm_100a (tcgen05 + TMEM + TMA), one CTA per 128 rows.
+// Fused position-wise feed-forward block for sm_100a (tcgen05 + TMEM + TMA), 128 rows per tile.
 //
 //   plain  :  x <- x + W2s . swish(W1 . y + b1) + b2s                      (W2s = alpha*W2, b2s = alpha*b2)
 //   chained:  x <- x + mask * (Wp . z + bp)        (conv module's pointwise_conv2 + residual, pad rows masked)
@@ -10,17 +10,28 @@
 // surrounding residual / LayerNorm code of ConformerEncoderLayer.forward (conformer/encoder.py:380-386,
 // 407-429); chained mode additionally covers convolution.py:133-140 (pointwise_conv2 + pad masking).
 //
-// TMEM plan: S double buffer in columns [0,256), output accumulator O in [256,512).
-//  * The fp32 residual tile is preloaded INTO O (coalesced global loads -> smem slab -> tcgen05.st) while the
-//    first weight tiles stream in, and every MMA that produces a residual-branch term accumulates on top of it,
-//    so the residual add costs nothing and the epilogue never re-reads x.
-//  * The 2048-wide hidden activation never leaves the SM: 16 chunks of 128,
-//      GEMM1(j): S[j&1] = Y[128x256] . W1_j^T                 16 x tcgen05.mma 128x128x16
-//      swish(j): 256 threads: TMEM -> +b1 -> swish -> bf16 -> 128B-swizzled smem H[j&1]
-//      GEMM2(j): O += H[j&1][128x128] . W2s_j^T                8 x tcgen05.mma 128x256x16
-//    GEMM1(j+2) is issued right after GEMM2(j) so the tensor pipe always has queued work.
-//  * Weights stream through a 3 x 32 KB TMA ring (2 MB per CTA per call, L2 resident).
-//  * Epilogue: x/y tiles are staged in the (by then free) smem and written with coalesced 16-byte stores.
+// fused_ffn_split_kernel<PRE, SPLIT> computes one 128-row tile (PRE = chained mode). TMEM holds the S double buffer in
+// columns [0,256) and the output accumulator O in [256,512); the FF-wide hidden activation never leaves the SM:
+//     GEMM1(j): S[j&1] = Y[128x256] . W1_j^T                 16 x tcgen05.mma 128x128x16
+//     swish(j): TMEM -> +b1 -> swish -> bf16 -> 128B-swizzled smem H[j&1]
+//     GEMM2(j): O += H[j&1][128x128] . W2s_j^T                8 x tcgen05.mma 128x256x16
+//  * Swish runs on two teams of 8 warps (even / odd chunks), S is released right after the TMEM load, and GEMM1(j+2) is
+//    issued BEFORE GEMM2(j): the tensor pipe always has the next GEMM1 queued while a team is still in its Swish.
+//  * Weights stream through a 3 x 32 KB TMA ring; the tiles that do not depend on the predecessor kernel are requested
+//    before griddepcontrol.wait.
+//  * SPLIT (ffn_split mode 1): the tile is shared by a 2-CTA thread-block cluster. CTA `rank` owns hidden chunks
+//    [rank*NCH/2, (rank+1)*NCH/2) and ends with a PARTIAL output tile O_rank in TMEM. The two partials are reduced through
+//    distributed shared memory: each CTA stages its tile in shared memory, bulk-copies the 64 rows the PEER finalises into
+//    the peer's receive buffer (cp.async.bulk.shared::cluster, completion on the peer's mbarrier) and finalises its own 64
+//    rows. One launch therefore covers 2 x ceil(M/128) CTAs (124 at C2 instead of 62 on 148 SMs).
+//  * !SPLIT (ffn_split mode 2): the same pipeline on one CTA per tile, all chunks, all 128 rows (least SM time per launch).
+//  * The output tile is staged in fp32 shared memory and finalised warp-per-row: partial(s) + b2s [+ residual from global
+//    memory] -> LayerNorm(s) -> coalesced x / y stores.
+//  * plain mode: no residual preload at all -- x is added in the final pass from global memory (coalesced).
+//  * chained mode: the residual tile (+ masked bp) is preloaded into O through a coalesced smem slab, the pre-GEMM
+//    accumulates on top of it, and LN(x_mid) replaces z in the A tiles. Under SPLIT both CTAs run the small pre-GEMM +
+//    LayerNorm redundantly (1/16 of the FLOPs); rank 1 then discards the residual by starting its GEMM2 chain with
+//    accumulate = 0, so x_mid is counted once.
 #include "kernels.h"
 #include "launch.h"
 #include "ptx.cuh"
@@ -28,13 +39,13 @@
 
 #include <atomic>
 #include <cstdlib>
+#include <cstring>
 #include <mutex>
 
 namespace ppasr {
 
 void count_launch();
 
-constexpr int FFN_THREADS = 384;             // warps 0..3 control, 4..11 compute
 constexpr int FFN_TILE = 128 * 64 * 2;       // 16 KB: [128 rows x 64 bf16] swizzled tile
 constexpr int FFN_SMEM_A = 0;                // 4 tiles (Y or Z, K = 256)
 constexpr int FFN_SMEM_H = 4 * FFN_TILE;     // 2 buffers x 2 tiles (also: residual preload slab)
@@ -42,7 +53,6 @@ constexpr int FFN_SMEM_W = 8 * FFN_TILE;     // ring: 3 big slots x 32 KB
 constexpr int FFN_RING = 3;
 constexpr int FFN_SMEM_BAR = 14 * FFN_TILE;  // 229376
 constexpr int FFN_SMEM_TOTAL = FFN_SMEM_BAR + 512 + 1024;
-constexpr int FFN_XS_PITCH = 260;            // fp32 staging tile [128][260]: 16B-aligned rows, float4 access conflict-free
 constexpr int FFN_SLAB_PITCH = 68;           // residual preload slab [128][68] fp32 (64 columns at a time)
 
 struct FfnParams {
@@ -68,585 +78,8 @@ struct FfnParams {
   // residual itself becomes x <- LN(x + Wp z + bp; gp, bpn) (written back into TMEM O) and the FFN input is its adaptive
   // affine pre_ys * x + pre_yb (squeezeformer/encoder.py:468-487: MHA -> layer_norm1 -> ffn1, conv -> layer_norm3 -> ffn2)
   const float *pre_ys, *pre_yb;
-  // chained mode with the depthwise conv in front (dw_g != null): the A operand z of the pre-GEMM is not loaded but computed
-  // by the compute warps, z = swish(norm(depthwise_conv(g))) with causal left padding (convolution.py:108-133), rows t >=
-  // lens[b] zeroed -- the conv module's depthwise stage never leaves the SM either.
-  const __nv_bfloat16* dw_g;  // [M, 256] GLU output
-  const float *dw_w, *dw_b;   // [256, K], [256]
-  const float* dw_pad;        // [256] value of a left-padding frame (GLU(bias)); causal only
-  const float *dw_ng, *dw_nb; // norm gamma / beta (LayerNorm) or folded BatchNorm scale / shift
-  int dw_K, dw_ln;
 };
 
-// depthwise conv (+ norm + swish) of one 128-row tile straight into the swizzled A tiles. thread = channel for the
-// convolution (K-wide register ring over time, restarted every 16 rows and at utterance starts), warp = row for the norm.
-template <int K>
-DEVINL void dwconv_a_tiles(const FfnParams& p, int m0, int ct, int ew, int lane, uint8_t* s_a, uint8_t* scratch) {
-  // scratch (the idle H region, 64 KB): staged bf16 input rows [64 + K - 1][256], then the fp32 conv output of one
-  // 16-row sub-tile [16][256]
-  __nv_bfloat16* sin = reinterpret_cast<__nv_bfloat16*>(scratch);
-  float* sout = reinterpret_cast<float*>(scratch + (size_t)(64 + K - 1) * 512);
-  const int c = ct;
-  float wk[K];
-#pragma unroll
-  for (int j = 0; j < K; ++j) wk[j] = __ldg(p.dw_w + c * K + j);
-  const float bs = __ldg(p.dw_b + c);
-  const float padv = __bfloat162float(__float2bfloat16_rn(__ldg(p.dw_pad + c)));
-  const float sc = p.dw_ln ? 1.f : __ldg(p.dw_ng + c);
-  const float sh = p.dw_ln ? 0.f : __ldg(p.dw_nb + c);
-  const int T = p.T;
-#pragma unroll 1
-  for (int hf = 0; hf < 2; ++hf) {
-    // ---- stage rows [m0 + 64 hf - (K-1), m0 + 64 hf + 64) with coalesced 16-byte loads (all in flight together) ----
-    const int gr0 = m0 + hf * 64 - (K - 1);
-    constexpr int NCHUNK = (64 + K - 1) * 32;
-    for (int i = ct; i < NCHUNK; i += 256) {
-      const int rr = i >> 5, seg = i & 31;
-      const int gr = gr0 + rr;
-      uint4 v = make_uint4(0u, 0u, 0u, 0u);
-      if (gr >= 0 && gr < p.M) v = *reinterpret_cast<const uint4*>(p.dw_g + (size_t)gr * 256 + seg * 8);
-      *reinterpret_cast<uint4*>(sin + (size_t)rr * 256 + seg * 8) = v;
-    }
-    named_bar_sync(1, 256);
-#pragma unroll 1
-    for (int sub = 0; sub < 4; ++sub) {
-      const int l0 = sub * 16;            // first local row of the sub-tile inside this half
-      const int R0 = m0 + hf * 64 + l0;
-      int b = R0 / T, t = R0 - b * T;
-      float win[K];
-#pragma unroll
-      for (int j = 0; j < K - 1; ++j)     // history: frames t-(K-1)+j, left padding before the utterance start
-        win[j] = (t - (K - 1) + j >= 0) ? __bfloat162float(sin[(size_t)(l0 + j) * 256 + c]) : padv;
-#pragma unroll
-      for (int tb = 0; tb < 16; tb += K) {
-#pragma unroll
-        for (int u = 0; u < K; ++u) {
-          const int r = tb + u;
-          if (r < 16) {
-            if (t == 0 && r > 0) {  // a new utterance starts inside the sub-tile: its history is left padding
-#pragma unroll
-              for (int j = 0; j < K; ++j) win[j] = padv;
-            }
-            win[(u + K - 1) % K] = __bfloat162float(sin[(size_t)(l0 + r + K - 1) * 256 + c]);
-            float acc = bs;
-#pragma unroll
-            for (int j = 0; j < K; ++j) acc = fmaf(wk[j], win[(u + j) % K], acc);
-            sout[r * 256 + c] = acc * sc + sh;
-            if (++t == T) t = 0, ++b;
-          }
-        }
-      }
-      named_bar_sync(1, 256);
-      // norm + swish, warp = row, lane = 8 channels = one 16-byte chunk of the A tile
-#pragma unroll
-      for (int q = 0; q < 2; ++q) {
-        const int r = ew + 8 * q;
-        const int R = R0 + r;
-        float v[8];
-        const float4 a0 = *reinterpret_cast<const float4*>(sout + r * 256 + lane * 8);
-        const float4 a1 = *reinterpret_cast<const float4*>(sout + r * 256 + lane * 8 + 4);
-        v[0] = a0.x, v[1] = a0.y, v[2] = a0.z, v[3] = a0.w, v[4] = a1.x, v[5] = a1.y, v[6] = a1.z, v[7] = a1.w;
-        if (p.dw_ln) {
-          float s = 0.f;
-#pragma unroll
-          for (int i = 0; i < 8; ++i) s += v[i];
-          const float mean = warp_sum(s) * (1.0f / 256.0f);
-          float qq = 0.f;
-#pragma unroll
-          for (int i = 0; i < 8; ++i) qq += (v[i] - mean) * (v[i] - mean);
-          const float rstd = rsqrtf(warp_sum(qq) * (1.0f / 256.0f) + p.eps);
-#pragma unroll
-          for (int i = 0; i < 8; ++i) v[i] = (v[i] - mean) * rstd * __ldg(p.dw_ng + lane * 8 + i) + __ldg(p.dw_nb + lane * 8 + i);
-        }
-        bool zero = R >= p.M;
-        if (!zero && p.lens != nullptr) {
-          const int bb = R / T;
-          zero = (R - bb * T) >= __ldg(p.lens + bb);
-        }
-        uint32_t pk[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) pk[i] = zero ? 0u : pack_bf16x2(swish_rcp(v[2 * i]), swish_rcp(v[2 * i + 1]));
-        const int row = hf * 64 + l0 + r;
-        uint8_t* atile = s_a + (lane >> 3) * FFN_TILE + row * 128;
-        *reinterpret_cast<uint4*>(atile + (((lane & 7) ^ (row & 7)) << 4)) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-      }
-      named_bar_sync(1, 256);
-    }
-  }
-}
-
-template <bool PRE>
-__global__ void __launch_bounds__(FFN_THREADS, 1)
-fused_ffn_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_wp,
-                 const __grid_constant__ CUtensorMap tm_w1, const __grid_constant__ CUtensorMap tm_w2,
-                 const FfnParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* s_a = smem + FFN_SMEM_A;
-  uint8_t* s_h = smem + FFN_SMEM_H;
-  uint8_t* s_w = smem + FFN_SMEM_W;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + FFN_SMEM_BAR);
-  uint64_t* a_full = bars;       // TMA: A-operand tile (y, or z in chained mode)
-  uint64_t* w_full = bars + 1;   // [3]
-  uint64_t* w_empty = bars + 4;  // [3]
-  uint64_t* s_full = bars + 7;   // [2]
-  uint64_t* s_free = bars + 9;   // [2]
-  uint64_t* h_full = bars + 11;  // [2]
-  uint64_t* h_free = bars + 13;  // [2]
-  uint64_t* o_full = bars + 15;
-  uint64_t* x_loaded = bars + 16;  // residual tile is in TMEM O (256 arrivals)
-  uint64_t* pre_full = bars + 17;  // chained: pre-GEMM accumulated into O
-  uint64_t* a_ready = bars + 18;   // chained: LN output written to the A tiles (256 arrivals)
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 19);
-
-  const int warp_idx = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int m0 = blockIdx.x * 128;
-  const int NCH = p.nchunks;
-
-  if (warp_idx == 0 && elect_one()) {
-    tma_prefetch_desc(&tm_a);
-    tma_prefetch_desc(&tm_w1);
-    tma_prefetch_desc(&tm_w2);
-    if (PRE) tma_prefetch_desc(&tm_wp);
-  }
-  if (warp_idx == 1 && elect_one()) {
-    mbar_init(a_full, (PRE && p.dw_g != nullptr) ? 256 : 1);
-    for (int i = 0; i < FFN_RING; ++i) {
-      mbar_init(&w_full[i], 1);
-      mbar_init(&w_empty[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&s_full[i], 1);
-      mbar_init(&s_free[i], 256);
-      mbar_init(&h_full[i], 256);
-      mbar_init(&h_free[i], 1);
-    }
-    mbar_init(o_full, 1);
-    mbar_init(x_loaded, 256);
-    mbar_init(pre_full, 1);
-    mbar_init(a_ready, 256);
-    fence_barrier_init();
-    fence_proxy_async_smem();
-  }
-  if (warp_idx == 2) tmem_alloc<512>(tmem_ptr_smem);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_ptr_smem;
-  const uint32_t tmem_o = tmem_base + 256;
-  pdl_wait();
-  pdl_launch_dependents();
-
-  if (warp_idx == 0) {
-    // ============================ TMA producer ============================
-    if (elect_one()) {
-      if (!(PRE && p.dw_g != nullptr)) {
-        mbar_arrive_expect_tx(a_full, 4 * FFN_TILE);
-        for (int kb = 0; kb < 4; ++kb) tma_load_2d(s_a + kb * FFN_TILE, &tm_a, a_full, kb * 64, m0);
-      }
-      int slot = 0;
-      uint32_t phase = 0;
-      auto load_rows256 = [&](const CUtensorMap* tm, int k0) {  // one big slot: [256 rows x 64 K]
-        mbar_wait(&w_empty[slot], phase ^ 1);
-        mbar_arrive_expect_tx(&w_full[slot], 2 * FFN_TILE);
-        tma_load_2d(s_w + slot * 2 * FFN_TILE, tm, &w_full[slot], k0, 0);
-        if (++slot == FFN_RING) slot = 0, phase ^= 1;
-      };
-      auto load_w1 = [&](int j) {  // two big slots: k-blocks (0,1) and (2,3) of W1 rows [j*128, +128)
-        for (int s = 0; s < 2; ++s) {
-          mbar_wait(&w_empty[slot], phase ^ 1);
-          mbar_arrive_expect_tx(&w_full[slot], 2 * FFN_TILE);
-          tma_load_2d(s_w + slot * 2 * FFN_TILE, &tm_w1, &w_full[slot], (2 * s) * 64, j * 128);
-          tma_load_2d(s_w + slot * 2 * FFN_TILE + FFN_TILE, &tm_w1, &w_full[slot], (2 * s + 1) * 64, j * 128);
-          if (++slot == FFN_RING) slot = 0, phase ^= 1;
-        }
-      };
-      if (PRE)
-        for (int kb = 0; kb < 4; ++kb) load_rows256(&tm_wp, kb * 64);
-      load_w1(0);
-      if (NCH > 1) load_w1(1);
-      for (int j = 0; j < NCH; ++j) {
-        load_rows256(&tm_w2, j * 128);
-        load_rows256(&tm_w2, j * 128 + 64);
-        if (j + 2 < NCH) load_w1(j + 2);
-      }
-    }
-  } else if (warp_idx == 1) {
-    // ============================ MMA issuer ============================
-    if (elect_one()) {
-      constexpr uint32_t idesc_g1 = umma_idesc_bf16(128, 128);
-      constexpr uint32_t idesc_g2 = umma_idesc_bf16(128, 256);
-      int slot = 0;
-      uint32_t phase = 0;
-      const uint32_t a_addr = smem_u32(s_a);
-      mbar_wait(a_full, 0);
-      tc_fence_after();
-      if (PRE) {
-        // O (= x + mask*bp, preloaded) += Z . Wp^T
-        mbar_wait(x_loaded, 0);
-        tc_fence_after();
-        for (int kb = 0; kb < 4; ++kb) {
-          mbar_wait(&w_full[slot], phase);
-          tc_fence_after();
-          const uint32_t w_addr = smem_u32(s_w + slot * 2 * FFN_TILE);
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            umma_bf16(tmem_o, umma_desc_k_sw128(a_addr + kb * FFN_TILE + k * 32), umma_desc_k_sw128(w_addr + k * 32),
-                      idesc_g2, 1u);
-          umma_commit(&w_empty[slot]);
-          if (++slot == FFN_RING) slot = 0, phase ^= 1;
-        }
-        umma_commit(pre_full);
-        mbar_wait(a_ready, 0);  // LN(x) has replaced Z in the A tiles
-        tc_fence_after();
-      }
-      auto gemm1 = [&](int j) {
-        const int b = j & 1;
-        if (j >= 2) {
-          mbar_wait(&s_free[b], ((j >> 1) + 1) & 1);  // swish(j-2) has drained S[b]
-          tc_fence_after();
-        }
-        const uint32_t tmem_s = tmem_base + b * 128;
-        for (int s = 0; s < 2; ++s) {
-          mbar_wait(&w_full[slot], phase);
-          tc_fence_after();
-          const uint32_t w_addr = smem_u32(s_w + slot * 2 * FFN_TILE);
-#pragma unroll
-          for (int t = 0; t < 2; ++t) {
-            const int kb = 2 * s + t;
-#pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_bf16(tmem_s, umma_desc_k_sw128(a_addr + kb * FFN_TILE + k * 32),
-                        umma_desc_k_sw128(w_addr + t * FFN_TILE + k * 32), idesc_g1, (kb | k) != 0);
-          }
-          umma_commit(&w_empty[slot]);
-          if (++slot == FFN_RING) slot = 0, phase ^= 1;
-        }
-        umma_commit(&s_full[b]);
-      };
-      auto gemm2 = [&](int j) {
-        const int b = j & 1;
-        mbar_wait(&h_full[b], (j >> 1) & 1);
-        tc_fence_after();
-        const uint32_t h_addr = smem_u32(s_h + b * 2 * FFN_TILE);
-        for (int kb = 0; kb < 2; ++kb) {
-          mbar_wait(&w_full[slot], phase);
-          tc_fence_after();
-          const uint32_t w_addr = smem_u32(s_w + slot * 2 * FFN_TILE);
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            umma_bf16(tmem_o, umma_desc_k_sw128(h_addr + kb * FFN_TILE + k * 32), umma_desc_k_sw128(w_addr + k * 32),
-                      idesc_g2, 1u);  // always accumulate: O holds the residual
-          umma_commit(&w_empty[slot]);
-          if (++slot == FFN_RING) slot = 0, phase ^= 1;
-        }
-        umma_commit(&h_free[b]);
-      };
-      gemm1(0);
-      if (NCH > 1) gemm1(1);
-      if (!PRE) {
-        mbar_wait(x_loaded, 0);
-        tc_fence_after();
-      }
-      for (int j = 0; j < NCH; ++j) {
-        gemm2(j);
-        if (j + 2 < NCH) gemm1(j + 2);
-      }
-      umma_commit(o_full);
-    }
-  } else if (warp_idx >= 4) {
-    // ============================ compute warps ============================
-    const int ew = warp_idx - 4;
-    const int quad = ew & 3;
-    const int half = ew >> 2;
-    const int r = quad * 32 + lane;  // tile row owned by this thread (with its partner in the other half)
-    const int ct = threadIdx.x - 128;
-    const uint32_t lane_base = ((uint32_t)(quad * 32)) << 16;
-    const int row_g = m0 + r;
-    bool pad = false;
-    if (PRE && p.lens != nullptr && row_g < p.M) {
-      const int b = row_g / p.T;
-      pad = (row_g - b * p.T) >= __ldg(p.lens + b);
-    }
-    if (PRE && p.dw_g != nullptr) {
-      // ---- z = swish(norm(dwconv(g))) -> A tiles of the pre-GEMM (H region = fp32 scratch of one 16-row sub-tile) ----
-      if (p.dw_K == 15) dwconv_a_tiles<15>(p, m0, ct, ew, lane, s_a, s_h);
-      else if (p.dw_K == 31) dwconv_a_tiles<31>(p, m0, ct, ew, lane, s_a, s_h);
-      else dwconv_a_tiles<7>(p, m0, ct, ew, lane, s_a, s_h);
-      fence_proxy_async_smem();
-      mbar_arrive(a_full);
-    }
-    // ---- residual tile -> TMEM O, 64 columns at a time through a coalesced smem slab (the H region is idle) ----
-    {
-      float* slab = reinterpret_cast<float*>(s_h);
-      for (int s = 0; s < 4; ++s) {
-        // coalesced: 16 threads per row (16 B each), 16 rows per pass; all 8 loads in flight before the stores
-        {
-          const int cq = ct & 15;
-          float4 v[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            const int rr = (ct >> 4) + 16 * i;
-            v[i] = ((m0 + rr) < p.M)
-                       ? __ldcg(reinterpret_cast<const float4*>(p.x + (size_t)(m0 + rr) * 256 + s * 64) + cq)
-                       : make_float4(0.f, 0.f, 0.f, 0.f);
-          }
-#pragma unroll
-          for (int i = 0; i < 8; ++i)
-            *reinterpret_cast<float4*>(slab + ((ct >> 4) + 16 * i) * FFN_SLAB_PITCH + cq * 4) = v[i];
-        }
-        named_bar_sync(1, 256);
-        if (half == (s >> 1)) {
-#pragma unroll
-          for (int c = 0; c < 2; ++c) {
-            uint32_t v[32];
-            const int col0 = s * 64 + c * 32;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              float4 t = *reinterpret_cast<const float4*>(slab + r * FFN_SLAB_PITCH + c * 32 + 4 * j);
-              if (PRE && !pad) {
-                const float4 bb = __ldg(reinterpret_cast<const float4*>(p.bp + col0) + j);
-                t.x += bb.x, t.y += bb.y, t.z += bb.z, t.w += bb.w;
-              }
-              v[4 * j] = __float_as_uint(t.x), v[4 * j + 1] = __float_as_uint(t.y);
-              v[4 * j + 2] = __float_as_uint(t.z), v[4 * j + 3] = __float_as_uint(t.w);
-            }
-            tmem_st_32x32b_x32(tmem_o + lane_base + col0, v);
-          }
-          tmem_st_wait();
-        }
-        named_bar_sync(1, 256);
-      }
-      tc_fence_before();
-      mbar_arrive(x_loaded);
-    }
-    float4* scratch = reinterpret_cast<float4*>(smem + 128 * FFN_XS_PITCH * 4);  // [2][256] exchange slots (ring region)
-    if (PRE) {
-      // ---- y = LN(x_mid) -> A tiles (bf16, 128B swizzle); x_mid stays in TMEM O ----
-      mbar_wait(pre_full, 0);
-      tc_fence_after();
-      float4* sc = reinterpret_cast<float4*>(s_h);  // H region is idle until the first swish
-      FfnStat st{0.f, 0.f, 0.f};
-#pragma unroll 1
-      for (int c = 0; c < 4; ++c) {
-        uint32_t ro[32];
-        tmem_ld_32x32b_x32(tmem_o + lane_base + half * 128 + c * 32, ro);
-        tmem_ld_wait();
-        float v[32];
-#pragma unroll
-        for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(ro[j]);
-        ffn_add_chunk(st, v);
-      }
-      ffn_exchange(st, sc, r, half, 2);
-      const float mean = st.mean;
-      const float rstd = rsqrtf(st.m2 * (1.0f / 256.0f) + p.eps);
-#pragma unroll 1
-      for (int c = 0; c < 4; ++c) {
-        const int cc = half * 128 + c * 32;
-        uint32_t ro[32];
-        tmem_ld_32x32b_x32(tmem_o + lane_base + cc, ro);
-        tmem_ld_wait();
-        uint32_t pk[16];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const float4 gg = __ldg(reinterpret_cast<const float4*>(p.gp + cc) + j);
-          const float4 bb = __ldg(reinterpret_cast<const float4*>(p.bpn + cc) + j);
-          float y0 = (__uint_as_float(ro[4 * j + 0]) - mean) * rstd * gg.x + bb.x;
-          float y1 = (__uint_as_float(ro[4 * j + 1]) - mean) * rstd * gg.y + bb.y;
-          float y2 = (__uint_as_float(ro[4 * j + 2]) - mean) * rstd * gg.z + bb.z;
-          float y3 = (__uint_as_float(ro[4 * j + 3]) - mean) * rstd * gg.w + bb.w;
-          if (p.pre_ys != nullptr) {
-            ro[4 * j + 0] = __float_as_uint(y0), ro[4 * j + 1] = __float_as_uint(y1);
-            ro[4 * j + 2] = __float_as_uint(y2), ro[4 * j + 3] = __float_as_uint(y3);
-            const float4 as = __ldg(reinterpret_cast<const float4*>(p.pre_ys + cc) + j);
-            const float4 ab = __ldg(reinterpret_cast<const float4*>(p.pre_yb + cc) + j);
-            y0 = fmaf(as.x, y0, ab.x), y1 = fmaf(as.y, y1, ab.y), y2 = fmaf(as.z, y2, ab.z), y3 = fmaf(as.w, y3, ab.w);
-          }
-          pk[2 * j] = pack_bf16x2(y0, y1);
-          pk[2 * j + 1] = pack_bf16x2(y2, y3);
-        }
-        if (p.pre_ys != nullptr) tmem_st_32x32b_x32(tmem_o + lane_base + cc, ro);  // the normalised row is the new residual
-        // columns cc .. cc+31 live in k-block cc/64, 16-byte chunks (cc%64)/8 .. +3
-        uint8_t* atile = s_a + (cc >> 6) * FFN_TILE + r * 128;
-        const int ch0 = (cc & 63) >> 3;
-#pragma unroll
-        for (int q4 = 0; q4 < 4; ++q4)
-          *reinterpret_cast<uint4*>(atile + (((ch0 + q4) ^ (r & 7)) << 4)) =
-              make_uint4(pk[4 * q4], pk[4 * q4 + 1], pk[4 * q4 + 2], pk[4 * q4 + 3]);
-      }
-      if (p.pre_ys != nullptr) tmem_st_wait();
-      tc_fence_before();
-      fence_proxy_async_smem();
-      mbar_arrive(a_ready);
-    }
-    // ---- swish between the two GEMMs ----
-    for (int j = 0; j < NCH; ++j) {
-      const int b = j & 1;
-      mbar_wait(&s_full[b], (j >> 1) & 1);
-      tc_fence_after();
-      if (j >= 2) mbar_wait(&h_free[b], ((j >> 1) + 1) & 1);  // GEMM2(j-2) has consumed H[b]
-      uint8_t* htile = s_h + b * 2 * FFN_TILE + half * FFN_TILE + r * 128;
-      const float* b1p = p.b1 + j * 128 + half * 64;
-      uint32_t rr2[2][32];
-      tmem_ld_32x32b_x32(tmem_base + lane_base + b * 128 + half * 64, rr2[0]);
-      tmem_ld_32x32b_x32(tmem_base + lane_base + b * 128 + half * 64 + 32, rr2[1]);
-      tmem_ld_wait();
-#pragma unroll
-      for (int c = 0; c < 2; ++c) {
-        const uint32_t(&rr)[32] = rr2[c];
-        uint32_t pk[16];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const float4 bv = __ldg(reinterpret_cast<const float4*>(b1p + c * 32) + i);
-          pk[2 * i] = pack_bf16x2(swish_f(__uint_as_float(rr[4 * i]) + bv.x), swish_f(__uint_as_float(rr[4 * i + 1]) + bv.y));
-          pk[2 * i + 1] =
-              pack_bf16x2(swish_f(__uint_as_float(rr[4 * i + 2]) + bv.z), swish_f(__uint_as_float(rr[4 * i + 3]) + bv.w));
-        }
-#pragma unroll
-        for (int q4 = 0; q4 < 4; ++q4) {
-          const int chunk = c * 4 + q4;
-          *reinterpret_cast<uint4*>(htile + ((chunk ^ (r & 7)) << 4)) =
-              make_uint4(pk[4 * q4], pk[4 * q4 + 1], pk[4 * q4 + 2], pk[4 * q4 + 3]);
-        }
-      }
-      tc_fence_before();
-      mbar_arrive(&s_free[b]);
-      fence_proxy_async_smem();
-      mbar_arrive(&h_full[b]);
-    }
-    // ---- epilogue: x_new = O + b2s, LayerNorm(s), coalesced write-out through an fp32 staging tile ----
-    mbar_wait(o_full, 0);
-    tc_fence_after();
-    float* xs = reinterpret_cast<float*>(smem);  // [128][FFN_XS_PITCH]  (A + H + part of the ring: all idle now)
-    float2* stats = reinterpret_cast<float2*>(scratch + 512);  // [128] (mean, rstd) of the last LN
-    float* prm = reinterpret_cast<float*>(stats + 128);        // [5][256]: b2s, g1, bn1, g2, bn2
-    prm[ct] = __ldg(p.b2s + ct);
-    prm[256 + ct] = __ldg(p.g1 + ct);
-    prm[512 + ct] = __ldg(p.bn1 + ct);
-    if (p.g2 != nullptr) {
-      prm[768 + ct] = __ldg(p.g2 + ct);
-      prm[1024 + ct] = __ldg(p.bn2 + ct);
-    }
-    named_bar_sync(1, 256);
-    float* xrow = xs + r * FFN_XS_PITCH;
-    FfnStat st{0.f, 0.f, 0.f};
-#pragma unroll 1
-    for (int c = 0; c < 4; c += 2) {
-      uint32_t ro[2][32];
-      tmem_ld_32x32b_x32(tmem_o + lane_base + half * 128 + c * 32, ro[0]);
-      tmem_ld_32x32b_x32(tmem_o + lane_base + half * 128 + c * 32 + 32, ro[1]);
-      tmem_ld_wait();
-#pragma unroll
-      for (int u = 0; u < 2; ++u) {
-        const int cc = half * 128 + (c + u) * 32;
-        float v[32];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const float4 bb = *reinterpret_cast<const float4*>(prm + cc + 4 * j);
-          v[4 * j + 0] = __uint_as_float(ro[u][4 * j + 0]) + bb.x;
-          v[4 * j + 1] = __uint_as_float(ro[u][4 * j + 1]) + bb.y;
-          v[4 * j + 2] = __uint_as_float(ro[u][4 * j + 2]) + bb.z;
-          v[4 * j + 3] = __uint_as_float(ro[u][4 * j + 3]) + bb.w;
-          *reinterpret_cast<float4*>(xrow + cc + 4 * j) = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-        }
-        ffn_add_chunk(st, v);
-      }
-    }
-    ffn_exchange(st, scratch, r, half, 2);
-    float mean = st.mean;
-    float rstd = rsqrtf(st.m2 * (1.0f / 256.0f) + p.eps);
-    if (p.g2 != nullptr) {
-      FfnStat s2{0.f, 0.f, 0.f};
-#pragma unroll 1
-      for (int c = 0; c < 4; ++c) {
-        const int cc = half * 128 + c * 32;
-        float v[32];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const float4 xo = *reinterpret_cast<const float4*>(xrow + cc + 4 * j);
-          const float4 gg = *reinterpret_cast<const float4*>(prm + 256 + cc + 4 * j);
-          const float4 bb = *reinterpret_cast<const float4*>(prm + 512 + cc + 4 * j);
-          v[4 * j + 0] = (xo.x - mean) * rstd * gg.x + bb.x;
-          v[4 * j + 1] = (xo.y - mean) * rstd * gg.y + bb.y;
-          v[4 * j + 2] = (xo.z - mean) * rstd * gg.z + bb.z;
-          v[4 * j + 3] = (xo.w - mean) * rstd * gg.w + bb.w;
-          *reinterpret_cast<float4*>(xrow + cc + 4 * j) = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-        }
-        ffn_add_chunk(s2, v);
-      }
-      if (p.y_affine) {
-        mean = 0.f, rstd = 1.f;
-      } else {
-        ffn_exchange(s2, scratch + 256, r, half, 3);
-        mean = s2.mean;
-        rstd = rsqrtf(s2.m2 * (1.0f / 256.0f) + p.eps);
-      }
-    }
-    if (half == 0) stats[r] = make_float2(mean, rstd);
-    named_bar_sync(1, 256);
-    // coalesced write-out of x (fp32, 16 B per lane) and y = LN(x) (bf16, 8 B per lane)
-    const float* gl = prm + (p.g2 ? 768 : 256);
-    const float* bl = prm + (p.g2 ? 1024 : 512);
-    float4 gv[2], bv[2];
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-      gv[i] = *reinterpret_cast<const float4*>(gl + 4 * lane + 128 * i);
-      bv[i] = *reinterpret_cast<const float4*>(bl + 4 * lane + 128 * i);
-    }
-    for (int row = ew; row < 128; row += 8) {
-      if (m0 + row >= p.M) break;
-      const float2 ms = stats[row];
-      const float4* src = reinterpret_cast<const float4*>(xs + row * FFN_XS_PITCH);
-      float4* dx = reinterpret_cast<float4*>(p.x + (size_t)(m0 + row) * 256);
-      uint2* dy = reinterpret_cast<uint2*>(p.y + (size_t)(m0 + row) * 256);
-      bool zero_y = false;
-      if (p.ylens != nullptr) {
-        const int bb = (m0 + row) / p.T;
-        zero_y = (m0 + row - bb * p.T) >= __ldg(p.ylens + bb);
-      }
-#pragma unroll
-      for (int i = 0; i < 2; ++i) {
-        const float4 v = src[lane + 32 * i];
-        dx[lane + 32 * i] = v;
-        if (zero_y) {
-          dy[lane + 32 * i] = make_uint2(0u, 0u);
-          continue;
-        }
-        const float y0 = (v.x - ms.x) * ms.y * gv[i].x + bv[i].x;
-        const float y1 = (v.y - ms.x) * ms.y * gv[i].y + bv[i].y;
-        const float y2 = (v.z - ms.x) * ms.y * gv[i].z + bv[i].z;
-        const float y3 = (v.w - ms.x) * ms.y * gv[i].w + bv[i].w;
-        dy[lane + 32 * i] = make_uint2(pack_bf16x2(y0, y1), pack_bf16x2(y2, y3));
-      }
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp_idx == 2) {
-    tc_fence_after();
-    tmem_dealloc<512>(tmem_base);
-  }
-}
-
-
-// =====================================================================================================================
-// Split variant: one 128-row tile is shared by a 2-CTA thread-block cluster. CTA `rank` owns hidden chunks
-// [rank*NCH/2, (rank+1)*NCH/2): it runs GEMM1 / Swish / GEMM2 over its half of the 2048-wide hidden dimension and ends
-// with a PARTIAL output tile O_rank in TMEM. The two partials are reduced through distributed shared memory: each CTA
-// stages its tile in shared memory, bulk-copies the 64 rows the PEER finalises into the peer's receive buffer
-// (cp.async.bulk.shared::cluster, completion on the peer's mbarrier) and finalises its own 64 rows warp-per-row
-// (partial + peer partial + b2s [+ residual from global memory] -> LayerNorm(s) -> coalesced x / y stores).
-// One launch therefore covers 2 x ceil(M/128) CTAs (124 at C2 instead of 62 on 148 SMs).
-//  * plain mode: no residual preload at all -- x is added in the final pass from global memory (coalesced).
-//  * chained mode: both CTAs preload x and run the small pre-GEMM + LayerNorm redundantly (1/16 of the FLOPs); rank 1
-//    then discards the residual by starting its GEMM2 chain with accumulate = 0, so x_mid is counted once.
-//  * Swish stage on two teams of 8 warps (even / odd chunks), S released right after the TMEM load, GEMM1(j+2) issued
-//    BEFORE GEMM2(j): the tensor pipe always has the next GEMM1 queued while a team is still in its Swish.
-//  * weight tiles are requested before griddepcontrol.wait (they do not depend on the predecessor kernel).
-// Same arithmetic as fused_ffn_kernel except for the fp32 summation order of the two hidden halves and a two-pass
-// (instead of chunk-merged) LayerNorm variance.
 constexpr int FS_THREADS = 640;                     // warps 0..3 control, 4..11 team 0, 12..19 team 1
 constexpr int FS_PITCH = 260;                       // fp32 staging pitch
 constexpr int FS_SMEM_XS = 0;                       // [128][260] fp32: own partial tile
@@ -1163,28 +596,27 @@ int ffn_split_mode() {
   int v = g_ffn_split.load(std::memory_order_relaxed);
   if (v < 0) {
     const char* e = getenv("PPASR_B200_FFN_SPLIT");
-    v = (e != nullptr && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 1;
+    v = (e != nullptr && std::strcmp(e, "2") == 0) ? 2 : 1;
     g_ffn_split.store(v, std::memory_order_relaxed);
   }
   return v;
 }
-void set_ffn_split_mode(int mode) { g_ffn_split.store(mode < 0 || mode > 2 ? 1 : mode, std::memory_order_relaxed); }
+bool set_ffn_split_mode(int mode) {
+  if (mode != 1 && mode != 2) return false;
+  g_ffn_split.store(mode, std::memory_order_relaxed);
+  return true;
+}
 
 cudaError_t launch_fused_ffn(const CUtensorMap& tm_a, const CUtensorMap* tm_wp, const CUtensorMap& tm_w1,
                              const CUtensorMap& tm_w2, int M, int FF, float* x, __nv_bfloat16* y, const float* b1,
                              const float* b2s, const float* g1, const float* bn1, const float* g2, const float* bn2,
                              float eps, const float* bp, const float* gp, const float* bpn, const int* lens, int T,
-                             cudaStream_t st, int y_affine, const int* ylens, const float* pre_ys, const float* pre_yb,
-                             const FfnDw* dw) {
-  if (FF % 128 != 0 || M <= 0) return cudaErrorInvalidValue;
+                             cudaStream_t st, int y_affine, const int* ylens, const float* pre_ys, const float* pre_yb) {
+  if (FF % 128 != 0 || FF < 256 || M <= 0) return cudaErrorInvalidValue;  // the pipeline starts with GEMM1(0) and GEMM1(1)
   static std::once_flag once;
   static cudaError_t cfg_err = cudaSuccess;
   std::call_once(once, [] {
-    cudaError_t e = cudaFuncSetAttribute(fused_ffn_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, FFN_SMEM_TOTAL);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(fused_ffn_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FFN_SMEM_TOTAL);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(fused_ffn_split_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FFN_SMEM_TOTAL);
+    cudaError_t e = cudaFuncSetAttribute(fused_ffn_split_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FFN_SMEM_TOTAL);
     if (e == cudaSuccess)
       e = cudaFuncSetAttribute(fused_ffn_split_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FFN_SMEM_TOTAL);
     if (e == cudaSuccess)
@@ -1199,27 +631,17 @@ cudaError_t launch_fused_ffn(const CUtensorMap& tm_a, const CUtensorMap* tm_wp, 
   p.g1 = g1, p.bn1 = bn1, p.g2 = g2, p.bn2 = bn2, p.eps = eps;
   p.bp = bp, p.gp = gp, p.bpn = bpn, p.lens = lens, p.T = T;
   p.y_affine = y_affine, p.ylens = ylens, p.pre_ys = pre_ys, p.pre_yb = pre_yb;
-  p.dw_g = nullptr, p.dw_w = p.dw_b = p.dw_pad = p.dw_ng = p.dw_nb = nullptr, p.dw_K = 0, p.dw_ln = 0;
-  if (dw != nullptr && tm_wp != nullptr) {
-    if (dw->K != 7 && dw->K != 15 && dw->K != 31) return cudaErrorInvalidValue;
-    p.dw_g = dw->g, p.dw_w = dw->w, p.dw_b = dw->bias, p.dw_pad = dw->pad_left, p.dw_ng = dw->ng, p.dw_nb = dw->nb;
-    p.dw_K = dw->K, p.dw_ln = dw->layer_norm;
-  }
   const int grid = (M + 127) / 128;
   cudaError_t le;
-  const int mode = ffn_split_mode();
-  if (mode == 1 && p.dw_g == nullptr && p.nchunks >= 4 && (p.nchunks & 1) == 0) {
-    // 2-CTA cluster per row tile, hidden dimension split over the pair
+  if (ffn_split_mode() == 1 && p.nchunks >= 4 && (p.nchunks & 1) == 0) {
+    // 2-CTA cluster per row tile, hidden dimension split over the pair (each half needs at least two chunks)
     if (tm_wp != nullptr)
       le = launch_pdl_cluster(fused_ffn_split_kernel<true, true>, dim3(2 * grid), dim3(FS_THREADS), (size_t)FFN_SMEM_TOTAL, st, 2u,
                               tm_a, *tm_wp, tm_w1, tm_w2, p);
     else
       le = launch_pdl_cluster(fused_ffn_split_kernel<false, true>, dim3(2 * grid), dim3(FS_THREADS), (size_t)FFN_SMEM_TOTAL, st, 2u,
                               tm_a, tm_w1, tm_w1, tm_w2, p);
-    count_launch();
-    return le != cudaSuccess ? le : cudaGetLastError();
-  }
-  if (mode == 2 && p.dw_g == nullptr && p.nchunks >= 2) {
+  } else {
     // the two-team pipeline on one CTA per row tile (least SM time per launch: several batches in flight)
     if (tm_wp != nullptr)
       le = launch_pdl(fused_ffn_split_kernel<true, false>, dim3(grid), dim3(FS_THREADS), (size_t)FFN_SMEM_TOTAL, st, tm_a, *tm_wp,
@@ -1227,13 +649,7 @@ cudaError_t launch_fused_ffn(const CUtensorMap& tm_a, const CUtensorMap* tm_wp, 
     else
       le = launch_pdl(fused_ffn_split_kernel<false, false>, dim3(grid), dim3(FS_THREADS), (size_t)FFN_SMEM_TOTAL, st, tm_a, tm_w1,
                       tm_w1, tm_w2, p);
-    count_launch();
-    return le != cudaSuccess ? le : cudaGetLastError();
   }
-  if (tm_wp != nullptr)
-    le = launch_pdl(fused_ffn_kernel<true>, dim3(grid), dim3(FFN_THREADS), (size_t)FFN_SMEM_TOTAL, st, tm_a, *tm_wp, tm_w1, tm_w2, p);
-  else
-    le = launch_pdl(fused_ffn_kernel<false>, dim3(grid), dim3(FFN_THREADS), (size_t)FFN_SMEM_TOTAL, st, tm_a, tm_w1, tm_w1, tm_w2, p);
   count_launch();
   return le != cudaSuccess ? le : cudaGetLastError();
 }

@@ -459,10 +459,9 @@ struct EpiGLU {
 //   q2[b,h,t,64:128] = q + pos_bias_v[h]
 //   kk[b,h,tk,0:64 ] = k                      (tk = kofs + t : KV-cache append position)
 //   vt[b,h,d,tk]     = v  (transposed so P.V^T is a K-major UMMA B operand)
-template <int BLOCK_N, int EPI_WARPS = 16, int MIN_BLOCKS = 1>
+template <int BLOCK_N>
 struct EpiQKV {
-  static constexpr int kEpiWarps = EPI_WARPS;  // 16: four column parts, one 32-column chunk per warp and 128-wide tile
-  static constexpr int kMinBlocks = MIN_BLOCKS;
+  static constexpr int kEpiWarps = 16;  // four column parts, one 32-column chunk per warp and 128-wide tile
   __nv_bfloat16* q2;
   __nv_bfloat16* kk;
   __nv_bfloat16* vt;
@@ -488,7 +487,7 @@ struct EpiQKV {
     }
     const int kb = slots ? __ldg(slots + b) : b;               // cache slot of the K / V rows
     const int kofs = kofs_b ? __ldg(kofs_b + b) : this->kofs;  // shadows the member on purpose
-    epi_for_chunks<BLOCK_N, EPI_WARPS / 4>(taddr, half, [&](int cc, const uint32_t(&r)[32]) {
+    epi_for_chunks<BLOCK_N, kEpiWarps / 4>(taddr, half, [&](int cc, const uint32_t(&r)[32]) {
       const int col = n0 + cc;
       if (row >= M || col >= 3 * D) return;
       const int which = col / D;
@@ -752,23 +751,12 @@ template <class Epi>
 struct EpiWarps<Epi, decltype((void)Epi::kEpiWarps)> {
   static constexpr int value = Epi::kEpiWarps;
 };
-// CTAs of this instantiation that may share an SM (register cap via __launch_bounds__, grid = min(tiles, kMinBlocks * SMs)).
-// A latency-bound GEMM that leaves room (few ring stages, <= 256 TMEM columns, <= 85 registers at 384 threads) lets a second
-// CTA -- of the same launch, or of another stream's kernel in the throughput pipeline -- use the SM while it waits.
-template <class Epi, class = void>
-struct EpiMinBlocks {
-  static constexpr int value = 1;
-};
-template <class Epi>
-struct EpiMinBlocks<Epi, decltype((void)Epi::kMinBlocks)> {
-  static constexpr int value = Epi::kMinBlocks;
-};
 
 // ------------------------------------------------------------------------------------------------
 // The kernel
 // ------------------------------------------------------------------------------------------------
 template <int BLOCK_N, int STAGES, bool CONV, class Epi>
-__global__ void __launch_bounds__(128 + EpiWarps<Epi>::value * 32, EpiMinBlocks<Epi>::value)
+__global__ void __launch_bounds__(128 + EpiWarps<Epi>::value * 32, 1)
 gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                          const GemmShape shape, const Epi epi) {
   using SM = GemmSmem<BLOCK_N, STAGES>;
@@ -941,8 +929,7 @@ inline cudaError_t launch_gemm(const CUtensorMap& tmap_a, const CUtensorMap& tma
   }
   const int num_tiles = shape.num_m_tiles * shape.num_n_tiles;
   if (num_tiles <= 0) return cudaSuccess;
-  const int slots = num_sms * EpiMinBlocks<Epi>::value;
-  const int grid = num_tiles < slots ? num_tiles : slots;
+  const int grid = num_tiles < num_sms ? num_tiles : num_sms;
   cudaError_t le = launch_pdl(kern, dim3(grid), dim3(128 + EpiWarps<Epi>::value * 32), (size_t)SM::TOTAL, stream, tmap_a, tmap_b, shape, epi);
   count_launch();
   return le != cudaSuccess ? le : cudaGetLastError();

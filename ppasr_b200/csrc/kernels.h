@@ -53,42 +53,29 @@ cudaError_t launch_ctc_collapse(const int* idx, const float* maxp, int B, int T,
                                 int* ids_out, int ld_out, int* out_len, float* score, float* score_sum,
                                 int* score_cnt, cudaStream_t st);
 
-// depthwise-conv stage folded into the chained fused FFN kernel (causal conv module only)
-struct FfnDw {
-  const __nv_bfloat16* g;  // [M, 256] GLU output
-  const float *w, *bias, *pad_left, *ng, *nb;
-  int K, layer_norm;
-};
-
 // Fused feed-forward block (fused_ffn.cu): x += W2s swish(W1 y + b1) + b2s with trailing LayerNorm(s); optional
 // chained pre-GEMM (tm_wp != null): x += mask (Wp z + bp), y = LN(x; gp, bpn) first (tm_a is then the z tile map).
+// FF must be a multiple of 128 and at least 256 (cudaErrorInvalidValue otherwise).
 cudaError_t launch_fused_ffn(const CUtensorMap& tm_a, const CUtensorMap* tm_wp, const CUtensorMap& tm_w1,
                              const CUtensorMap& tm_w2, int M, int FF, float* x, __nv_bfloat16* y, const float* b1,
                              const float* b2s, const float* g1, const float* bn1, const float* g2, const float* bn2,
                              float eps, const float* bp, const float* gp, const float* bpn, const int* lens, int T,
                              cudaStream_t st, int y_affine = 0, const int* ylens = nullptr, const float* pre_ys = nullptr,
-                             const float* pre_yb = nullptr, const FfnDw* dw = nullptr);
+                             const float* pre_yb = nullptr);
 
-// fused_ffn variant (process-wide; env PPASR_B200_FFN_SPLIT=0/1/2 or ppasr_b200_set_option(ctx, "ffn_split", v)):
+// fused_ffn variant (process-wide; env PPASR_B200_FFN_SPLIT=1/2 or ppasr_b200_set_option(ctx, "ffn_split", v)):
 //   1 (default) = 2-CTA cluster per row tile, hidden dimension split over the pair, distributed-shared-memory reduction
-//                 (2 x ceil(M/128) CTAs per launch: shortest single-launch latency);
-//   2 = the same two-team pipeline on one CTA per row tile (least SM time per launch; the throughput pipeline uses it);
-//   0 = the round-1 kernel (one CTA per row tile, single Swish team; still used for the opt-in fused_dwconv mode).
+//                 (2 x ceil(M/128) CTAs per launch: shortest single-launch latency); FF / 128 must be even and >= 4,
+//                 otherwise the launch falls back to mode 2;
+//   2 = the same two-team pipeline on one CTA per row tile (least SM time per launch; the throughput pipeline uses it).
+// set_ffn_split_mode returns false and keeps the current mode for any other value.
 int ffn_split_mode();
-void set_ffn_split_mode(int mode);
+bool set_ffn_split_mode(int mode);
 
-// Fused attention out-projection + residual + norm_conv + pointwise_conv1 + GLU (fused_attn_out.cu). Variant (process-wide,
-// env PPASR_B200_ATTN_OUT_V2 / set_option "attn_out_v2"): 1 (default) = no serial residual preload, 0 = round-1 kernel.
-int attn_out_variant();
-void set_attn_out_variant(int v);
+// Fused attention out-projection + residual + norm_conv + pointwise_conv1 + GLU (fused_attn_out.cu)
 cudaError_t launch_fused_attn_out(const CUtensorMap& tm_att, const CUtensorMap& tm_wo, const CUtensorMap& tm_wpw1, int M,
                                   float* x, __nv_bfloat16* g, const float* bo, const float* ln_g, const float* ln_b,
                                   const float* bpw1, const int* lens, int T, float eps, cudaStream_t st);
-
-// Fused CMVN + conv1 + ReLU + conv2 + ReLU (conv_front.cu); tmap_w2 = conv2 weights [256, 9*256] K-major, box {64, 256}
-cudaError_t launch_conv_front(const CUtensorMap& tmap_w2, const float* feats, const float* mean, const float* istd,
-                              const float* w1, const float* b1, const float* b2, __nv_bfloat16* out, int B, int T, int F,
-                              int Th, int FH, int Tout, int Fout, int num_sms, cudaStream_t st);
 
 // Squeezeformer time reduction, depthwise part (squeezeformer/time_reduction.py:61-84 conv1d k5 s2 pad3, :183-206 stream
 // k1 s2): out[b, tr, c] = bias[c] + sum_k w[c, k] * xm[b, 2 tr + k - pad, c] with xm = x zeroed at t >= lens[b] -> bf16

@@ -75,8 +75,8 @@ int ppasr_b200_set_pdl(int32_t enable) {
   return PPASR_OK;
 }
 
-int ppasr_b200_set_ffn_split(int32_t enable) {
-  set_ffn_split_mode(enable);
+int ppasr_b200_set_ffn_split(int32_t mode) {
+  PPASR_REQUIRE(set_ffn_split_mode(mode), "ffn_split must be 1 or 2");
   return PPASR_OK;
 }
 int ppasr_b200_get_ffn_split(void) { return ffn_split_mode(); }
@@ -249,7 +249,7 @@ int ppasr_b200_op_fused_ffn(const void* y_bf16, const void* w1_bf16, const void*
                             const float* b1, const float* b2s, const float* g1, const float* bn1, const float* g2,
                             const float* bn2, int32_t M, int32_t FF, float eps, void* stream) {
   PPASR_REQUIRE(y_bf16 && w1_bf16 && w2s_bf16 && x && y_out && b1 && b2s && g1 && bn1, "null pointer");
-  PPASR_REQUIRE(M > 0 && FF > 0 && FF % 128 == 0, "FF must be a positive multiple of 128");
+  PPASR_REQUIRE(M > 0 && FF >= 256 && FF % 128 == 0, "FF must be a multiple of 128 and at least 256");
   std::string err;
   CUtensorMap ta, t1, t2;
   if (!make_tmap_2d(&ta, y_bf16, 256, (uint64_t)M, 512, 128, &err) ||

@@ -118,7 +118,7 @@ struct ppasr_b200_ctx {
   // weight tensor maps (B operands)
   CUtensorMap tm_conv2_w, tm_emb_w, tm_ctc_w, tm_pos;
   struct LayerMaps {
-    CUtensorMap ffm_w1, ffm_w2, ff_w1, ff_w2, wqkv, wqkv_wide, wo, pw1, pw2, ffm_w1_128, ff_w1_128, ffm_w2s, ff_w2s;
+    CUtensorMap ffm_w1, ffm_w2, ff_w1, ff_w2, wqkv, wo, pw1, pw2, ffm_w1_128, ff_w1_128, ffm_w2s, ff_w2s;
   };
   std::vector<LayerMaps> lmaps;
   // ---- Squeezeformer (model_type 1; squeezeformer/encoder.py) ----
@@ -190,16 +190,7 @@ struct ppasr_b200_ctx {
   bool fused_ffn = true;
   bool fused_attn_out = true;
   bool conv1_tc = true;   // conv1 on the tensor cores (conv1_tc.cu); 0 = the CUDA-core kernel (env PPASR_B200_CONV1_TC / option "conv1_tc")
-  bool qkv_co = false;    // QKV GEMM sized for two CTAs per SM (experiment switch, env PPASR_B200_QKV_CO / option "qkv_co")
-  bool qkv_wide = false;  // QKV GEMM with 128 x 256 tiles (experiment switch, env PPASR_B200_QKV_WIDE / option "qkv_wide")
-  // causal models: depthwise conv + norm + swish computed in the chained FFN kernel's prologue. Bit-identical to the
-  // stand-alone kernel but slower (2.53 vs 2.20 ms single stream, 1.45 vs 1.36 ms in throughput mode at C2): the
-  // prologue (~27 us on 62 CTAs, before any MMA can start) costs more SM time than the 13 us grid-wide kernel. Opt-in.
-  bool fused_dwconv = false;
-  // conv1 computed inside the conv2 GEMM's A producer (conv_front.cu). Bit-identical to the two-kernel path but slower
-  // on B200 (382 us vs 145 + 145 us at C2): the producers' LDS/STS traffic shares the 128 B/clk shared-memory data pipe
-  // with the tensor core's operand reads (ncu: lsu 57 % + tc 20 % of the pipe), so it is opt-in.
-  int fused_conv = 2;  // 2 (default): conv_front_tc (tensor-core conv1 producer inside the conv2 GEMM), 0: conv1 + conv2 GEMM, 1: conv_front.cu (CUDA-core producer); env PPASR_B200_FUSED_CONV
+  int fused_conv = 2;  // 2 (default): conv_front_tc (tensor-core conv1 producer inside the conv2 GEMM), 0: conv1 + conv2 GEMM; env PPASR_B200_FUSED_CONV
   bool host_sync = true;  // ctc_* with host outputs synchronise the stream before returning
   // valid-length staging (pinned: the H2D copy may be part of a captured CUDA graph and is re-read at every replay)
   int* h_vlen = nullptr;
@@ -334,11 +325,11 @@ int ppasr_b200_create(const ppasr_b200_config* cfg, ppasr_b200_ctx** out) {
   auto* c = new ppasr_b200_ctx();
   c->cfg = *cfg;
   c->layer_k.assign(cfg->n_layers, cfg->conv_kernel);
-  if (const char* e = std::getenv("PPASR_B200_FUSED_DWCONV")) c->fused_dwconv = std::atoi(e) != 0;  // A/B switch for bench runs
-  if (const char* e = std::getenv("PPASR_B200_QKV_WIDE")) c->qkv_wide = std::atoi(e) != 0;
-  if (const char* e = std::getenv("PPASR_B200_QKV_CO")) c->qkv_co = std::atoi(e) != 0;
   if (const char* e = std::getenv("PPASR_B200_CONV1_TC")) c->conv1_tc = std::atoi(e) != 0;
-  if (const char* e = std::getenv("PPASR_B200_FUSED_CONV")) c->fused_conv = std::atoi(e);
+  if (const char* e = std::getenv("PPASR_B200_FUSED_CONV")) {  // an invalid value keeps the default
+    const int v = std::atoi(e);
+    if (v == 0 || v == 2) c->fused_conv = v;
+  }
   if (cfg->model_type == 3) {
     c->eff_stride_idx = cfg->stride_layer_idx;
     c->eff_group_mask = (unsigned)cfg->group_layer_mask;
@@ -625,7 +616,6 @@ int ppasr_b200_finalize(ppasr_b200_ctx* c) {
               make_tmap_2d(&m.ff_w1_128, w.ff_w1, D, FF, (uint64_t)D * 2, 128, &err) &&
               make_tmap_2d(&m.ff_w2, w.ff_w2, FF, D, (uint64_t)FF * 2, BN_WIDE, &err) &&
               make_tmap_2d(&m.wqkv, w.wqkv, D, 3 * D, (uint64_t)D * 2, BN_NARROW, &err) &&
-              make_tmap_2d(&m.wqkv_wide, w.wqkv, D, 3 * D, (uint64_t)D * 2, BN_WIDE, &err) &&
               make_tmap_2d(&m.wo, w.wo, D, D, (uint64_t)D * 2, BN_WIDE, &err) &&
               make_tmap_2d(&m.pw1, w.pw1, D, 2 * D, (uint64_t)D * 2, BN_WIDE, &err) &&
               make_tmap_2d(&m.pw2, w.pw2, D, D, (uint64_t)D * 2, BN_WIDE, &err);
@@ -835,11 +825,6 @@ int run_subsampling_convs(ppasr_b200_ctx* c, cudaStream_t st) {
     PROF(PC_CONV_FRONT);
     PPASR_CUDA_CHECK(launch_conv_front_tc(c->tm_conv2_w, p.feats, c->cmvn_mean, c->cmvn_istd, c->conv1_w, c->conv1_b, c->conv2_b,
                                           p.c2, p.B, p.T, cfg.feat_dim, p.T1, c->F1, p.Th, c->FH, p.Tp, c->F2, c->sms, st));
-  } else if (c->fused_conv == 1 && D == 256 && c->FH == 20) {  // patch geometry of conv_front.cu assumes feat_dim 80 (pitch 20)
-    // CMVN + conv1 + ReLU + conv2 + ReLU in one kernel (conv_front.cu) -> c2 [M, F2*D]
-    PROF(PC_CONV_FRONT);
-    PPASR_CUDA_CHECK(launch_conv_front(c->tm_conv2_w, p.feats, c->cmvn_mean, c->cmvn_istd, c->conv1_w, c->conv1_b, c->conv2_b,
-                                       p.c2, p.B, p.T, cfg.feat_dim, p.Th, c->FH, p.Tp, c->F2, c->sms, st));
   } else {
     // CMVN + conv1 + ReLU -> stride-phase images
     { PROF(PC_CONV1);
@@ -905,21 +890,8 @@ int run_encoder(ppasr_b200_ctx* c, cudaStream_t st, bool chunk) {
       AttnParams ap{};
       ap.B = p.B, ap.H = H, ap.T1 = p.Tp, ap.D = D, ap.pos_col0 = l * D, ap.out = p.att, ap.q_rows_per_bh = p.Tp;
       if (!chunk) {
-        if (c->qkv_wide) {  // 128 x 256 tiles: one tile = the q, k or v third of a row tile (186 tiles instead of 372 at C2)
-          EpiQKV<BN_WIDE> e{p.q2, p.kk, p.vt, w.bqkv, w.pos_u, w.pos_v, M, p.Tp, H, p.Tp, p.Tkp, 0};
-          PROF(PC_QKV);
-          PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_y, m.wqkv_wide, M, 3 * D, D, e, st)));
-        } else {
-          if (c->qkv_co) {  // two CTAs per SM: 3-stage ring, 8 epilogue warps, <= 85 registers
-            EpiQKV<BN_NARROW, 8, 2> e{p.q2, p.kk, p.vt, w.bqkv, w.pos_u, w.pos_v, M, p.Tp, H, p.Tp, p.Tkp, 0};
-            PROF(PC_QKV);
-            PPASR_CUDA_CHECK((gemm<BN_NARROW, 3>(c, p.tm_y, m.wqkv, M, 3 * D, D, e, st)));
-          } else {
-            EpiQKV<BN_NARROW> e{p.q2, p.kk, p.vt, w.bqkv, w.pos_u, w.pos_v, M, p.Tp, H, p.Tp, p.Tkp, 0};
-            PROF(PC_QKV);
-            PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, M, 3 * D, D, e, st)));
-          }
-        }
+        EpiQKV<BN_NARROW> e{p.q2, p.kk, p.vt, w.bqkv, w.pos_u, w.pos_v, M, p.Tp, H, p.Tp, p.Tkp, 0};
+        { PROF(PC_QKV); PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, M, 3 * D, D, e, st))); }
         ap.T2 = p.Tp, ap.k_rows_per_bh = p.Tp, ap.k_row0 = 0, ap.pos_row0 = 0, ap.klens = p.vlen;
         { PROF(PC_ATTENTION); PPASR_CUDA_CHECK(launch_rel_attention(p.tm_q, p.tm_k, c->tm_pos, p.tm_vt, ap, st)); }
       } else {
@@ -958,11 +930,9 @@ int run_encoder(ppasr_b200_ctx* c, cudaStream_t st, bool chunk) {
           PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_y, m.pw1, M, 2 * D, D, eg, st)));
         }
         const int lpad = cfg.causal ? K - 1 : (K - 1) / 2;
-        if (!(cfg.causal && c->fused_ffn && c->fused_dwconv)) {
-          PROF(PC_DWCONV);
-          PPASR_CUDA_CHECK(launch_dwconv_norm_swish(p.g, w.dw_w, w.dw_b, cfg.causal ? w.glu_pad : nullptr, w.cn_g, w.cn_b,
-                                                    cfg.conv_norm == 0, p.z, p.B, p.Tp, p.Tp, D, K, lpad, eps, vl, st));
-        }
+        PROF(PC_DWCONV);
+        PPASR_CUDA_CHECK(launch_dwconv_norm_swish(p.g, w.dw_w, w.dw_b, cfg.causal ? w.glu_pad : nullptr, w.cn_g, w.cn_b,
+                                                  cfg.conv_norm == 0, p.z, p.B, p.Tp, p.Tp, D, K, lpad, eps, vl, st));
       } else {
         // [cnn_cache ; chunk] -> pw1 + GLU -> "valid" depthwise conv; cache <- last K-1 input rows (convolution.py:108-117)
         const int lorder = K - 1;
@@ -985,13 +955,9 @@ int run_encoder(ppasr_b200_ctx* c, cudaStream_t st, bool chunk) {
       const float* b2 = (l + 1 < L) ? c->layers[l + 1].ln_ffm_b : c->after_b;
       if (c->fused_ffn) {
         PROF(PC_FUSED_FFN);
-        // pointwise_conv2 + residual + norm_ff chained in front (z rows of pad frames are zero, bias masked); for causal
-        // models the depthwise conv + norm + swish that produces z runs in the same kernel's prologue
-        FfnDw dw{p.g, w.dw_w, w.dw_b, w.glu_pad, w.cn_g, w.cn_b, cfg.conv_kernel, cfg.conv_norm == 0};
-        const bool fdw = !chunk && cfg.causal && c->fused_dwconv;
+        // pointwise_conv2 + residual + norm_ff chained in front (z rows of pad frames are zero, bias masked)
         PPASR_CUDA_CHECK(launch_fused_ffn(p.tm_z, &m.pw2, m.ff_w1_128, m.ff_w2s, M, FF, p.x, p.y, w.ff_b1, w.ff_b2s, w.ln_fin_g,
-                                          w.ln_fin_b, g2, b2, eps, w.pw2_b, w.ln_ff_g, w.ln_ff_b, vl, p.Tp, st, 0, nullptr, nullptr,
-                                          nullptr, fdw ? &dw : nullptr));
+                                          w.ln_fin_b, g2, b2, eps, w.pw2_b, w.ln_ff_g, w.ln_ff_b, vl, p.Tp, st));
       } else {
         EpiStoreBF16<BN_WIDE, ACT_SWISH> e1{p.h, w.ff_b1, FF, M, FF};
         { PROF(PC_FFN1); PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_y, m.ff_w1, M, FF, D, e1, st))); }
@@ -1515,31 +1481,16 @@ int ppasr_b200_set_option(ppasr_b200_ctx* c, const char* name, int32_t value) {
     c->host_sync = value != 0;
     return PPASR_OK;
   }
-  if (n == "qkv_wide") {
-    c->qkv_wide = value != 0;
-    return PPASR_OK;
-  }
-  if (n == "qkv_co") {
-    c->qkv_co = value != 0;
-    return PPASR_OK;
-  }
   if (n == "conv1_tc") {
     c->conv1_tc = value != 0;
     return PPASR_OK;
   }
-  if (n == "attn_out_v2") {  // process-wide: fused_attn_out kernel variant
-    set_attn_out_variant(value);
-    return PPASR_OK;
-  }
   if (n == "ffn_split") {  // process-wide: which fused_ffn kernel launch_fused_ffn dispatches to
-    set_ffn_split_mode(value);
-    return PPASR_OK;
-  }
-  if (n == "fused_dwconv") {
-    c->fused_dwconv = value != 0;
+    PPASR_REQUIRE(set_ffn_split_mode(value), "ffn_split must be 1 or 2");
     return PPASR_OK;
   }
   if (n == "fused_conv") {
+    PPASR_REQUIRE(value == 0 || value == 2, "fused_conv must be 0 or 2");
     c->fused_conv = value;
     return PPASR_OK;
   }

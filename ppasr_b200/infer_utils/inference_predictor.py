@@ -241,7 +241,7 @@ class DecodePipeline:
         if depth > 1:
             predictor.engine.lib.ppasr_b200_set_pdl(0)  # early-started dependent CTAs would only hold SMs
             # several batches in flight fill the GPU by themselves: use the FFN variant with the least SM time per launch
-            predictor.engine.lib.ppasr_b200_set_ffn_split(int(os.environ.get("PPASR_B200_FFN_PIPE", "2")))
+            L.check(predictor.engine.lib.ppasr_b200_set_ffn_split(int(os.environ.get("PPASR_B200_FFN_PIPE", "2"))))
 
     def submit(self, speech, speech_lengths=None, trim_to_lens=False, blank_id=0, to_host=True):
         torch = self.torch
@@ -290,4 +290,4 @@ class DecodePipeline:
             slot["eng"].close()
         self.slots[0]["eng"].set_option("host_sync", 1)
         self.pred.engine.lib.ppasr_b200_set_pdl(1)
-        self.pred.engine.lib.ppasr_b200_set_ffn_split(int(os.environ.get("PPASR_B200_FFN_SPLIT", "1")))
+        L.check(self.pred.engine.lib.ppasr_b200_set_ffn_split(int(os.environ.get("PPASR_B200_FFN_SPLIT", "1"))))

@@ -13,8 +13,8 @@ for FF in (512, 1024, 2048, 4096):
     g1 = torch.rand(256, device=dev) + 0.5; bn1 = torch.randn(256, device=dev) * 0.1
     g2 = torch.rand(256, device=dev) + 0.5; bn2 = torch.randn(256, device=dev) * 0.1
     x0 = torch.randn(M, 256, device=dev)
-    for dbl, split in ((0, 0), (0, 1), (0, 2), (1, 0), (1, 1), (1, 2)):
-        lib.ppasr_b200_set_ffn_split(split)
+    for dbl, split in ((0, 1), (0, 2), (1, 1), (1, 2)):
+        L.check(lib.ppasr_b200_set_ffn_split(split))
         x = x0.clone(); yo = torch.zeros(M, 256, device=dev, dtype=torch.bfloat16)
         args = lambda: lib.ppasr_b200_op_fused_ffn(L.ptr(y), L.ptr(w1), L.ptr(w2), L.ptr(x), L.ptr(yo), L.ptr(b1), L.ptr(b2), L.ptr(g1), L.ptr(bn1),
                                                    L.ptr(g2) if dbl else None, L.ptr(bn2) if dbl else None, M, FF, 1e-5, L.stream_ptr())

@@ -563,6 +563,13 @@ def test_c_abi_state_errors_and_host_helpers_without_a_gpu():
     assert lib.ppasr_b200_set_option(ctx, b"fused_ffn", 0) == 0 and lib.ppasr_b200_set_option(ctx, b"fused_ffn", 1) == 0
     assert lib.ppasr_b200_set_option(ctx, b"no_such_option", 1) != 0
     assert lib.ppasr_b200_set_option(None, b"fused_ffn", 1) != 0
+    for gone in (b"qkv_wide", b"qkv_co", b"fused_dwconv", b"attn_out_v2"):  # removed kernel variants
+        assert lib.ppasr_b200_set_option(ctx, gone, 1) != 0 and "unknown option" in lib.ppasr_b200_last_error().decode()
+    assert lib.ppasr_b200_set_option(ctx, b"fused_conv", 0) == 0 and lib.ppasr_b200_set_option(ctx, b"fused_conv", 2) == 0
+    assert lib.ppasr_b200_set_option(ctx, b"fused_conv", 1) != 0
+    split = lib.ppasr_b200_get_ffn_split()
+    assert lib.ppasr_b200_set_ffn_split(0) != 0 and lib.ppasr_b200_set_option(ctx, b"ffn_split", 3) != 0
+    assert lib.ppasr_b200_get_ffn_split() == split
     lib.ppasr_b200_destroy(ctx)
     # sizes grow with the problem and are positive
     s1, s2, s3 = (lib.ppasr_b200_beam_state_bytes(1, 100, 10), lib.ppasr_b200_beam_state_bytes(2, 100, 10),
