@@ -234,8 +234,7 @@ int ppasr_b200_fbank(const float* audio, int32_t B, int64_t stride, int32_t N, c
                      int32_t sample_rate, int32_t db_normalize, float target_db, float* gain_ws, float* out, int32_t Tmax,
                      void* stream);
 
-/* Switches: "fused_ffn" / "fused_attn_out" (default 1) select the fused row-tile kernels, "fused_conv" (default 2) the
- * subsampling front end: 2 = conv1 (split-tf32 GEMM) as the A-operand producer of the conv2 GEMM in one kernel, 0 = conv1 kernel + conv2 GEMM
+/* Switches: "fused_conv" (default 2) selects the subsampling front end: 2 = conv1 (split-tf32 GEMM) as the A-operand producer of the conv2 GEMM in one kernel, 0 = conv1 kernel + conv2 GEMM
  * through the stride-phase images (bit-identical to 2 with conv1_tc = 1; the only front end for feat_dim > 96); "conv1_tc" (default 1) the first
  * subsampling conv on the tensor cores (split-tf32, conv1_tc.cu; 0 = the CUDA-core kernel); "ffn_split" (1 or 2) = ppasr_b200_set_ffn_split;
  * "host_sync" (default 1): ppasr_b200_ctc_greedy with host outputs synchronises the stream before

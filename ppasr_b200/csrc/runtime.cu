@@ -1,5 +1,5 @@
 // Model-level runtime behind the C-ABI (include/ppasr_b200.h): parameter packing, workspace,
-// the Conformer encoder launch sequence and the CTC head / greedy decode.
+// the Conformer / Efficient Conformer encoder launch sequence and the CTC head / greedy decode.
 //
 // Reference call path being replaced (yeyupiaoling/PPASR @ c8bb3b96):
 //   InferencePredictor.predict (ppasr/infer_utils/inference_predictor.py:103-145)
@@ -37,6 +37,7 @@ struct HostTensor {
 struct DeviceSlab {
   uint8_t* base = nullptr;
   size_t cap = 0, used = 0;
+  bool overflow = false;  // a take() did not fit: it returned nullptr and every later take() does too
   cudaError_t reserve(size_t bytes) {
     if (bytes <= cap) return cudaSuccess;
     if (base) cudaFree(base);
@@ -46,9 +47,14 @@ struct DeviceSlab {
     if (e == cudaSuccess) cap = bytes;
     return e;
   }
+  void rewind() { used = 0, overflow = false; }
   template <class T>
   T* take(size_t count) {
-    size_t off = (used + 255) & ~size_t(255);
+    const size_t off = (used + 255) & ~size_t(255);
+    if (overflow || off + count * sizeof(T) > cap) {
+      overflow = true;
+      return nullptr;
+    }
     used = off + count * sizeof(T);
     return reinterpret_cast<T*>(base + off);
   }
@@ -59,19 +65,22 @@ struct DeviceSlab {
   }
 };
 
-struct LayerW {
+// attention and conv-module weights of a Conformer-family block (Conformer, Efficient Conformer, Squeezeformer)
+struct BlockW {
+  const __nv_bfloat16 *wqkv, *wo, *pw1, *pw2;  // K-major bf16
+  const float *bqkv, *bo, *pos_u, *pos_v, *pw1_b, *pw2_b, *dw_w, *dw_b, *cn_g, *cn_b, *glu_pad;
+};
+struct BlockMaps {  // their tensor maps (B operands)
+  CUtensorMap wqkv, wo, pw1, pw2;
+};
+
+struct LayerW : BlockW {
   // layer norms (gamma, beta) fp32 [D]
   const float *ln_ffm_g, *ln_ffm_b, *ln_mha_g, *ln_mha_b, *ln_conv_g, *ln_conv_b, *ln_ff_g, *ln_ff_b, *ln_fin_g,
       *ln_fin_b;
-  // feed-forward (macaron, final): K-major bf16
-  const __nv_bfloat16 *ffm_w1, *ffm_w2, *ff_w1, *ff_w2, *ffm_w2s, *ff_w2s;  // *_w2s = 0.5 * W2 (macaron scale folded)
-  const float *ffm_b1, *ffm_b2, *ff_b1, *ff_b2, *ffm_b2s, *ff_b2s;
-  // attention
-  const __nv_bfloat16 *wqkv, *wo;
-  const float *bqkv, *bo, *pos_u, *pos_v;
-  // conv module
-  const __nv_bfloat16 *pw1, *pw2;
-  const float *pw1_b, *pw2_b, *dw_w, *dw_b, *cn_g, *cn_b, *glu_pad;
+  // feed-forward (macaron, final): K-major bf16, *_w2s / *_b2s = 0.5 * W2 / b2 (macaron scale folded)
+  const __nv_bfloat16 *ffm_w1, *ff_w1, *ffm_w2s, *ff_w2s;
+  const float *ffm_b1, *ff_b1, *ffm_b2s, *ff_b2s;
 };
 
 struct Plan {  // everything that depends on (B, T)
@@ -79,8 +88,8 @@ struct Plan {  // everything that depends on (B, T)
   // activations
   float* feats = nullptr;
   int* vlen = nullptr;
-  __nv_bfloat16 *phase = nullptr, *c2 = nullptr, *y = nullptr, *h = nullptr, *q2 = nullptr, *kk = nullptr,
-                *vt = nullptr, *att = nullptr, *g = nullptr, *z = nullptr;
+  __nv_bfloat16 *phase = nullptr, *c2 = nullptr, *y = nullptr, *q2 = nullptr, *kk = nullptr, *vt = nullptr,
+                *att = nullptr, *g = nullptr, *z = nullptr;
   // view of the encoder output the CTC head reads (== M / Tp / vlen unless the model changes the frame rate)
   int Mc = 0, Tc = 0;
   int* vc = nullptr;
@@ -97,7 +106,7 @@ struct Plan {  // everything that depends on (B, T)
   int Tcat = 0, Mcat = 0;
   __nv_bfloat16 *ycat = nullptr, *gcat = nullptr;
   // tensor maps (A operands)
-  CUtensorMap tm_phase, tm_c2, tm_y, tm_h, tm_att, tm_g, tm_z, tm_q, tm_k, tm_vt, tm_ycat;
+  CUtensorMap tm_phase, tm_c2, tm_y, tm_att, tm_g, tm_z, tm_q, tm_k, tm_vt, tm_ycat;
 };
 
 }  // namespace ppasr
@@ -112,32 +121,33 @@ struct ppasr_b200_ctx {
   DeviceSlab wslab, aslab;
   // global weights
   const float *cmvn_mean = nullptr, *cmvn_istd = nullptr, *conv1_w = nullptr, *conv1_b = nullptr, *conv2_b = nullptr,
-              *emb_b = nullptr, *after_g = nullptr, *after_b = nullptr, *ctc_b = nullptr, *zero_bias = nullptr;
+              *emb_b = nullptr, *after_g = nullptr, *after_b = nullptr, *ctc_b = nullptr;
   const __nv_bfloat16 *conv2_w = nullptr, *emb_w = nullptr, *ctc_w = nullptr, *pos_tab = nullptr;
   std::vector<LayerW> layers;
-  // weight tensor maps (B operands)
-  CUtensorMap tm_conv2_w, tm_emb_w, tm_ctc_w, tm_pos;
-  struct LayerMaps {
-    CUtensorMap ffm_w1, ffm_w2, ff_w1, ff_w2, wqkv, wo, pw1, pw2, ffm_w1_128, ff_w1_128, ffm_w2s, ff_w2s;
+  // weight tensor maps (B operands); tm_pos2: every second row of the positional table (pos_emb[:, ::2])
+  CUtensorMap tm_conv2_w, tm_emb_w, tm_ctc_w, tm_pos, tm_pos2;
+  struct LayerMaps : BlockMaps {
+    CUtensorMap ffm_w1_128, ff_w1_128, ffm_w2s, ff_w2s;
   };
   std::vector<LayerMaps> lmaps;
+  cudaError_t upload_err = cudaSuccess;  // first failed weight copy of finalize
   // ---- Squeezeformer (model_type 1; squeezeformer/encoder.py) ----
-  struct SqLayerW {
+  struct SqLayerW : BlockW {
     const float *ln_g[4], *ln_b[4];    // layer_norm1..4
     const float *ada_s[4], *ada_b[4];  // adaptive scale/bias of: 0 self_attn, 1 ffn1, 2 conv_module, 3 ffn2
-    const __nv_bfloat16 *wqkv, *wo, *w1[2], *w2[2], *pw1, *pw2;
-    const float *bqkv, *bo, *pos_u, *pos_v, *b1[2], *b2[2], *pw1_b, *pw2_b, *dw_w, *dw_b, *cn_g, *cn_b, *glu_pad;
+    const __nv_bfloat16 *w1[2], *w2[2];
+    const float *b1[2], *b2[2];
   };
-  struct SqLayerMaps {
-    CUtensorMap wqkv, wo, w1_128[2], w2[2], pw1, pw2;
+  struct SqLayerMaps : BlockMaps {
+    CUtensorMap w1_128[2], w2[2];
   };
   struct Sqz {
     std::vector<SqLayerW> layers;
     std::vector<SqLayerMaps> maps;
-    const float *preln_g = nullptr, *preln_b = nullptr, *emb_b_scaled = nullptr, *tr_dw_w = nullptr, *tr_dw_b = nullptr,
-                *tr_pw_b = nullptr, *rec_b = nullptr, *ones = nullptr, *zeros = nullptr;
+    const float *preln_g = nullptr, *preln_b = nullptr, *tr_dw_w = nullptr, *tr_dw_b = nullptr, *tr_pw_b = nullptr,
+                *rec_b = nullptr, *ones = nullptr, *zeros = nullptr;
     const __nv_bfloat16 *tr_pw = nullptr, *rec_w = nullptr;
-    CUtensorMap tm_tr_pw, tm_rec_w, tm_pos2;  // tm_pos2: every second row of the positional table (pos_emb[:, ::2])
+    CUtensorMap tm_tr_pw, tm_rec_w;
     int reduce_idx = -1, recover_idx = -1, tr_k = 1;
   } sq;
   // ---- DeepSpeech2 (model_type 2; deepspeech2/encoder.py) ----
@@ -157,12 +167,11 @@ struct ppasr_b200_ctx {
     float *h_state = nullptr, *c_state = nullptr;
     int state_B = 0;
   } ds;
-  int ctc_k = 0;  // input features of the CTC projection (0 = d_model)
+  int ctc_k = 0;  // input features of the CTC projection
   // ---- Efficient Conformer (model_type 3; efficient_conformer/encoder.py) ----
   int eff_stride_idx = -1;      // block with the strided depthwise conv (-1: none)
   unsigned eff_group_mask = 0;  // bit l: block l uses grouped attention
   std::vector<int> layer_k;     // depthwise kernel size per block
-  CUtensorMap tm_pos2;          // every second row of the positional table (pos_emb[:, ::2])
   Plan plan;
   int sms = 148;
   // ---- streaming state (reference: inference_predictor.py:35-39,215-220; device resident here) ----
@@ -186,9 +195,6 @@ struct ppasr_b200_ctx {
     int* d_step = nullptr;                      // device [5][B]: slots, kofs, k_row0, pos_row0, klen of the current step
     int step_T2 = 0;
   } ss;
-  // optional per-kernel-class timing (cudaEvent pairs around every launch of the step)
-  bool fused_ffn = true;
-  bool fused_attn_out = true;
   bool conv1_tc = true;   // conv1 on the tensor cores (conv1_tc.cu); 0 = the CUDA-core kernel (env PPASR_B200_CONV1_TC / option "conv1_tc")
   int fused_conv = 2;  // 2 (default): conv_front_tc (tensor-core conv1 producer inside the conv2 GEMM), 0: conv1 + conv2 GEMM; env PPASR_B200_FUSED_CONV
   bool host_sync = true;  // ctc_* with host outputs synchronise the stream before returning
@@ -201,6 +207,7 @@ struct ppasr_b200_ctx {
   cudaGraphExec_t graph_exec = nullptr;
   bool capturing = false;
   long long graph_kernels = 0, capture_count0 = 0;
+  // optional per-kernel-class timing (cudaEvent pairs around every launch of the step)
   bool profiling = false;
   int prof_only = -1;  // >= 0: event pairs only around launches of this kernel class (undisturbed neighbours)
   struct ProfRec {
@@ -277,11 +284,275 @@ std::vector<float> transpose_in_out(const HostTensor& w, int rows_pad = 0) {
 int finalize_squeezeformer(ppasr_b200_ctx* c);  // runtime_squeezeformer.inl
 int finalize_ds2(ppasr_b200_ctx* c);            // runtime_ds2.inl
 
+// ---- weight packing shared by the finalize of every model ------------------------------------------------------------
+// An upload that does not fit the slab, or whose copy fails, returns nullptr (or an unwritten pointer) and is reported by
+// check_weights(), which runs before anything launches on the slab and at the end of finalize.
 template <class T>
 const T* upload(ppasr_b200_ctx* c, const std::vector<T>& v) {
   T* d = c->wslab.take<T>(v.size());
-  cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
+  if (d && c->upload_err == cudaSuccess) c->upload_err = cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice);
   return d;
+}
+
+const float* vecf(ppasr_b200_ctx* c, const std::string& n) { return upload(c, c->host[n].data); }
+
+int check_weights(ppasr_b200_ctx* c) {
+  if (c->wslab.overflow) {
+    set_last_error("internal error: weight slab too small");
+    return PPASR_ERR_STATE;
+  }
+  PPASR_CUDA_CHECK(c->upload_err);
+  return PPASR_OK;
+}
+
+int require_present(ppasr_b200_ctx* c, const std::vector<std::string>& names) {
+  std::string missing;
+  for (auto& n : names) find(c, n, &missing);
+  if (!missing.empty()) {
+    set_last_error("missing parameters: " + missing);
+    return PPASR_ERR_STATE;
+  }
+  return PPASR_OK;
+}
+
+// parameters of block prefix p read by pack_attention / pack_conv_module
+void block_names(const ppasr_b200_config& cfg, const std::string& p, bool pos_bias, std::vector<std::string>* names) {
+  for (const char* s : {"linear_q", "linear_k", "linear_v", "linear_out"}) {
+    names->push_back(p + "self_attn." + s + ".weight");
+    names->push_back(p + "self_attn." + s + ".bias");
+  }
+  names->push_back(p + "self_attn.linear_pos.weight");
+  if (pos_bias) names->push_back(p + "self_attn.linear_pos.bias");
+  names->push_back(p + "self_attn.pos_bias_u");
+  names->push_back(p + "self_attn.pos_bias_v");
+  for (const char* s : {"pointwise_conv1", "depthwise_conv", "pointwise_conv2", "norm"}) {
+    names->push_back(p + "conv_module." + s + ".weight");
+    names->push_back(p + "conv_module." + s + ".bias");
+  }
+  if (cfg.conv_norm == 1) {
+    names->push_back(p + "conv_module.norm._mean");
+    names->push_back(p + "conv_module.norm._variance");
+  }
+}
+
+// Weight slab size of the Conformer family: no packed weight is larger than its fp32 host tensor (bf16 halves it;
+// transposes, the value/gate interleave and BatchNorm folding keep it), plus what finalize derives (sinusoid and
+// positional tables, linear_pos biases, GLU pads, zero / one vectors, the padded CTC head) and 256 B alignment each.
+size_t conformer_slab_bytes(const ppasr_b200_ctx* c) {
+  const auto& cfg = c->cfg;
+  const size_t D = cfg.d_model, L = cfg.n_layers, ML = cfg.max_len;
+  size_t bytes = 0;
+  for (auto& t : c->host) bytes += (size_t)t.second.numel() * 4;
+  bytes += ML * (L + 1) * D * 2 + (3 * L * D + D + 4096 + (size_t)c->Vpad * (D + 1)) * 4;
+  bytes += (c->host.size() + 8 * L + 64) * 256;
+  return bytes;
+}
+
+// front end: CMVN, conv1 [D,1,3,3] (conv1_name), conv2 [D,D,3,3] (conv2_name) as K-major [D, (kh*3+kw)*D + i] and the
+// embedding Linear [D*F2 (c*F2+f), D] (emb_name) as K-major [D, f*D + c]; its bias is stored times emb_b_scale
+int pack_front(ppasr_b200_ctx* c, const std::string& conv1_name, const std::string& conv2_name, const std::string& emb_name,
+               float emb_b_scale) {
+  const int D = c->cfg.d_model;
+  c->cmvn_mean = vecf(c, "encoder.global_cmvn.mean");
+  c->cmvn_istd = vecf(c, "encoder.global_cmvn.istd");
+  {
+    const HostTensor& w = c->host[conv1_name + ".weight"];
+    PPASR_REQUIRE(w.numel() == (int64_t)D * 9, conv1_name + ".weight shape");
+    c->conv1_w = upload(c, w.data);
+    c->conv1_b = vecf(c, conv1_name + ".bias");
+  }
+  {
+    const HostTensor& w = c->host[conv2_name + ".weight"];
+    PPASR_REQUIRE(w.numel() == (int64_t)D * D * 9, conv2_name + ".weight shape");
+    std::vector<float> p((size_t)D * 9 * D);
+    for (int o = 0; o < D; ++o)
+      for (int i = 0; i < D; ++i)
+        for (int t = 0; t < 9; ++t) p[(size_t)o * 9 * D + (size_t)t * D + i] = w.data[((size_t)o * D + i) * 9 + t];
+    c->conv2_w = upload(c, to_bf16(p));
+    c->conv2_b = vecf(c, conv2_name + ".bias");
+  }
+  {
+    const HostTensor& w = c->host[emb_name + ".weight"];
+    PPASR_REQUIRE(w.shape.size() == 2 && w.shape[0] == (int64_t)D * c->F2 && w.shape[1] == D, emb_name + ".weight shape");
+    std::vector<float> p((size_t)D * c->Kemb);
+    for (int ch = 0; ch < D; ++ch)
+      for (int f = 0; f < c->F2; ++f)
+        for (int o = 0; o < D; ++o) p[(size_t)o * c->Kemb + (size_t)f * D + ch] = w.data[((size_t)ch * c->F2 + f) * D + o];
+    c->emb_w = upload(c, to_bf16(p));
+    std::vector<float> b = c->host[emb_name + ".bias"].data;
+    for (auto& v : b) v *= emb_b_scale;
+    c->emb_b = upload(c, b);
+  }
+  if (int rc = check_weights(c)) return rc;
+  std::string err;
+  if (!make_tmap_2d(&c->tm_conv2_w, c->conv2_w, (uint64_t)9 * D, D, (uint64_t)9 * D * 2, BN_WIDE, &err) ||
+      !make_tmap_2d(&c->tm_emb_w, c->emb_w, c->Kemb, D, (uint64_t)c->Kemb * 2, BN_WIDE, &err)) {
+    set_last_error(err);
+    return PPASR_ERR_CUDA;
+  }
+  return PPASR_OK;
+}
+
+// CTC head: <prefix>ctc_lo.weight [K, V] -> K-major [Vpad, K] bf16, bias zero-padded to Vpad
+int pack_ctc(ppasr_b200_ctx* c, const std::string& prefix, int K) {
+  const int V = c->cfg.vocab_size;
+  const HostTensor& w = c->host[prefix + "ctc_lo.weight"];
+  PPASR_REQUIRE(w.shape.size() == 2 && w.shape[0] == K && w.shape[1] == V, prefix + "ctc_lo.weight shape");
+  c->ctc_w = upload(c, to_bf16(transpose_in_out(w, c->Vpad)));
+  std::vector<float> b(c->Vpad, 0.f);
+  std::memcpy(b.data(), c->host[prefix + "ctc_lo.bias"].data.data(), sizeof(float) * V);
+  c->ctc_b = upload(c, b);
+  c->ctc_k = K;
+  if (int rc = check_weights(c)) return rc;
+  std::string err;
+  if (!make_tmap_2d(&c->tm_ctc_w, c->ctc_w, K, c->Vpad, (uint64_t)K * 2, BN_NARROW, &err)) {
+    set_last_error(err);
+    return PPASR_ERR_CUDA;
+  }
+  return PPASR_OK;
+}
+
+// self-attention of block l (prefix p): Q/K/V concatenated into one [3D, D] GEMM operand; linear_pos goes into the
+// positional table's operands wpos_all [L*D, D] / bpos_all [L*D] (with its bias where the block has one)
+int pack_attention(ppasr_b200_ctx* c, const std::string& p, int l, bool grouped, bool pos_bias, BlockW& w, BlockMaps& m,
+                   std::vector<float>& wpos_all, std::vector<float>& bpos_all) {
+  const int D = c->cfg.d_model;
+  PPASR_REQUIRE(c->host[p + "self_attn.pos_bias_u"].numel() == (int64_t)c->cfg.n_heads * (grouped ? 192 : 64) &&
+                    c->host[p + "self_attn.pos_bias_v"].numel() == (int64_t)c->cfg.n_heads * (grouped ? 192 : 64),
+                "pos_bias_u / pos_bias_v shape");
+  {
+    std::vector<float> qkv((size_t)3 * D * D), bq((size_t)3 * D);
+    const char* nm[3] = {"linear_q", "linear_k", "linear_v"};
+    for (int s = 0; s < 3; ++s) {
+      auto t = transpose_in_out(c->host[p + "self_attn." + nm[s] + ".weight"]);
+      std::memcpy(qkv.data() + (size_t)s * D * D, t.data(), sizeof(float) * D * D);
+      std::memcpy(bq.data() + (size_t)s * D, c->host[p + "self_attn." + nm[s] + ".bias"].data.data(), sizeof(float) * D);
+    }
+    w.wqkv = upload(c, to_bf16(qkv));
+    w.bqkv = upload(c, bq);
+  }
+  w.wo = upload(c, to_bf16(transpose_in_out(c->host[p + "self_attn.linear_out.weight"])));
+  w.bo = vecf(c, p + "self_attn.linear_out.bias");
+  w.pos_u = vecf(c, p + "self_attn.pos_bias_u");
+  w.pos_v = vecf(c, p + "self_attn.pos_bias_v");
+  {
+    auto t = transpose_in_out(c->host[p + "self_attn.linear_pos.weight"]);
+    std::memcpy(wpos_all.data() + (size_t)l * D * D, t.data(), sizeof(float) * D * D);
+    if (pos_bias)
+      std::memcpy(bpos_all.data() + (size_t)l * D, c->host[p + "self_attn.linear_pos.bias"].data.data(), sizeof(float) * D);
+  }
+  if (int rc = check_weights(c)) return rc;
+  std::string err;
+  if (!make_tmap_2d(&m.wqkv, w.wqkv, D, 3 * D, (uint64_t)D * 2, BN_NARROW, &err) ||
+      !make_tmap_2d(&m.wo, w.wo, D, D, (uint64_t)D * 2, BN_WIDE, &err)) {
+    set_last_error(err);
+    return PPASR_ERR_CUDA;
+  }
+  return PPASR_OK;
+}
+
+// conv module of a block (prefix p) with depthwise kernel K
+int pack_conv_module(ppasr_b200_ctx* c, const std::string& p, int K, BlockW& w, BlockMaps& m) {
+  const auto& cfg = c->cfg;
+  const int D = cfg.d_model;
+  {
+    // pointwise_conv1.weight [2D, D, 1]: rows [0,D) = "a", [D,2D) = gate -> interleave (2c, 2c+1)
+    const HostTensor& pw = c->host[p + "conv_module.pointwise_conv1.weight"];
+    const HostTensor& pb = c->host[p + "conv_module.pointwise_conv1.bias"];
+    PPASR_REQUIRE(pw.numel() == (int64_t)2 * D * D, "pointwise_conv1.weight shape");
+    std::vector<float> wi((size_t)2 * D * D), bi((size_t)2 * D);
+    for (int ch = 0; ch < D; ++ch) {
+      std::memcpy(&wi[(size_t)(2 * ch) * D], &pw.data[(size_t)ch * D], sizeof(float) * D);
+      std::memcpy(&wi[(size_t)(2 * ch + 1) * D], &pw.data[(size_t)(ch + D) * D], sizeof(float) * D);
+      bi[2 * ch] = pb.data[ch];
+      bi[2 * ch + 1] = pb.data[ch + D];
+    }
+    w.pw1 = upload(c, to_bf16(wi));
+    w.pw1_b = upload(c, bi);
+  }
+  float* pad = c->wslab.take<float>(D);
+  {
+    const HostTensor& dw = c->host[p + "conv_module.depthwise_conv.weight"];  // [D,1,K]
+    PPASR_REQUIRE(dw.numel() == (int64_t)D * K, "depthwise_conv.weight shape");
+    w.dw_w = upload(c, dw.data);
+    w.dw_b = vecf(c, p + "conv_module.depthwise_conv.bias");
+  }
+  if (cfg.conv_norm == 0) {
+    w.cn_g = vecf(c, p + "conv_module.norm.weight");
+    w.cn_b = vecf(c, p + "conv_module.norm.bias");
+  } else {
+    // eval-mode BatchNorm1D folded to scale/shift (epsilon 1e-5)
+    const auto& g = c->host[p + "conv_module.norm.weight"].data;
+    const auto& b = c->host[p + "conv_module.norm.bias"].data;
+    const auto& mu = c->host[p + "conv_module.norm._mean"].data;
+    const auto& var = c->host[p + "conv_module.norm._variance"].data;
+    std::vector<float> sc(D), sh(D);
+    for (int i = 0; i < D; ++i) {
+      sc[i] = g[i] / std::sqrt(var[i] + 1e-5f);
+      sh[i] = b[i] - mu[i] * sc[i];
+    }
+    w.cn_g = upload(c, sc);
+    w.cn_b = upload(c, sh);
+  }
+  {
+    const HostTensor& pw = c->host[p + "conv_module.pointwise_conv2.weight"];  // [D, D, 1] = [out, in]
+    PPASR_REQUIRE(pw.numel() == (int64_t)D * D, "pointwise_conv2.weight shape");
+    w.pw2 = upload(c, to_bf16(pw.data));
+    w.pw2_b = vecf(c, p + "conv_module.pointwise_conv2.bias");
+  }
+  if (int rc = check_weights(c)) return rc;
+  PPASR_CUDA_CHECK(launch_glu_pad(w.pw1_b, pad, D, 0));
+  w.glu_pad = pad;
+  std::string err;
+  if (!make_tmap_2d(&m.pw1, w.pw1, D, 2 * D, (uint64_t)D * 2, BN_WIDE, &err) ||
+      !make_tmap_2d(&m.pw2, w.pw2, D, D, (uint64_t)D * 2, BN_WIDE, &err)) {
+    set_last_error(err);
+    return PPASR_ERR_CUDA;
+  }
+  return PPASR_OK;
+}
+
+// weight-only precompute: pos_tab[pos, l*D + h*64 + d] = linear_pos_l(pe[pos]) + bpos_l, and the tensor maps of all its
+// rows (tm_pos) and of every second row (tm_pos2, the half-rate blocks)
+// (reference: conformer/embedding.py:41-53 table, attention.py:234-236 projection; the projection of a constant table by a
+//  constant matrix is folded here, like BatchNorm folding)
+int pack_pos_table(ppasr_b200_ctx* c, const std::vector<float>& wpos_all, const std::vector<float>& bpos_all) {
+  const int D = c->cfg.d_model, L = c->cfg.n_layers, ML = c->cfg.max_len;
+  std::vector<float> pe((size_t)ML * D);
+  for (int pos = 0; pos < ML; ++pos)
+    for (int i = 0; i < D / 2; ++i) {
+      const float div = std::exp((float)(2 * i) * -(std::log(10000.0f) / (float)D));
+      pe[(size_t)pos * D + 2 * i] = std::sin((float)pos * div);
+      pe[(size_t)pos * D + 2 * i + 1] = std::cos((float)pos * div);
+    }
+  const __nv_bfloat16* pe_d = upload(c, to_bf16(pe));
+  const __nv_bfloat16* wpos_d = upload(c, to_bf16(wpos_all));
+  __nv_bfloat16* tab = c->wslab.take<__nv_bfloat16>((size_t)ML * L * D);
+  const float* bpos_d = upload(c, bpos_all);
+  if (int rc = check_weights(c)) return rc;
+  std::string err;
+  CUtensorMap ta, tb;
+  if (!make_tmap_2d(&ta, pe_d, D, ML, (uint64_t)D * 2, GEMM_BLOCK_M, &err) ||
+      !make_tmap_2d(&tb, wpos_d, D, (uint64_t)L * D, (uint64_t)D * 2, BN_WIDE, &err) ||
+      !make_tmap_2d(&c->tm_pos, tab, (uint64_t)L * D, ML, (uint64_t)L * D * 2, 128, &err) ||
+      !make_tmap_2d(&c->tm_pos2, tab, (uint64_t)L * D, ML / 2, (uint64_t)2 * L * D * 2, 128, &err)) {
+    set_last_error(err);
+    return PPASR_ERR_CUDA;
+  }
+  GemmShape s = make_shape(ML, L * D, D, BN_WIDE);
+  EpiStoreBF16<BN_WIDE, ACT_NONE> epi{tab, bpos_d, L * D, ML, L * D};
+  PPASR_CUDA_CHECK((launch_gemm<BN_WIDE, ST_WIDE, false>(ta, tb, s, epi, c->sms, 0)));
+  c->pos_tab = tab;
+  return PPASR_OK;
+}
+
+// waits for the packing kernels, reports any failed upload, and drops the host copies
+int finish_finalize(ppasr_b200_ctx* c) {
+  PPASR_CUDA_CHECK(cudaDeviceSynchronize());
+  if (int rc = check_weights(c)) return rc;
+  c->host.clear();
+  c->finalized = true;
+  return PPASR_OK;
 }
 
 }  // namespace
@@ -388,8 +659,7 @@ int ppasr_b200_finalize(ppasr_b200_ctx* c) {
   PPASR_REQUIRE(c, "null ctx");
   if (c->finalized) return PPASR_OK;
   const auto& cfg = c->cfg;
-  const int D = cfg.d_model, L = cfg.n_layers, FF = cfg.ffn_dim, V = cfg.vocab_size;
-  const int Kmax = cfg.conv_kernel;
+  const int D = cfg.d_model, L = cfg.n_layers, FF = cfg.ffn_dim;
   int dev = 0;
   PPASR_CUDA_CHECK(cudaGetDevice(&dev));
   cudaDeviceProp prop;
@@ -400,11 +670,10 @@ int ppasr_b200_finalize(ppasr_b200_ctx* c) {
     return PPASR_ERR_CUDA;
   }
   c->sms = prop.multiProcessorCount;
+  c->upload_err = cudaSuccess;
   if (cfg.model_type == 1) return finalize_squeezeformer(c);
   if (cfg.model_type == 2) return finalize_ds2(c);
 
-  std::string missing;
-  auto need = [&](const std::string& n) { return find(c, n, &missing); };
   // ---- presence check first, so the error lists everything -------------------------------------
   std::vector<std::string> names = {"encoder.global_cmvn.mean", "encoder.global_cmvn.istd",
                                     "encoder.embed.conv.0.weight", "encoder.embed.conv.0.bias",
@@ -420,111 +689,36 @@ int ppasr_b200_finalize(ppasr_b200_ctx* c) {
     }
     for (const char* s : {"feed_forward_macaron", "feed_forward"})
       for (const char* t : {".w_1.weight", ".w_1.bias", ".w_2.weight", ".w_2.bias"}) names.push_back(p + s + t);
-    for (const char* s : {"linear_q", "linear_k", "linear_v", "linear_out"}) {
-      names.push_back(p + "self_attn." + s + ".weight");
-      names.push_back(p + "self_attn." + s + ".bias");
-    }
-    names.push_back(p + "self_attn.linear_pos.weight");
-    if ((c->eff_group_mask >> l) & 1) names.push_back(p + "self_attn.linear_pos.bias");  // efficient_conformer/attention.py:31
-    names.push_back(p + "self_attn.pos_bias_u");
-    names.push_back(p + "self_attn.pos_bias_v");
-    for (const char* s : {"pointwise_conv1", "depthwise_conv", "pointwise_conv2", "norm"}) {
-      names.push_back(p + "conv_module." + s + ".weight");
-      names.push_back(p + "conv_module." + s + ".bias");
-    }
-    if (cfg.conv_norm == 1) {
-      names.push_back(p + "conv_module.norm._mean");
-      names.push_back(p + "conv_module.norm._variance");
-    }
+    block_names(cfg, p, (c->eff_group_mask >> l) & 1, &names);  // grouped linear_pos has a bias (efficient_conformer/attention.py:31)
   }
-  for (auto& n : names) need(n);
-  if (!missing.empty()) {
-    set_last_error("missing parameters: " + missing);
-    return PPASR_ERR_STATE;
-  }
+  if (int rc = require_present(c, names)) return rc;
 
-  // ---- size the weight slab ----------------------------------------------------------------------
-  size_t bytes = 0;
-  bytes += (size_t)L * ((size_t)6 * D * FF + 3 * D * D + D * D + 2 * D * D + D * D) * 2;  // bf16 matrices
-  bytes += (size_t)D * 9 * D * 2 + (size_t)D * c->Kemb * 2 + (size_t)c->Vpad * D * 2;
-  bytes += (size_t)cfg.max_len * L * D * 2 + (size_t)cfg.max_len * D * 2 + (size_t)L * D * D * 2;
-  bytes += (size_t)L * (20 * D + 2 * FF + 3 * D + 2 * D + D * Kmax + 64 + 8 * 192) * 4 + (size_t)(c->Vpad + 4 * D + 2 * L * D + 4096) * 4;
-  bytes += 4u << 20;  // alignment slack
-  PPASR_CUDA_CHECK(c->wslab.reserve(bytes));
-  c->wslab.used = 0;
-
-  std::string err;
-  auto vecf = [&](const std::string& n) -> const float* { return upload(c, c->host[n].data); };
-
-  // ---- front end ------------------------------------------------------------------------------
-  c->cmvn_mean = vecf("encoder.global_cmvn.mean");
-  c->cmvn_istd = vecf("encoder.global_cmvn.istd");
-  {
-    const HostTensor& w = c->host["encoder.embed.conv.0.weight"];  // [D,1,3,3]
-    PPASR_REQUIRE(w.numel() == (int64_t)D * 9, "conv.0.weight shape");
-    c->conv1_w = upload(c, w.data);
-    c->conv1_b = vecf("encoder.embed.conv.0.bias");
-  }
-  {
-    // conv.2.weight [O, I, 3, 3] -> K-major [O, (kh*3+kw)*I + i]
-    const HostTensor& w = c->host["encoder.embed.conv.2.weight"];
-    PPASR_REQUIRE(w.numel() == (int64_t)D * D * 9, "conv.2.weight shape");
-    std::vector<float> p((size_t)D * 9 * D);
-    for (int o = 0; o < D; ++o)
-      for (int i = 0; i < D; ++i)
-        for (int t = 0; t < 9; ++t) p[(size_t)o * 9 * D + (size_t)t * D + i] = w.data[((size_t)o * D + i) * 9 + t];
-    c->conv2_w = upload(c, to_bf16(p));
-    c->conv2_b = vecf("encoder.embed.conv.2.bias");
-  }
-  {
-    // out.0.weight [C*F2 (c*F2+f), D] -> K-major [D, f*D + c]
-    const HostTensor& w = c->host["encoder.embed.out.0.weight"];
-    PPASR_REQUIRE(w.shape.size() == 2 && w.shape[0] == (int64_t)D * c->F2 && w.shape[1] == D, "embed.out.0.weight shape");
-    std::vector<float> p((size_t)D * c->Kemb);
-    for (int ch = 0; ch < D; ++ch)
-      for (int f = 0; f < c->F2; ++f)
-        for (int o = 0; o < D; ++o) p[(size_t)o * c->Kemb + (size_t)f * D + ch] = w.data[((size_t)ch * c->F2 + f) * D + o];
-    c->emb_w = upload(c, to_bf16(p));
-    c->emb_b = vecf("encoder.embed.out.0.bias");
-  }
-  c->after_g = vecf("encoder.after_norm.weight");
-  c->after_b = vecf("encoder.after_norm.bias");
-  {
-    const HostTensor& w = c->host["ctc.ctc_lo.weight"];  // [D, V]
-    PPASR_REQUIRE(w.shape.size() == 2 && w.shape[0] == D && w.shape[1] == V, "ctc_lo.weight shape");
-    c->ctc_w = upload(c, to_bf16(transpose_in_out(w, c->Vpad)));
-    std::vector<float> b(c->Vpad, 0.f);
-    std::memcpy(b.data(), c->host["ctc.ctc_lo.bias"].data.data(), sizeof(float) * V);
-    c->ctc_b = upload(c, b);
-  }
-  {
-    std::vector<float> z((size_t)std::max(L * D, 4096), 0.f);
-    c->zero_bias = upload(c, z);
-  }
+  PPASR_CUDA_CHECK(c->wslab.reserve(conformer_slab_bytes(c)));
+  c->wslab.rewind();
+  int rc;
+  if ((rc = pack_front(c, "encoder.embed.conv.0", "encoder.embed.conv.2", "encoder.embed.out.0", 1.0f))) return rc;
+  c->after_g = vecf(c, "encoder.after_norm.weight");
+  c->after_b = vecf(c, "encoder.after_norm.bias");
+  if ((rc = pack_ctc(c, "ctc.", D))) return rc;
 
   // ---- encoder layers -------------------------------------------------------------------------
   c->layers.resize(L);
   c->lmaps.resize(L);
-  std::vector<float> wpos_all((size_t)L * D * D), bpos_all((size_t)L * D, 0.f);
+  std::vector<float> wpos_all((size_t)L * D * D), bpos_all((size_t)L * D, 0.f);  // bias: grouped blocks only
   for (int l = 0; l < L; ++l) {
     const std::string p = "encoder.encoders." + std::to_string(l) + ".";
     LayerW& w = c->layers[l];
-    const int K = c->layer_k[l];
+    auto& m = c->lmaps[l];
     const bool grouped = (c->eff_group_mask >> l) & 1;
-    PPASR_REQUIRE(c->host[p + "self_attn.pos_bias_u"].numel() == (int64_t)cfg.n_heads * (grouped ? 192 : 64) &&
-                      c->host[p + "self_attn.pos_bias_v"].numel() == (int64_t)cfg.n_heads * (grouped ? 192 : 64),
-                  "pos_bias_u / pos_bias_v shape");
-    w.ln_ffm_g = vecf(p + "norm_ff_macaron.weight"), w.ln_ffm_b = vecf(p + "norm_ff_macaron.bias");
-    w.ln_mha_g = vecf(p + "norm_mha.weight"), w.ln_mha_b = vecf(p + "norm_mha.bias");
-    w.ln_conv_g = vecf(p + "norm_conv.weight"), w.ln_conv_b = vecf(p + "norm_conv.bias");
-    w.ln_ff_g = vecf(p + "norm_ff.weight"), w.ln_ff_b = vecf(p + "norm_ff.bias");
-    w.ln_fin_g = vecf(p + "norm_final.weight"), w.ln_fin_b = vecf(p + "norm_final.bias");
+    w.ln_ffm_g = vecf(c, p + "norm_ff_macaron.weight"), w.ln_ffm_b = vecf(c, p + "norm_ff_macaron.bias");
+    w.ln_mha_g = vecf(c, p + "norm_mha.weight"), w.ln_mha_b = vecf(c, p + "norm_mha.bias");
+    w.ln_conv_g = vecf(c, p + "norm_conv.weight"), w.ln_conv_b = vecf(c, p + "norm_conv.bias");
+    w.ln_ff_g = vecf(c, p + "norm_ff.weight"), w.ln_ff_b = vecf(c, p + "norm_ff.bias");
+    w.ln_fin_g = vecf(c, p + "norm_final.weight"), w.ln_fin_b = vecf(c, p + "norm_final.bias");
     w.ffm_w1 = upload(c, to_bf16(transpose_in_out(c->host[p + "feed_forward_macaron.w_1.weight"])));
-    w.ffm_w2 = upload(c, to_bf16(transpose_in_out(c->host[p + "feed_forward_macaron.w_2.weight"])));
     w.ff_w1 = upload(c, to_bf16(transpose_in_out(c->host[p + "feed_forward.w_1.weight"])));
-    w.ff_w2 = upload(c, to_bf16(transpose_in_out(c->host[p + "feed_forward.w_2.weight"])));
-    w.ffm_b1 = vecf(p + "feed_forward_macaron.w_1.bias"), w.ffm_b2 = vecf(p + "feed_forward_macaron.w_2.bias");
-    w.ff_b1 = vecf(p + "feed_forward.w_1.bias"), w.ff_b2 = vecf(p + "feed_forward.w_2.bias");
+    w.ffm_b1 = vecf(c, p + "feed_forward_macaron.w_1.bias");
+    w.ff_b1 = vecf(c, p + "feed_forward.w_1.bias");
     {
       // ff_scale = 0.5 (encoder.py:331-332) folded into W2 / b2 for the fused kernel (exact: power of two)
       auto scaled = [&](const std::string& wn, const std::string& bn, const __nv_bfloat16** wd, const float** bd) {
@@ -538,136 +732,19 @@ int ppasr_b200_finalize(ppasr_b200_ctx* c) {
       scaled(p + "feed_forward_macaron.w_2.weight", p + "feed_forward_macaron.w_2.bias", &w.ffm_w2s, &w.ffm_b2s);
       scaled(p + "feed_forward.w_2.weight", p + "feed_forward.w_2.bias", &w.ff_w2s, &w.ff_b2s);
     }
-    {
-      std::vector<float> qkv((size_t)3 * D * D), bq((size_t)3 * D);
-      const char* nm[3] = {"linear_q", "linear_k", "linear_v"};
-      for (int s = 0; s < 3; ++s) {
-        auto t = transpose_in_out(c->host[p + "self_attn." + nm[s] + ".weight"]);
-        std::memcpy(qkv.data() + (size_t)s * D * D, t.data(), sizeof(float) * D * D);
-        std::memcpy(bq.data() + (size_t)s * D, c->host[p + "self_attn." + nm[s] + ".bias"].data.data(), sizeof(float) * D);
-      }
-      w.wqkv = upload(c, to_bf16(qkv));
-      w.bqkv = upload(c, bq);
-    }
-    w.wo = upload(c, to_bf16(transpose_in_out(c->host[p + "self_attn.linear_out.weight"])));
-    w.bo = vecf(p + "self_attn.linear_out.bias");
-    w.pos_u = vecf(p + "self_attn.pos_bias_u");
-    w.pos_v = vecf(p + "self_attn.pos_bias_v");
-    {
-      auto t = transpose_in_out(c->host[p + "self_attn.linear_pos.weight"]);
-      std::memcpy(wpos_all.data() + (size_t)l * D * D, t.data(), sizeof(float) * D * D);
-      if (grouped)
-        std::memcpy(bpos_all.data() + (size_t)l * D, c->host[p + "self_attn.linear_pos.bias"].data.data(), sizeof(float) * D);
-    }
-    {
-      // pointwise_conv1.weight [2D, D, 1]: rows [0,D) = "a", [D,2D) = gate -> interleave (2c, 2c+1)
-      const HostTensor& pw = c->host[p + "conv_module.pointwise_conv1.weight"];
-      const HostTensor& pb = c->host[p + "conv_module.pointwise_conv1.bias"];
-      PPASR_REQUIRE(pw.numel() == (int64_t)2 * D * D, "pointwise_conv1.weight shape");
-      std::vector<float> wi((size_t)2 * D * D), bi((size_t)2 * D);
-      for (int ch = 0; ch < D; ++ch) {
-        std::memcpy(&wi[(size_t)(2 * ch) * D], &pw.data[(size_t)ch * D], sizeof(float) * D);
-        std::memcpy(&wi[(size_t)(2 * ch + 1) * D], &pw.data[(size_t)(ch + D) * D], sizeof(float) * D);
-        bi[2 * ch] = pb.data[ch];
-        bi[2 * ch + 1] = pb.data[ch + D];
-      }
-      w.pw1 = upload(c, to_bf16(wi));
-      w.pw1_b = upload(c, bi);
-      float* pad = c->wslab.take<float>(D);
-      PPASR_CUDA_CHECK(launch_glu_pad(w.pw1_b, pad, D, 0));
-      w.glu_pad = pad;
-    }
-    {
-      const HostTensor& dw = c->host[p + "conv_module.depthwise_conv.weight"];  // [D,1,K]
-      PPASR_REQUIRE(dw.numel() == (int64_t)D * K, "depthwise_conv.weight shape");
-      w.dw_w = upload(c, dw.data);
-      w.dw_b = vecf(p + "conv_module.depthwise_conv.bias");
-    }
-    if (cfg.conv_norm == 0) {
-      w.cn_g = vecf(p + "conv_module.norm.weight");
-      w.cn_b = vecf(p + "conv_module.norm.bias");
-    } else {
-      // eval-mode BatchNorm1D folded to scale/shift (epsilon 1e-5)
-      const auto& g = c->host[p + "conv_module.norm.weight"].data;
-      const auto& b = c->host[p + "conv_module.norm.bias"].data;
-      const auto& mu = c->host[p + "conv_module.norm._mean"].data;
-      const auto& var = c->host[p + "conv_module.norm._variance"].data;
-      std::vector<float> sc(D), sh(D);
-      for (int i = 0; i < D; ++i) {
-        sc[i] = g[i] / std::sqrt(var[i] + 1e-5f);
-        sh[i] = b[i] - mu[i] * sc[i];
-      }
-      w.cn_g = upload(c, sc);
-      w.cn_b = upload(c, sh);
-    }
-    {
-      const HostTensor& pw = c->host[p + "conv_module.pointwise_conv2.weight"];  // [D, D, 1] = [out, in]
-      PPASR_REQUIRE(pw.numel() == (int64_t)D * D, "pointwise_conv2.weight shape");
-      w.pw2 = upload(c, to_bf16(pw.data));
-      w.pw2_b = vecf(p + "conv_module.pointwise_conv2.bias");
-    }
-    auto& m = c->lmaps[l];
-    bool ok = make_tmap_2d(&m.ffm_w1, w.ffm_w1, D, FF, (uint64_t)D * 2, BN_WIDE, &err) &&
-              make_tmap_2d(&m.ffm_w2, w.ffm_w2, FF, D, (uint64_t)FF * 2, BN_WIDE, &err) &&
-              make_tmap_2d(&m.ff_w1, w.ff_w1, D, FF, (uint64_t)D * 2, BN_WIDE, &err) &&
-              make_tmap_2d(&m.ffm_w2s, w.ffm_w2s, FF, D, (uint64_t)FF * 2, BN_WIDE, &err) &&
-              make_tmap_2d(&m.ff_w2s, w.ff_w2s, FF, D, (uint64_t)FF * 2, BN_WIDE, &err) &&
-              make_tmap_2d(&m.ffm_w1_128, w.ffm_w1, D, FF, (uint64_t)D * 2, 128, &err) &&
-              make_tmap_2d(&m.ff_w1_128, w.ff_w1, D, FF, (uint64_t)D * 2, 128, &err) &&
-              make_tmap_2d(&m.ff_w2, w.ff_w2, FF, D, (uint64_t)FF * 2, BN_WIDE, &err) &&
-              make_tmap_2d(&m.wqkv, w.wqkv, D, 3 * D, (uint64_t)D * 2, BN_NARROW, &err) &&
-              make_tmap_2d(&m.wo, w.wo, D, D, (uint64_t)D * 2, BN_WIDE, &err) &&
-              make_tmap_2d(&m.pw1, w.pw1, D, 2 * D, (uint64_t)D * 2, BN_WIDE, &err) &&
-              make_tmap_2d(&m.pw2, w.pw2, D, D, (uint64_t)D * 2, BN_WIDE, &err);
-    if (!ok) {
+    if ((rc = pack_attention(c, p, l, grouped, grouped, w, m, wpos_all, bpos_all))) return rc;
+    if ((rc = pack_conv_module(c, p, c->layer_k[l], w, m))) return rc;
+    std::string err;
+    if (!make_tmap_2d(&m.ffm_w2s, w.ffm_w2s, FF, D, (uint64_t)FF * 2, BN_WIDE, &err) ||
+        !make_tmap_2d(&m.ff_w2s, w.ff_w2s, FF, D, (uint64_t)FF * 2, BN_WIDE, &err) ||
+        !make_tmap_2d(&m.ffm_w1_128, w.ffm_w1, D, FF, (uint64_t)D * 2, 128, &err) ||
+        !make_tmap_2d(&m.ff_w1_128, w.ff_w1, D, FF, (uint64_t)D * 2, 128, &err)) {
       set_last_error(err);
       return PPASR_ERR_CUDA;
     }
   }
-  if (!make_tmap_2d(&c->tm_conv2_w, c->conv2_w, (uint64_t)9 * D, D, (uint64_t)9 * D * 2, BN_WIDE, &err) ||
-      !make_tmap_2d(&c->tm_emb_w, c->emb_w, c->Kemb, D, (uint64_t)c->Kemb * 2, BN_WIDE, &err) ||
-      !make_tmap_2d(&c->tm_ctc_w, c->ctc_w, D, c->Vpad, (uint64_t)D * 2, BN_NARROW, &err)) {
-    set_last_error(err);
-    return PPASR_ERR_CUDA;
-  }
-
-  // ---- weight-only precompute: pos_tab[pos, l*D + h*64 + d] = linear_pos_l(pe[pos]) --------------
-  // (reference: conformer/embedding.py:41-53 table, attention.py:234-236 projection; the projection
-  //  of a constant table by a constant matrix is folded here, like BatchNorm folding)
-  {
-    const int ML = cfg.max_len;
-    std::vector<float> pe((size_t)ML * D);
-    for (int pos = 0; pos < ML; ++pos)
-      for (int i = 0; i < D / 2; ++i) {
-        const float div = std::exp((float)(2 * i) * -(std::log(10000.0f) / (float)D));
-        pe[(size_t)pos * D + 2 * i] = std::sin((float)pos * div);
-        pe[(size_t)pos * D + 2 * i + 1] = std::cos((float)pos * div);
-      }
-    const __nv_bfloat16* pe_d = upload(c, to_bf16(pe));
-    const __nv_bfloat16* wpos_d = upload(c, to_bf16(wpos_all));
-    __nv_bfloat16* tab = c->wslab.take<__nv_bfloat16>((size_t)ML * L * D);
-    CUtensorMap ta, tb;
-    if (!make_tmap_2d(&ta, pe_d, D, ML, (uint64_t)D * 2, GEMM_BLOCK_M, &err) ||
-        !make_tmap_2d(&tb, wpos_d, D, (uint64_t)L * D, (uint64_t)D * 2, BN_WIDE, &err) ||
-        !make_tmap_2d(&c->tm_pos, tab, (uint64_t)L * D, ML, (uint64_t)L * D * 2, 128, &err) ||
-        !make_tmap_2d(&c->tm_pos2, tab, (uint64_t)L * D, ML / 2, (uint64_t)2 * L * D * 2, 128, &err)) {
-      set_last_error(err);
-      return PPASR_ERR_CUDA;
-    }
-    GemmShape s = make_shape(ML, L * D, D, BN_WIDE);
-    const float* bpos_d = upload(c, bpos_all);  // zero except for grouped blocks (their linear_pos has a bias)
-    EpiStoreBF16<BN_WIDE, ACT_NONE> epi{tab, bpos_d, L * D, ML, L * D};
-    PPASR_CUDA_CHECK((launch_gemm<BN_WIDE, ST_WIDE, false>(ta, tb, s, epi, c->sms, 0)));
-    c->pos_tab = tab;
-  }
-  PPASR_CUDA_CHECK(cudaDeviceSynchronize());
-  if (c->wslab.used > c->wslab.cap) {
-    set_last_error("internal error: weight slab overflow");
-    return PPASR_ERR_STATE;
-  }
-  c->host.clear();
-  c->finalized = true;
-  return PPASR_OK;
+  if ((rc = pack_pos_table(c, wpos_all, bpos_all))) return rc;
+  return finish_finalize(c);
 }
 
 int ppasr_b200_out_frames(const ppasr_b200_ctx* c, int32_t T) {
@@ -686,7 +763,7 @@ int build_plan(ppasr_b200_ctx* c, int B, int T) {
   Plan& p = c->plan;
   if (p.B == B && p.T == T) return PPASR_OK;
   const auto& cfg = c->cfg;
-  const int D = cfg.d_model, H = cfg.n_heads, FF = cfg.ffn_dim, F = cfg.feat_dim;
+  const int D = cfg.d_model, H = cfg.n_heads, F = cfg.feat_dim;
   PPASR_REQUIRE(T >= 7, "need at least 7 feature frames (subsampling right context, predict.py:288)");
   Plan n;
   n.B = B, n.T = T;
@@ -718,7 +795,6 @@ int build_plan(ppasr_b200_ctx* c, int B, int T) {
   acc(B * 4);
   acc(M * D * 2 * 4);                               // y, att, g, z
   acc((size_t)n.Mcat * D * 2 * 2);                  // ycat, gcat
-  acc(M * FF * 2);                                  // h
   acc((size_t)B * H * n.Tp * 128 * 2);              // q2
   acc((size_t)B * H * n.Tp * 64 * 2);               // kk
   acc((size_t)B * H * 64 * n.Tkp * 2);              // vt
@@ -733,7 +809,7 @@ int build_plan(ppasr_b200_ctx* c, int B, int T) {
     // q2/kk/vt padding regions must be finite for masked-out MMA operands
     PPASR_CUDA_CHECK(cudaMemset(c->aslab.base, 0, c->aslab.cap));
   }
-  c->aslab.used = 0;
+  c->aslab.rewind();
   auto& a = c->aslab;
   n.feats = a.take<float>((size_t)B * T * F);
   n.vlen = a.take<int>(B);
@@ -756,7 +832,6 @@ int build_plan(ppasr_b200_ctx* c, int B, int T) {
   n.z = a.take<__nv_bfloat16>(M * D);
   n.ycat = a.take<__nv_bfloat16>((size_t)n.Mcat * D);
   n.gcat = a.take<__nv_bfloat16>((size_t)n.Mcat * D);
-  n.h = a.take<__nv_bfloat16>(M * FF);
   n.q2 = a.take<__nv_bfloat16>((size_t)B * H * n.Tp * 128);
   n.kk = a.take<__nv_bfloat16>((size_t)B * H * n.Tp * 64);
   n.vt = a.take<__nv_bfloat16>((size_t)B * H * 64 * n.Tkp);
@@ -770,7 +845,7 @@ int build_plan(ppasr_b200_ctx* c, int B, int T) {
   n.ids = a.take<int>(M);
   n.out_len = a.take<int>(B);
   n.score = a.take<float>(B);
-  if (a.used > a.cap) {
+  if (a.overflow) {
     set_last_error("internal error: activation slab overflow");
     return PPASR_ERR_STATE;
   }
@@ -778,7 +853,6 @@ int build_plan(ppasr_b200_ctx* c, int B, int T) {
   bool ok = make_tmap_3d(&n.tm_phase, n.phase, D, n.Mr, 4, (uint64_t)D * 2, (uint64_t)n.Mr * D * 2, GEMM_BLOCK_M, &err) &&
             make_tmap_2d(&n.tm_c2, n.c2, c->Kemb, M, (uint64_t)c->Kemb * 2, GEMM_BLOCK_M, &err) &&
             make_tmap_2d(&n.tm_y, n.y, D, M, (uint64_t)D * 2, GEMM_BLOCK_M, &err) &&
-            make_tmap_2d(&n.tm_h, n.h, FF, M, (uint64_t)FF * 2, GEMM_BLOCK_M, &err) &&
             make_tmap_2d(&n.tm_att, n.att, D, M, (uint64_t)D * 2, GEMM_BLOCK_M, &err) &&
             make_tmap_2d(&n.tm_g, n.g, D, M, (uint64_t)D * 2, GEMM_BLOCK_M, &err) &&
             make_tmap_2d(&n.tm_z, n.z, D, M, (uint64_t)D * 2, GEMM_BLOCK_M, &err) &&
@@ -847,123 +921,159 @@ int run_subsampling_convs(ppasr_b200_ctx* c, cudaStream_t st) {
 
 #include "runtime_squeezeformer.inl"
 #include "runtime_ds2.inl"
-#include "runtime_effconf.inl"
 
+constexpr int EFF_GCAP = 256;  // key groups a grouped block can attend (grouped_attention_kernel keeps the score row in TMEM)
+
+// Conformer (model_type 0) and Efficient Conformer (model_type 3): the pre-norm macaron block on the fused kernels.
+// Reference: conformer/encoder.py:164-206 (forward), :380-429 (block); efficient_conformer/encoder.py:212-264 (forward),
+// :455-548 (stride block), attention.py:128-193 (grouped attention), convolution.py:80-138 (strided conv module).
+// What the Efficient Conformer changes per block:
+//   * grouped blocks: the QKV epilogue writes the (T/3 tokens x 4 heads x 192) views, grouped_attention_kernel;
+//   * the stride block: strided depthwise conv, AvgPool1D(2, ceil) on the residual, then everything (rows, lengths,
+//     positional rows) at half rate; blocks after it use depthwise kernel 7 (layer_k).
+//
+// chunk: forward_chunk (conformer/encoder.py:208-275, efficient_conformer/encoder.py:266-394) on the device-resident caches
+// in c->ss, no padding masks. This chunk's K/V are appended to the block's cache at row kend (at the block's rate) and
+// keys kstart .. kend + chunk are attended with positions offset - cache_t ... (conformer/attention.py:225-232,
+// encoder.py:253). The Efficient Conformer streams with required_cache_size < 0 (PPASRPredictor, predict.py:304-306), so
+// its caches are append-only (kstart = 0, offset = kend) and pad4group's re-grouping from the first cached frame
+// (attention.py:153-160) is simply group = absolute_frame // 3:
+//   * grouped blocks keep K as [B,H,group,192] and V^T as [B,H,192,group] (the EpiQKVGrouped operand layout) inside the
+//     same per-layer cache slices the plain blocks use; a new frame f lands in group f / 3 at feature (f % 3) * 256 + c;
+//     the caches start zeroed, so the missing frames of a partially filled last group read as zero (a real, unmasked key);
+//   * queries are grouped from the CHUNK start (zero padded before pos_bias_u/v are added);
+//   * p = linear_pos(pos_emb[0 : t_total]) zero-padded to a multiple of 3 is rebuilt per chunk (grouped_pos_kernel);
+//   * blocks after the stride block run at half rate: keys at positions 2 j (tm_pos2), caches hold kend / 2 frames
+//     (the reference stores them repeated x2 and reads ::2, encoder.py:351,368), conv caches of K/2 - 1 = 6 rows;
+//   * the stride block's stride-2 "valid" conv over [cache 14 | chunk] is aligned with the offline run because chunks
+//     start at even frames; its residual goes through AvgPool1D(2, 2, ceil).
+// tests/test_effconf_chunk_layout_spec_cpu.py states this layout in NumPy and checks it against the reference code's own
+// streaming outputs.
 int run_encoder(ppasr_b200_ctx* c, cudaStream_t st, bool chunk) {
   Plan& p = c->plan;
   auto& ss = c->ss;
   const auto& cfg = c->cfg;
-  const int D = cfg.d_model, H = cfg.n_heads, FF = cfg.ffn_dim, L = cfg.n_layers, M = p.M;
+  const int D = cfg.d_model, H = cfg.n_heads, FF = cfg.ffn_dim, L = cfg.n_layers, B = p.B;
+  const int lmax = cfg.conv_kernel - 1;  // conv-cache rows per (layer, stream)
   const float eps = 1e-5f;
   { int rcf = run_subsampling_convs(c, st); if (rcf) return rcf; }
-  // Linear(F2*D -> D) then x * sqrt(D) (subsampling.py:113, embedding.py:113), fused with block 0's first LayerNorm
-  auto resid_ln = [&](int cls, const CUtensorMap& ta, const CUtensorMap& tb, int K, const float* bias, float alpha,
-                      int residual, const int* lens, int mask_resid, int zero_y_pad, const float* g1, const float* b1,
-                      const float* g2, const float* b2) -> int {
-    EpiResidLN<BN_WIDE> e{p.x, bias, D, M, D, alpha, residual, lens, p.Tp, mask_resid, zero_y_pad, g1, b1, g2, b2, p.y, eps};
-    PROF(cls);
-    PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, ta, tb, M, D, K, e, st)));
-    return PPASR_OK;
-  };
-  int rc;
-  if ((rc = resid_ln(PC_EMBED, p.tm_c2, c->tm_emb_w, c->Kemb, c->emb_b, std::sqrt((float)D), 0, nullptr, 0, 0,
-                     c->layers[0].ln_ffm_g, c->layers[0].ln_ffm_b, nullptr, nullptr)))
-    return rc;
+  // the residual stream at the current rate: rows, frames per utterance, valid lengths, positional rows
+  float* xc = p.x;
+  int Tc = p.Tp, Mc = p.M, rate = 1;
   const int* vl = chunk ? nullptr : p.vlen;
+  const CUtensorMap* tmpos = &c->tm_pos;
+  // Linear(F2*D -> D) then x * sqrt(D) (subsampling.py:113, embedding.py:113), fused with block 0's first LayerNorm
+  {
+    EpiResidLN<BN_WIDE> e{p.x, c->emb_b, D, p.M, D, std::sqrt((float)D), 0, nullptr, p.Tp, 0, 0, c->layers[0].ln_ffm_g,
+                          c->layers[0].ln_ffm_b, nullptr, nullptr, p.y, eps};
+    PROF(PC_EMBED);
+    PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_c2, c->tm_emb_w, p.M, D, c->Kemb, e, st)));
+  }
+  int gi = 0;  // index of the grouped block (its padded positional rows live in slot gi of p.pg / ss.pgc)
   for (int l = 0; l < L; ++l) {
     const LayerW& w = c->layers[l];
     const auto& m = c->lmaps[l];
+    const int K = c->layer_k[l];
+    const bool grouped = (c->eff_group_mask >> l) & 1;
+    const bool strided = l == c->eff_stride_idx;
     // ---- macaron FFN: x += 0.5 * W2 swish(W1 LN(x)); then y = norm_mha(x)        (encoder.py:380-390)
-    if (c->fused_ffn) {
-      PROF(PC_FUSED_FFN);
-      PPASR_CUDA_CHECK(launch_fused_ffn(p.tm_y, nullptr, m.ffm_w1_128, m.ffm_w2s, M, FF, p.x, p.y, w.ffm_b1, w.ffm_b2s,
-                                        w.ln_mha_g, w.ln_mha_b, nullptr, nullptr, eps, nullptr, nullptr, nullptr, nullptr,
-                                        p.Tp, st));
-    } else {
-      EpiStoreBF16<BN_WIDE, ACT_SWISH> e1{p.h, w.ffm_b1, FF, M, FF};
-      { PROF(PC_FFN1); PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_y, m.ffm_w1, M, FF, D, e1, st))); }
-      if ((rc = resid_ln(PC_FFN2, p.tm_h, m.ffm_w2, FF, w.ffm_b2, 0.5f, 1, nullptr, 0, 0, w.ln_mha_g, w.ln_mha_b, nullptr, nullptr)))
-        return rc;
-    }
-    // ---- rel-pos MHA: x += Wo attn(y); then y = mask(norm_conv(x))                (encoder.py:389-409)
     {
+      PROF(PC_FUSED_FFN);
+      PPASR_CUDA_CHECK(launch_fused_ffn(p.tm_y, nullptr, m.ffm_w1_128, m.ffm_w2s, Mc, FF, xc, p.y, w.ffm_b1, w.ffm_b2s, w.ln_mha_g,
+                                        w.ln_mha_b, nullptr, nullptr, eps, nullptr, nullptr, nullptr, nullptr, Tc, st));
+    }
+    // ---- rel-pos MHA (encoder.py:389-409)
+    const size_t lk = (size_t)l * ss.B * H * ss.Tcap * 64;
+    const int kend = ss.kend / rate, kstart = ss.kstart / rate, cache_t = kend - kstart;  // chunk: cached keys at this rate
+    if (grouped && !chunk) {
+      // pad4group of p = linear_pos(pos_emb): rows >= T are zero (attention.py:73-77)
+      PPASR_CUDA_CHECK(launch_grouped_pos(c->pos_tab, L * D, l * D, Tc, 3 * p.Tg, p.pg + (size_t)gi * p.Tg * 768, st));
+      EpiQKVGrouped<BN_NARROW> e{p.q2g, p.kkg, p.vtg, w.bqkv, w.pos_u, w.pos_v, Mc, Tc, H, p.Tg, p.Tgp};
+      { PROF(PC_QKV); PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, Mc, 3 * D, D, e, st))); }
+      GroupedAttnParams gp{B, H, Tc, p.Tg, vl, p.att};
+      { PROF(PC_ATTENTION); PPASR_CUDA_CHECK(launch_grouped_attention(p.tm_qg, p.tm_kg, p.tm_pg[gi], p.tm_vtg, gp, st)); }
+      ++gi;
+    } else if (grouped) {
+      // positional operand of the T2 keys at positions j * rate, zero beyond T2 inside the last group
+      const int T2 = cache_t + Tc, G2 = (T2 + 2) / 3;
+      PPASR_CUDA_CHECK(launch_grouped_pos(c->pos_tab, L * D * rate, l * D, T2, 3 * G2, ss.pgc + (size_t)gi * EFF_GCAP * 768, st));
+      EpiQKVGrouped<BN_NARROW> e{p.q2g, ss.kk + lk, ss.vt + lk, w.bqkv, w.pos_u, w.pos_v, Mc, Tc, H, (Tc + 2) / 3, EFF_GCAP};
+      e.kofs = kend, e.Tgk = EFF_GCAP;
+      { PROF(PC_QKV); PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, Mc, 3 * D, D, e, st))); }
+      GroupedAttnParams gp{B, H, Tc, (Tc + 2) / 3, nullptr, p.att};
+      gp.Tgk = G2, gp.k_pitch = EFF_GCAP;
+      { PROF(PC_ATTENTION); PPASR_CUDA_CHECK(launch_grouped_attention(ss.tm_qgc, ss.tm_k[l], ss.tm_pgc[gi], ss.tm_vt[l], gp, st)); }
+      ++gi;
+    } else {
       AttnParams ap{};
-      ap.B = p.B, ap.H = H, ap.T1 = p.Tp, ap.D = D, ap.pos_col0 = l * D, ap.out = p.att, ap.q_rows_per_bh = p.Tp;
+      ap.B = B, ap.H = H, ap.T1 = Tc, ap.D = D, ap.pos_col0 = l * D, ap.out = p.att, ap.q_rows_per_bh = Tc;
       if (!chunk) {
-        EpiQKV<BN_NARROW> e{p.q2, p.kk, p.vt, w.bqkv, w.pos_u, w.pos_v, M, p.Tp, H, p.Tp, p.Tkp, 0};
-        { PROF(PC_QKV); PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, M, 3 * D, D, e, st))); }
-        ap.T2 = p.Tp, ap.k_rows_per_bh = p.Tp, ap.k_row0 = 0, ap.pos_row0 = 0, ap.klens = p.vlen;
-        { PROF(PC_ATTENTION); PPASR_CUDA_CHECK(launch_rel_attention(p.tm_q, p.tm_k, c->tm_pos, p.tm_vt, ap, st)); }
+        EpiQKV<BN_NARROW> e{p.q2, p.kk, p.vt, w.bqkv, w.pos_u, w.pos_v, Mc, Tc, H, Tc, p.Tkp, 0};
+        { PROF(PC_QKV); PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, Mc, 3 * D, D, e, st))); }
+        ap.T2 = Tc, ap.k_rows_per_bh = Tc, ap.k_row0 = 0, ap.pos_row0 = 0, ap.klens = vl;
+        { PROF(PC_ATTENTION); PPASR_CUDA_CHECK(launch_rel_attention(p.tm_q, p.tm_k, *tmpos, p.tm_vt, ap, st)); }
       } else {
-        // K/V of this chunk are appended to the device-resident cache at row kend (attention.py:225-232);
-        // keys kstart .. kend+chunk are attended, positions offset-cache_t .. (encoder.py:253)
-        const size_t lk = (size_t)l * ss.B * H * ss.Tcap * 64;
-        EpiQKV<BN_NARROW> e{p.q2, ss.kk + lk, ss.vt + lk, w.bqkv, w.pos_u, w.pos_v, M, p.Tp, H, ss.Tcap, ss.Tcap, ss.kend};
-        if (ss.ragged) e.slots = ss.d_step, e.kofs_b = ss.d_step + p.B;
-        { PROF(PC_QKV); PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, M, 3 * D, D, e, st))); }
-        const int cache_t = ss.kend - ss.kstart;
-        ap.T2 = cache_t + p.Tp, ap.k_rows_per_bh = ss.Tcap, ap.k_row0 = ss.kstart, ap.pos_row0 = ss.offset - cache_t;
-        ap.klens = nullptr;
+        EpiQKV<BN_NARROW> e{p.q2, ss.kk + lk, ss.vt + lk, w.bqkv, w.pos_u, w.pos_v, Mc, Tc, H, ss.Tcap, ss.Tcap, kend};
+        if (ss.ragged) e.slots = ss.d_step, e.kofs_b = ss.d_step + B;
+        { PROF(PC_QKV); PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, Mc, 3 * D, D, e, st))); }
+        ap.T2 = cache_t + Tc, ap.k_rows_per_bh = ss.Tcap, ap.k_row0 = kstart;
+        ap.pos_row0 = (ss.offset - (ss.kend - ss.kstart)) / rate, ap.klens = nullptr;
         if (ss.ragged) {  // per-session cache slot / key range / positions
           ap.T2 = ss.step_T2;
-          ap.slots = ss.d_step, ap.k_row0s = ss.d_step + 2 * p.B, ap.pos_row0s = ss.d_step + 3 * p.B, ap.klens = ss.d_step + 4 * p.B;
+          ap.slots = ss.d_step, ap.k_row0s = ss.d_step + 2 * B, ap.pos_row0s = ss.d_step + 3 * B, ap.klens = ss.d_step + 4 * B;
         }
-        { PROF(PC_ATTENTION); PPASR_CUDA_CHECK(launch_rel_attention(p.tm_q, ss.tm_k[l], c->tm_pos, ss.tm_vt[l], ap, st)); }
-      }
-      // pad frames of the conv-module input are zeroed (convolution.py:104-106 with the caller's inverted mask)
-      if (!chunk && c->fused_attn_out) {
-        PROF(PC_FUSED_ATTN_OUT);
-        PPASR_CUDA_CHECK(launch_fused_attn_out(p.tm_att, m.wo, m.pw1, M, p.x, p.g, w.bo, w.ln_conv_g, w.ln_conv_b, w.pw1_b, vl,
-                                               p.Tp, eps, st));
-      } else if ((rc = resid_ln(PC_OUTPROJ, p.tm_att, m.wo, D, w.bo, 1.0f, 1, vl, 0, 1, w.ln_conv_g, w.ln_conv_b, nullptr,
-                                nullptr))) {
-        return rc;
+        { PROF(PC_ATTENTION); PPASR_CUDA_CHECK(launch_rel_attention(p.tm_q, ss.tm_k[l], *tmpos, ss.tm_vt[l], ap, st)); }
       }
     }
-    // ---- conv module: x += mask * pw2 swish(norm(dw(glu(pw1(y))))); then y = norm_ff(x)   (encoder.py:407-421)
-    {
-      const int K = cfg.conv_kernel;
-      if (!chunk) {
-        if (!c->fused_attn_out) {
-          EpiGLU<BN_WIDE> eg{p.g, w.pw1_b, D, M, 2 * D};
-          PROF(PC_PW1_GLU);
-          PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_y, m.pw1, M, 2 * D, D, eg, st)));
-        }
-        const int lpad = cfg.causal ? K - 1 : (K - 1) / 2;
-        PROF(PC_DWCONV);
-        PPASR_CUDA_CHECK(launch_dwconv_norm_swish(p.g, w.dw_w, w.dw_b, cfg.causal ? w.glu_pad : nullptr, w.cn_g, w.cn_b,
-                                                  cfg.conv_norm == 0, p.z, p.B, p.Tp, p.Tp, D, K, lpad, eps, vl, st));
-      } else {
-        // [cnn_cache ; chunk] -> pw1 + GLU -> "valid" depthwise conv; cache <- last K-1 input rows (convolution.py:108-117)
-        const int lorder = K - 1;
-        PPASR_CUDA_CHECK(launch_conv_cache_concat(ss.cnn + (size_t)l * ss.B * lorder * D, p.y, p.ycat, p.B, p.Tp, lorder, D, st,
-                                                  ss.ragged ? ss.d_step : nullptr));
-        EpiGLU<BN_WIDE> eg{p.gcat, w.pw1_b, D, p.Mcat, 2 * D};
-        { PROF(PC_PW1_GLU); PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_ycat, m.pw1, p.Mcat, 2 * D, D, eg, st))); }
-        { PROF(PC_DWCONV); PPASR_CUDA_CHECK(launch_dwconv_norm_swish(p.gcat, w.dw_w, w.dw_b, nullptr, w.cn_g, w.cn_b, cfg.conv_norm == 0,
-                                                  p.z, p.B, p.Tcat, p.Tp, D, K, 0, eps, nullptr, st)); }
+    // ---- x += Wo att + bo; y = mask(norm_conv(x)); then the conv module's pw1 + GLU, depthwise conv, norm, swish -> z
+    //      (encoder.py:407-421; pad frames of the conv-module input are zeroed, convolution.py:104-106)
+    const __nv_bfloat16* gin = p.g;  // GLU output the depthwise conv reads
+    int Tin = Tc;                    // ... and its frames per utterance
+    if (!chunk) {
+      PROF(PC_FUSED_ATTN_OUT);
+      PPASR_CUDA_CHECK(launch_fused_attn_out(p.tm_att, m.wo, m.pw1, Mc, xc, p.g, w.bo, w.ln_conv_g, w.ln_conv_b, w.pw1_b, vl, Tc,
+                                             eps, st));
+    } else {
+      {
+        EpiResidLN<BN_WIDE> e{xc, w.bo, D, Mc, D, 1.0f, 1, nullptr, Tc, 0, 1, w.ln_conv_g, w.ln_conv_b, nullptr, nullptr, p.y, eps};
+        PROF(PC_OUTPROJ);
+        PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_att, m.wo, Mc, D, D, e, st)));
       }
-      if (!c->fused_ffn) {
-        if ((rc = resid_ln(PC_PW2, p.tm_z, m.pw2, D, w.pw2_b, 1.0f, 1, vl, 1, 0, w.ln_ff_g, w.ln_ff_b, nullptr, nullptr)))
-          return rc;
-      }
+      // [cnn_cache ; chunk] -> pw1 + GLU -> "valid" depthwise conv; cache <- last K-1 input rows (convolution.py:108-117)
+      const int lorder = K - 1, Mcat = B * (lorder + Tc);
+      PPASR_CUDA_CHECK(launch_conv_cache_concat(ss.cnn + (size_t)l * ss.B * lmax * D, p.y, p.ycat, B, Tc, lorder, D, st,
+                                                ss.ragged ? ss.d_step : nullptr));
+      EpiGLU<BN_WIDE> eg{p.gcat, w.pw1_b, D, Mcat, 2 * D};
+      { PROF(PC_PW1_GLU); PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_ycat, m.pw1, Mcat, 2 * D, D, eg, st))); }
+      gin = p.gcat, Tin = lorder + Tc;
     }
-    // ---- FFN: x += 0.5 * W2 swish(W1 y); x = norm_final(x); y = next block's first LayerNorm (or after_norm)
-    //      (encoder.py:419-429, 201-202)
+    // offline: 'same' padding (causal: K-1 rows on the left, read from glu_pad); chunk: the cache is the left context
+    const int lpad = chunk ? 0 : cfg.causal ? K - 1 : (K - 1) / 2;
+    const float* pad_left = (!chunk && cfg.causal) ? w.glu_pad : nullptr;
+    if (!strided) {
+      PROF(PC_DWCONV);
+      PPASR_CUDA_CHECK(launch_dwconv_norm_swish(gin, w.dw_w, w.dw_b, pad_left, w.cn_g, w.cn_b, cfg.conv_norm == 0, p.z, B, Tin,
+                                                Tc, D, K, lpad, eps, vl, st));
+    } else {
+      const int T2 = chunk ? (Tin - K) / 2 + 1 : (Tc + 1) / 2;  // == ceil(Tc / 2), the pooled residual's length
+      if (!chunk) PPASR_CUDA_CHECK(launch_halve_lens(p.vlen, p.vlen2, B, st));
+      { PROF(PC_DWCONV);
+        PPASR_CUDA_CHECK(launch_dwconv_stride(gin, w.dw_w, w.dw_b, pad_left, w.cn_g, w.cn_b, cfg.conv_norm == 0, p.z, B, Tin, T2,
+                                              D, K, lpad, 2, eps, chunk ? nullptr : p.vlen2, st)); }
+      // residual through AvgPool1D(2, 2, ceil_mode) (efficient_conformer/encoder.py:523-526)
+      PPASR_CUDA_CHECK(launch_avgpool2(xc, p.x2, B, Tc, T2, D, st));
+      if (chunk) PPASR_CUDA_CHECK(launch_halve_lens(p.vlen, p.vlen2, B, st));  // the CTC head's lengths: every row is valid
+      xc = p.x2, Tc = T2, Mc = B * T2, vl = chunk ? nullptr : p.vlen2, tmpos = &c->tm_pos2, rate = 2;
+    }
+    // ---- x += mask * (pw2 z + b); y = norm_ff(x); FFN: x += 0.5 * W2 swish(W1 y); x = norm_final(x);
+    //      y = next block's first LayerNorm (or after_norm)                                 (encoder.py:419-429, 201-202)
     {
       const float* g2 = (l + 1 < L) ? c->layers[l + 1].ln_ffm_g : c->after_g;
       const float* b2 = (l + 1 < L) ? c->layers[l + 1].ln_ffm_b : c->after_b;
-      if (c->fused_ffn) {
-        PROF(PC_FUSED_FFN);
-        // pointwise_conv2 + residual + norm_ff chained in front (z rows of pad frames are zero, bias masked)
-        PPASR_CUDA_CHECK(launch_fused_ffn(p.tm_z, &m.pw2, m.ff_w1_128, m.ff_w2s, M, FF, p.x, p.y, w.ff_b1, w.ff_b2s, w.ln_fin_g,
-                                          w.ln_fin_b, g2, b2, eps, w.pw2_b, w.ln_ff_g, w.ln_ff_b, vl, p.Tp, st));
-      } else {
-        EpiStoreBF16<BN_WIDE, ACT_SWISH> e1{p.h, w.ff_b1, FF, M, FF};
-        { PROF(PC_FFN1); PPASR_CUDA_CHECK((gemm<BN_WIDE, ST_WIDE>(c, p.tm_y, m.ff_w1, M, FF, D, e1, st))); }
-        if ((rc = resid_ln(PC_FFN2, p.tm_h, m.ff_w2, FF, w.ff_b2, 0.5f, 1, nullptr, 0, 0, w.ln_fin_g, w.ln_fin_b, g2, b2)))
-          return rc;
-      }
+      PROF(PC_FUSED_FFN);
+      // pointwise_conv2 + residual + norm_ff chained in front (z rows of pad frames are zero, bias masked)
+      PPASR_CUDA_CHECK(launch_fused_ffn(p.tm_z, &m.pw2, m.ff_w1_128, m.ff_w2s, Mc, FF, xc, p.y, w.ff_b1, w.ff_b2s, w.ln_fin_g,
+                                        w.ln_fin_b, g2, b2, eps, w.pw2_b, w.ln_ff_g, w.ln_ff_b, vl, Tc, st));
     }
   }
   return PPASR_OK;
@@ -1017,7 +1127,6 @@ int ppasr_b200_encode(ppasr_b200_ctx* c, const float* feats, int32_t feats_on_de
   }
   PPASR_CUDA_CHECK(cudaMemcpyAsync(p.vlen, vlen, sizeof(int) * B, cudaMemcpyHostToDevice, st));
   if (ds2) return run_encoder_ds2(c, st, false);
-  if (c->cfg.model_type == 3) return run_encoder_effconf(c, st);
   return c->cfg.model_type == 1 ? run_encoder_squeezeformer(c, st) : run_encoder(c, st, false);
 }
 
@@ -1139,10 +1248,8 @@ int ppasr_b200_encode_chunk(ppasr_b200_ctx* c, const float* feats, int32_t feats
     std::vector<int> vlen(B, p.Tp);
     PPASR_CUDA_CHECK(cudaMemcpyAsync(p.vlen, vlen.data(), sizeof(int) * B, cudaMemcpyHostToDevice, st));
   }
-  // per-layer cache maps with extent = keys valid after this chunk (TMA zero-fills beyond)
-  std::string err;
-  const int kend_new = ss.kend + p.Tp;
   const bool sqz = cfg.model_type == 1;
+  const int kend_new = ss.kend + p.Tp;
   if (sqz && c->sq.reduce_idx >= 0) {
     // the half-rate blocks address their caches / positions at half rate (runtime_squeezeformer.inl)
     // (an odd number of frames is fine for the LAST chunk of a stream: the state it leaves behind is not used again)
@@ -1150,58 +1257,48 @@ int ppasr_b200_encode_chunk(ppasr_b200_ctx* c, const float* feats, int32_t feats
                       (required_cache_size < 0 || required_cache_size % 2 == 0),
                   "squeezeformer chunk streaming needs even chunk sizes (all but the last chunk) and an even required_cache_size");
   }
-  const bool eff = cfg.model_type == 3;
-  if (eff) {
-    // forward_chunk of the Efficient Conformer: append-only caches (runtime_effconf.inl)
+  if (cfg.model_type == 3) {
+    // forward_chunk of the Efficient Conformer: append-only caches (run_encoder)
     PPASR_REQUIRE(required_cache_size < 0, "efficient_conformer streaming keeps the whole history (required_cache_size < 0, "
                                            "as PPASRPredictor passes, predict.py:304-306)");
     PPASR_REQUIRE(c->eff_stride_idx < 0 || ss.kend % 2 == 0,
                   "efficient_conformer chunk streaming needs even chunk sizes (all but the last chunk of a stream)");
-    if (c->eff_group_mask != 0 && (kend_new + 2) / 3 > 256) {
+    if (c->eff_group_mask != 0 && (kend_new + 2) / 3 > EFF_GCAP) {
       set_last_error("efficient_conformer stream longer than 768 encoder frames (30.7 s): the grouped attention keeps at most "
                      "256 key groups; call reset_stream");
       return PPASR_ERR_STATE;
     }
-    int gi = 0;
-    for (int l = 0; l < L; ++l) {
-      const size_t lk = (size_t)l * B * H * ss.Tcap * 64;
-      const int rate = (c->eff_stride_idx >= 0 && l > c->eff_stride_idx) ? 2 : 1;
-      const int kv = (kend_new + rate - 1) / rate;  // keys valid after this chunk, at the block's rate
-      bool ok;
-      if ((c->eff_group_mask >> l) & 1) {
-        ok = gi < 4 && make_tmap_2d(&ss.tm_k[l], ss.kk + lk, 192, (uint64_t)B * H * 256, 192 * 2, 64, &err) &&
-             make_tmap_2d(&ss.tm_vt[l], ss.vt + lk, (uint64_t)((kv + 2) / 3), (uint64_t)B * H * 192, 256 * 2, 192, &err) &&
-             make_tmap_2d(&ss.tm_pgc[gi], ss.pgc + (size_t)gi * 256 * 768, 768, 256, 768 * 2, 64, &err);
-        if (gi >= 4) err = "more than 4 grouped blocks are not supported";
-        ++gi;
-      } else {
-        ok = make_tmap_2d(&ss.tm_k[l], ss.kk + lk, 64, (uint64_t)B * H * ss.Tcap, 128, 128, &err) &&
-             make_tmap_2d(&ss.tm_vt[l], ss.vt + lk, kv, (uint64_t)B * H * 64, (uint64_t)ss.Tcap * 2, 64, &err);
-      }
-      if (!ok) {
-        set_last_error(err);
-        return PPASR_ERR_CUDA;
-      }
-    }
-    if (c->eff_group_mask != 0 &&
-        !make_tmap_2d(&ss.tm_qgc, p.q2g, 384, (uint64_t)B * H * ((p.Tp + 2) / 3), 384 * 2, 128, &err)) {
-      set_last_error(err);
-      return PPASR_ERR_CUDA;
-    }
-    rc = run_encoder_effconf_chunk(c, st);
-    if (rc) return rc;
-    ss.kend = kend_new;
-    ss.offset += p.Tp;
-    return PPASR_OK;
   }
+  // per-layer cache maps with extent = keys valid after this chunk (TMA zero-fills beyond)
+  std::string err;
+  int gi = 0;
   for (int l = 0; l < L; ++l) {
     const size_t lk = (size_t)l * B * H * ss.Tcap * 64;
-    const int rate = (sqz && c->sq.reduce_idx >= 0 && l >= c->sq.reduce_idx && l < c->sq.recover_idx) ? 2 : 1;
-    if (!make_tmap_2d(&ss.tm_k[l], ss.kk + lk, 64, (uint64_t)B * H * ss.Tcap, 128, 128, &err) ||
-        !make_tmap_2d(&ss.tm_vt[l], ss.vt + lk, (kend_new + rate - 1) / rate, (uint64_t)B * H * 64, (uint64_t)ss.Tcap * 2, 64, &err)) {
+    // half rate: the Squeezeformer's time-reduced section, the blocks after the Efficient Conformer's stride block
+    const bool half = sqz ? (c->sq.reduce_idx >= 0 && l >= c->sq.reduce_idx && l < c->sq.recover_idx)
+                          : (c->eff_stride_idx >= 0 && l > c->eff_stride_idx);
+    const int rate = half ? 2 : 1;
+    const int kv = (kend_new + rate - 1) / rate;  // keys valid after this chunk, at the block's rate
+    bool ok;
+    if ((c->eff_group_mask >> l) & 1) {
+      ok = gi < 4 && make_tmap_2d(&ss.tm_k[l], ss.kk + lk, 192, (uint64_t)B * H * EFF_GCAP, 192 * 2, 64, &err) &&
+           make_tmap_2d(&ss.tm_vt[l], ss.vt + lk, (uint64_t)((kv + 2) / 3), (uint64_t)B * H * 192, EFF_GCAP * 2, 192, &err) &&
+           make_tmap_2d(&ss.tm_pgc[gi], ss.pgc + (size_t)gi * EFF_GCAP * 768, 768, EFF_GCAP, 768 * 2, 64, &err);
+      if (gi >= 4) err = "more than 4 grouped blocks are not supported";
+      ++gi;
+    } else {
+      ok = make_tmap_2d(&ss.tm_k[l], ss.kk + lk, 64, (uint64_t)B * H * ss.Tcap, 128, 128, &err) &&
+           make_tmap_2d(&ss.tm_vt[l], ss.vt + lk, kv, (uint64_t)B * H * 64, (uint64_t)ss.Tcap * 2, 64, &err);
+    }
+    if (!ok) {
       set_last_error(err);
       return PPASR_ERR_CUDA;
     }
+  }
+  if (c->eff_group_mask != 0 &&
+      !make_tmap_2d(&ss.tm_qgc, p.q2g, 384, (uint64_t)B * H * ((p.Tp + 2) / 3), 384 * 2, 128, &err)) {
+    set_last_error(err);
+    return PPASR_ERR_CUDA;
   }
   rc = sqz ? run_encoder_squeezeformer(c, st, true) : run_encoder(c, st, true);
   if (rc) return rc;
@@ -1360,7 +1457,7 @@ static int run_ctc_logits(ppasr_b200_ctx* c, cudaStream_t st) {
   Plan& p = c->plan;
   EpiLogitsF32<BN_NARROW> e{p.logits, c->ctc_b, c->Vld, p.Mc, c->cfg.vocab_size};
   PROF(PC_CTC_LOGITS);
-  PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, c->tm_ctc_w, p.Mc, c->cfg.vocab_size, c->ctc_k ? c->ctc_k : c->cfg.d_model, e, st)));
+  PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, c->tm_ctc_w, p.Mc, c->cfg.vocab_size, c->ctc_k, e, st)));
   return PPASR_OK;
 }
 
@@ -1402,7 +1499,7 @@ int ppasr_b200_ctc_greedy(ppasr_b200_ctx* c, int32_t* ids, int32_t* out_lens, fl
   const int V = c->cfg.vocab_size;
   EpiCtcStats<BN_NARROW> e{p.pmax, p.parg, p.psum, c->ctc_b, p.Mc, V, c->ctc_parts};
   { PROF(PC_CTC_STATS);
-  PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, c->tm_ctc_w, p.Mc, V, c->ctc_k ? c->ctc_k : c->cfg.d_model, e, st))); }
+  PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, c->tm_ctc_w, p.Mc, V, c->ctc_k, e, st))); }
   { PROF(PC_CTC_FINALIZE);
   PPASR_CUDA_CHECK(launch_ctc_stats_finalize(p.pmax, p.parg, p.psum, c->ctc_parts, p.Mc, p.idx, p.maxp, st)); }
   PROF(PC_CTC_COLLAPSE);
@@ -1473,10 +1570,6 @@ int32_t ppasr_b200_graph_kernels(const ppasr_b200_ctx* c) { return c ? (int32_t)
 int ppasr_b200_set_option(ppasr_b200_ctx* c, const char* name, int32_t value) {
   PPASR_REQUIRE(c && name, "null pointer");
   const std::string n(name);
-  if (n == "fused_ffn") {
-    c->fused_ffn = value != 0;
-    return PPASR_OK;
-  }
   if (n == "host_sync") {
     c->host_sync = value != 0;
     return PPASR_OK;
@@ -1492,10 +1585,6 @@ int ppasr_b200_set_option(ppasr_b200_ctx* c, const char* name, int32_t value) {
   if (n == "fused_conv") {
     PPASR_REQUIRE(value == 0 || value == 2, "fused_conv must be 0 or 2");
     c->fused_conv = value;
-    return PPASR_OK;
-  }
-  if (n == "fused_attn_out") {
-    c->fused_attn_out = value != 0;
     return PPASR_OK;
   }
   set_last_error("unknown option: " + n);

@@ -544,9 +544,9 @@ def test_c_abi_create_validates_configs_without_a_gpu():
     lib.ppasr_b200_destroy(ctx)
 
 
-def test_c_abi_state_errors_and_host_helpers_without_a_gpu():
-    """Calls in the wrong state fail with a status + message before touching the device; the sizing / naming helpers are
-    pure host code."""
+def test_c_abi_state_errors_option_names_and_host_helpers_without_a_gpu():
+    """Calls in the wrong state fail with a status + message before touching the device; set_option accepts the current
+    switches and rejects removed ones; the sizing / naming helpers are pure host code."""
     import ctypes
     from ppasr_b200 import _lib as L
     lib = L.load()
@@ -560,10 +560,11 @@ def test_c_abi_state_errors_and_host_helpers_without_a_gpu():
     out = np.zeros((1, 16, 50), np.float32)
     assert lib.ppasr_b200_ctc_logits(ctx, out.ctypes.data_as(ctypes.c_void_p), 0, None) != 0
     assert "encode first" in lib.ppasr_b200_last_error().decode()
-    assert lib.ppasr_b200_set_option(ctx, b"fused_ffn", 0) == 0 and lib.ppasr_b200_set_option(ctx, b"fused_ffn", 1) == 0
+    assert lib.ppasr_b200_set_option(ctx, b"host_sync", 0) == 0 and lib.ppasr_b200_set_option(ctx, b"host_sync", 1) == 0
     assert lib.ppasr_b200_set_option(ctx, b"no_such_option", 1) != 0
-    assert lib.ppasr_b200_set_option(None, b"fused_ffn", 1) != 0
-    for gone in (b"qkv_wide", b"qkv_co", b"fused_dwconv", b"attn_out_v2"):  # removed kernel variants
+    assert lib.ppasr_b200_set_option(None, b"host_sync", 1) != 0
+    # removed kernel variants and unfused paths
+    for gone in (b"qkv_wide", b"qkv_co", b"fused_dwconv", b"attn_out_v2", b"fused_ffn", b"fused_attn_out"):
         assert lib.ppasr_b200_set_option(ctx, gone, 1) != 0 and "unknown option" in lib.ppasr_b200_last_error().decode()
     assert lib.ppasr_b200_set_option(ctx, b"fused_conv", 0) == 0 and lib.ppasr_b200_set_option(ctx, b"fused_conv", 2) == 0
     assert lib.ppasr_b200_set_option(ctx, b"fused_conv", 1) != 0
