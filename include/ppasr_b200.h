@@ -222,6 +222,13 @@ int ppasr_b200_op_fused_ffn(const void* y_bf16, const void* w1_bf16, const void*
 int ppasr_b200_op_attention(const void* q2, const void* kk, const void* vt, int32_t T2p, const void* pos,
                             int32_t pos_rows, int32_t pos_ld, int32_t pos_row0, int32_t pos_col0, void* out,
                             int32_t B, int32_t H, int32_t T1, int32_t T2, const int32_t* klens, void* stream);
+/* grouped rel-pos attention of the Efficient Conformer (group size 3, 4 heads x 192) on the operand layouts the grouped QKV
+ * epilogue writes: q2g [B,H,ceil(T/3),384] = [q+u | q+v], kk [B,H,k_pitch,192], vt [B,H,192,vt_pitch] (vt_pitch % 8 == 0),
+ * pos [Tgk,768] (all bf16) -> out bf16 [B*T,256]. Tgk key groups (<= k_pitch, vt_pitch; any count), klens nullable int32 [B]
+ * valid key FRAMES per utterance. Offline: Tgk = k_pitch = ceil(T/3); streaming: k_pitch = the cache's group capacity. */
+int ppasr_b200_op_grouped_attention(const void* q2g, const void* kk, int32_t k_pitch, const void* vt, int32_t vt_pitch,
+                                    const void* pos, void* out, int32_t B, int32_t H, int32_t T, int32_t Tgk,
+                                    const int32_t* klens, void* stream);
 
 /* ---- front end (the step before the hot path; SURVEY 8f rank 1) ----------------------------------------
  * replaces: AudioFeaturizer.featurize for feature_method 'fbank' (data_utils/featurizer/audio_featurizer.py:37-69,120-138):

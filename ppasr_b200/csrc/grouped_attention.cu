@@ -6,14 +6,19 @@
 //   keys g with 3g >= len are masked (mask[:, ::3, ::3]);  out = softmax(S) V, re-viewed as frames and trimmed to T.
 // As in attention.cu the two score terms are one contraction [q+u | q+v] . [k | p]^T, here over K = 384.
 //
-// Sequences are short (ceil(T'/3) <= 256 groups for 30 s of audio), so one CTA per (128-query tile, head, utterance)
-// keeps the WHOLE score row in TMEM: S blocks of 64 keys in columns [0,256), O in [256,448). The soft-max is a plain
-// two-pass one (global row maximum, then probabilities block by block feeding P.V with accumulation in TMEM); no
-// online rescaling and no 192-float output registers per thread.
+// One CTA per (128-query tile, head, utterance). TMEM holds four 64-column score slots in [0,256) and O in [256,448). The
+// soft-max is a plain two-pass one (global row maximum, then probabilities block by block feeding P.V with accumulation in
+// TMEM); no online rescaling and no 192-float output registers per thread.
 //   control thread : TMA Q (6 tiles), per 64-key block K|P (6 tiles) -> 24 x tcgen05.mma 128x64x16 -> S_j
 //   128 softmax thr: row max over all blocks; per block exp2 -> bf16 probabilities -> swizzled smem tile
 //   control thread : TMA V^T_j [192 x 64] -> 4 x tcgen05.mma 128x192x16, O += P_j V_j
 //   128 softmax thr: O / l -> bf16, stored at frame t = 3g + i/256, column i%256 (i = h*192 + d), rows t >= T dropped
+// Two paths, chosen by the number of 64-key blocks nblk:
+//   resident  (nblk <= 4, up to 256 key groups = 768 frames): every S_j stays in its slot and is scored once.
+//   recompute (nblk > 4): pass 1 streams S_j through the slots as a ring (the softmax threads hand a slot back through
+//             bar_sf once its maximum is read); pass 2 re-issues the K|P loads and S_j MMAs into the same ring, a few blocks
+//             ahead of P.V. The per-block probabilities, P.V and lsum order are the resident path's, so for the same S it
+//             gives what the resident path would with unbounded TMEM, at one extra QK^T (K = 384) per block.
 #include "kernels.h"
 #include "launch.h"
 #include "ptx.cuh"
@@ -22,7 +27,7 @@ namespace ppasr {
 
 void count_launch();
 
-constexpr int GA_MAX_BLOCKS = 4;               // 256 key groups
+constexpr int GA_SLOTS = 4;                    // 64-column score slots in TMEM (256 key groups resident)
 constexpr int GA_THREADS = 160;
 constexpr int GA_QT = 128 * 64 * 2;            // [128 x 64] tile, 16 KB
 constexpr int GA_KT = 64 * 64 * 2;             // [64 x 64] tile, 8 KB
@@ -48,8 +53,9 @@ grouped_attention_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_
   uint64_t* bar_v = bar_q + 2;
   uint64_t* bar_p = bar_q + 3;      // probabilities of block j written (128 arrivals)
   uint64_t* bar_pv = bar_q + 4;     // P.V of block j complete (P tile and V smem free)
-  uint64_t* bar_s = bar_q + 5;      // [GA_MAX_BLOCKS] single-use: S_j complete (also: K|P smem free)
-  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bar_q + 5 + GA_MAX_BLOCKS);
+  uint64_t* bar_s = bar_q + 5;      // [GA_SLOTS] S in slot s complete (also: K|P smem free); one phase per use of the slot
+  uint64_t* bar_sf = bar_s + GA_SLOTS;  // [GA_SLOTS] recompute path: the softmax threads have read slot s (128 arrivals)
+  uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bar_sf + GA_SLOTS);
 
   const int warp_idx = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -60,6 +66,7 @@ grouped_attention_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_
   const int kpitch = p.k_pitch > 0 ? p.k_pitch : p.Tg;
   const int klen = p.klens ? min(Tgk, (__ldg(p.klens + b) + 2) / 3) : Tgk;  // keys g with 3g < len
   const int nblk = (Tgk + 63) / 64;
+  const bool resident = nblk <= GA_SLOTS;  // the whole score row fits the slots: each S_j is computed once
 
   if (warp_idx == 4) {
     if (elect_one()) {
@@ -69,7 +76,7 @@ grouped_attention_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_
       tma_prefetch_desc(&tm_vt);
       mbar_init(bar_q, 1);
       mbar_init(bar_kp, 1);
-      for (int i = 0; i < GA_MAX_BLOCKS; ++i) mbar_init(bar_s + i, 1);
+      for (int i = 0; i < GA_SLOTS; ++i) mbar_init(bar_s + i, 1), mbar_init(bar_sf + i, 128);
       mbar_init(bar_v, 1);
       mbar_init(bar_p, 128);
       mbar_init(bar_pv, 1);
@@ -94,29 +101,31 @@ grouped_attention_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_
       constexpr uint32_t idesc_o = umma_idesc_bf16(128, 192);
       mbar_arrive_expect_tx(bar_q, 6 * GA_QT);
       for (int kt = 0; kt < 6; ++kt) tma_load_2d(s_q + kt * GA_QT, &tm_q, bar_q, kt * 64, bh * p.Tg + row0);
-      // ---- scores ----
-      for (int j = 0; j < nblk; ++j) {
+      // the n-th score issue computes S_j into slot n % GA_SLOTS (n = j in pass 1, nblk + j in pass 2)
+      auto issue_s = [&](int n, int j) {
+        const int slot = n % GA_SLOTS;
+        if (n > 0) mbar_wait(bar_s + (n - 1) % GA_SLOTS, ((n - 1) / GA_SLOTS) & 1);  // MMAs reading K|P of issue n-1 done
+        if (n >= GA_SLOTS) mbar_wait(bar_sf + slot, (n / GA_SLOTS - 1) & 1);      // the slot's previous block was read
         const int k0 = j * 64;
-        if (j > 0) mbar_wait(bar_s + j - 1, 0);  // MMAs reading the K|P tiles of block j-1 are done
         mbar_arrive_expect_tx(bar_kp, 6 * GA_KT);
         for (int kt = 0; kt < 3; ++kt) {
           tma_load_2d(s_kp + kt * GA_KT, &tm_k, bar_kp, kt * 64, bh * kpitch + k0);
           tma_load_2d(s_kp + (3 + kt) * GA_KT, &tm_p, bar_kp, h * 192 + kt * 64, k0);
         }
-        if (j == 0) mbar_wait(bar_q, 0);
-        mbar_wait(bar_kp, j & 1);
+        if (n == 0) mbar_wait(bar_q, 0);
+        mbar_wait(bar_kp, n & 1);
         tc_fence_after();
         const uint32_t qa = smem_u32(s_q), ka = smem_u32(s_kp);
 #pragma unroll
         for (int kt = 0; kt < 6; ++kt)
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            umma_bf16(tmem_s + j * 64, umma_desc_k_sw128(qa + kt * GA_QT + k * 32), umma_desc_k_sw128(ka + kt * GA_KT + k * 32),
+            umma_bf16(tmem_s + slot * 64, umma_desc_k_sw128(qa + kt * GA_QT + k * 32), umma_desc_k_sw128(ka + kt * GA_KT + k * 32),
                       idesc_s, (kt | k) != 0);
-        umma_commit(bar_s + j);
-      }
-      // ---- P.V ----
-      for (int j = 0; j < nblk; ++j) {
+        umma_commit(bar_s + slot);
+      };
+      // O += P_j V_j
+      auto issue_pv = [&](int j) {
         if (j > 0) mbar_wait(bar_pv, (j - 1) & 1);
         mbar_arrive_expect_tx(bar_v, 192 * 64 * 2);
         tma_load_2d(s_v, &tm_vt, bar_v, j * 64, bh * 192);
@@ -128,6 +137,18 @@ grouped_attention_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_
         for (int k = 0; k < 4; ++k)
           umma_bf16(tmem_o, umma_desc_k_sw128(pa + k * 32), umma_desc_k_sw128(va + k * 32), idesc_o, (j | k) != 0);
         umma_commit(bar_pv);
+      };
+      // ---- pass 1: scores (kept in their slots when resident, streamed through the ring for the row maximum otherwise)
+      for (int j = 0; j < nblk; ++j) issue_s(j, j);
+      // ---- pass 2: P.V (recompute: S_j re-issued up to GA_SLOTS - 1 blocks ahead of the P.V that consumes it)
+      if (resident) {
+        for (int j = 0; j < nblk; ++j) issue_pv(j);
+      } else {
+        int n = nblk;
+        for (int j = 0; j < nblk; ++j) {
+          for (; n < 2 * nblk && n - nblk < j + GA_SLOTS; ++n) issue_s(n, n - nblk);
+          issue_pv(j);
+        }
       }
     }
   } else {
@@ -135,26 +156,40 @@ grouped_attention_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_
     const int r = quad * 32 + lane;
     const uint32_t lane_base = ((uint32_t)(quad * 32)) << 16;
     const float sc = 0.07216878364870322f * 1.4426950408889634f;  // 1/sqrt(192) * log2(e)
-    // all score blocks complete
-    for (int j = 0; j < nblk; ++j) mbar_wait(bar_s + j, 0);
-    tc_fence_after();
+    // ---- pass 1: row maximum over all key blocks
     float mx = -INFINITY;
-#pragma unroll 1
-    for (int c = 0; c < nblk * 2; ++c) {
-      uint32_t rr[32];
-      tmem_ld_32x32b_x32(tmem_s + lane_base + c * 32, rr);
-      tmem_ld_wait();
-#pragma unroll
-      for (int i = 0; i < 32; ++i) mx = fmaxf(mx, (c * 32 + i) < klen ? __uint_as_float(rr[i]) : -INFINITY);
-    }
-    const float m_use = (mx == -INFINITY) ? 0.f : mx * sc;
-    float lsum = 0.f;
     for (int j = 0; j < nblk; ++j) {
-      if (j > 0) mbar_wait(bar_pv, (j - 1) & 1);  // the probability tile is free again
+      const int slot = j % GA_SLOTS;
+      mbar_wait(bar_s + slot, (j / GA_SLOTS) & 1);
+      tc_fence_after();
 #pragma unroll 1
       for (int c = 0; c < 2; ++c) {
         uint32_t rr[32];
-        tmem_ld_32x32b_x32(tmem_s + lane_base + j * 64 + c * 32, rr);
+        tmem_ld_32x32b_x32(tmem_s + lane_base + slot * 64 + c * 32, rr);
+        tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 32; ++i) mx = fmaxf(mx, (j * 64 + c * 32 + i) < klen ? __uint_as_float(rr[i]) : -INFINITY);
+      }
+      if (!resident) {
+        tc_fence_before();
+        mbar_arrive(bar_sf + slot);
+      }
+    }
+    const float m_use = (mx == -INFINITY) ? 0.f : mx * sc;
+    // ---- pass 2: probabilities block by block, in key order
+    float lsum = 0.f;
+    for (int j = 0; j < nblk; ++j) {
+      if (j > 0) mbar_wait(bar_pv, (j - 1) & 1);  // the probability tile is free again
+      int slot = j;
+      if (!resident) {
+        slot = (nblk + j) % GA_SLOTS;
+        mbar_wait(bar_s + slot, ((nblk + j) / GA_SLOTS) & 1);
+        tc_fence_after();
+      }
+#pragma unroll 1
+      for (int c = 0; c < 2; ++c) {
+        uint32_t rr[32];
+        tmem_ld_32x32b_x32(tmem_s + lane_base + slot * 64 + c * 32, rr);
         tmem_ld_wait();
         uint32_t pk[16];
 #pragma unroll
@@ -175,6 +210,7 @@ grouped_attention_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_
         }
       }
       tc_fence_before();
+      if (!resident) mbar_arrive(bar_sf + slot);  // slot read (tmem_ld_wait above): pass 2 may overwrite it
       fence_proxy_async_smem();
       mbar_arrive(bar_p);
     }
@@ -214,7 +250,7 @@ grouped_attention_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_
 
 cudaError_t launch_grouped_attention(const CUtensorMap& tm_q, const CUtensorMap& tm_k, const CUtensorMap& tm_p,
                                      const CUtensorMap& tm_vt, const GroupedAttnParams& p, cudaStream_t st) {
-  if (p.Tg > GA_MAX_BLOCKS * 64 || p.Tgk > GA_MAX_BLOCKS * 64 || p.H != 4) return cudaErrorInvalidValue;
+  if (p.H != 4) return cudaErrorInvalidValue;  // any key length: more than GA_SLOTS key blocks take the recompute path
   static bool configured = false;
   if (!configured) {
     cudaError_t e = cudaFuncSetAttribute(grouped_attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, GA_SMEM_TOTAL);

@@ -185,8 +185,12 @@ struct ppasr_b200_ctx {
     __nv_bfloat16* vt = nullptr;   // [L][B,H,64,Tcap]
     __nv_bfloat16* cnn = nullptr;  // [L][B,lorder,D]
     std::vector<CUtensorMap> tm_k, tm_vt;  // per layer, rebuilt every chunk (extent = kend)
-    // Efficient Conformer streaming: positional operands of the (<= 4) grouped blocks [4][256 groups][768], rebuilt per
-    // chunk, and the map of this chunk's grouped queries
+    // Efficient Conformer streaming: the grouped blocks keep K [B,H,Gcap,192] / V^T [B,H,192,Gcap] in their layer slices;
+    // groups at or past gdirty have been zero since the caches were last cleared (stream_reset zeroes [0, gdirty) only)
+    int Gcap = 0;
+    int gdirty = 0;
+    // positional operands of the (<= 4) grouped blocks [4][Gcap][768], rebuilt per chunk, and the map of this chunk's
+    // grouped queries
     __nv_bfloat16* pgc = nullptr;
     CUtensorMap tm_pgc[4], tm_qgc;
     // ragged sessions (ppasr_b200_sessions_*): every cache slot is an independent stream with its own positions
@@ -922,8 +926,6 @@ int run_subsampling_convs(ppasr_b200_ctx* c, cudaStream_t st) {
 #include "runtime_squeezeformer.inl"
 #include "runtime_ds2.inl"
 
-constexpr int EFF_GCAP = 256;  // key groups a grouped block can attend (grouped_attention_kernel keeps the score row in TMEM)
-
 // Conformer (model_type 0) and Efficient Conformer (model_type 3): the pre-norm macaron block on the fused kernels.
 // Reference: conformer/encoder.py:164-206 (forward), :380-429 (block); efficient_conformer/encoder.py:212-264 (forward),
 // :455-548 (stride block), attention.py:128-193 (grouped attention), convolution.py:80-138 (strided conv module).
@@ -996,12 +998,12 @@ int run_encoder(ppasr_b200_ctx* c, cudaStream_t st, bool chunk) {
     } else if (grouped) {
       // positional operand of the T2 keys at positions j * rate, zero beyond T2 inside the last group
       const int T2 = cache_t + Tc, G2 = (T2 + 2) / 3;
-      PPASR_CUDA_CHECK(launch_grouped_pos(c->pos_tab, L * D * rate, l * D, T2, 3 * G2, ss.pgc + (size_t)gi * EFF_GCAP * 768, st));
-      EpiQKVGrouped<BN_NARROW> e{p.q2g, ss.kk + lk, ss.vt + lk, w.bqkv, w.pos_u, w.pos_v, Mc, Tc, H, (Tc + 2) / 3, EFF_GCAP};
-      e.kofs = kend, e.Tgk = EFF_GCAP;
+      PPASR_CUDA_CHECK(launch_grouped_pos(c->pos_tab, L * D * rate, l * D, T2, 3 * G2, ss.pgc + (size_t)gi * ss.Gcap * 768, st));
+      EpiQKVGrouped<BN_NARROW> e{p.q2g, ss.kk + lk, ss.vt + lk, w.bqkv, w.pos_u, w.pos_v, Mc, Tc, H, (Tc + 2) / 3, ss.Gcap};
+      e.kofs = kend, e.Tgk = ss.Gcap;
       { PROF(PC_QKV); PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, Mc, 3 * D, D, e, st))); }
       GroupedAttnParams gp{B, H, Tc, (Tc + 2) / 3, nullptr, p.att};
-      gp.Tgk = G2, gp.k_pitch = EFF_GCAP;
+      gp.Tgk = G2, gp.k_pitch = ss.Gcap;
       { PROF(PC_ATTENTION); PPASR_CUDA_CHECK(launch_grouped_attention(ss.tm_qgc, ss.tm_k[l], ss.tm_pgc[gi], ss.tm_vt[l], gp, st)); }
       ++gi;
     } else {
@@ -1178,6 +1180,15 @@ int ppasr_b200_stream_reset(ppasr_b200_ctx* c, int32_t B) {
     if (ss.cnn) cudaFree(ss.cnn);
     ss.kk = ss.vt = ss.cnn = nullptr;
     ss.Tcap = (cfg.max_len + 63) / 64 * 64;
+    if (cfg.model_type == 3) {
+      // grouped blocks: the key groups of the longest stream (kend < max_len frames, full rate), a multiple of 8 so the
+      // V^T row pitch is a multiple of 16 bytes (TMA); their K / V^T views must fit the layer's slice of B*H*Tcap*64
+      ss.Gcap = ((cfg.max_len + 1) / 3 + 7) / 8 * 8;
+      ss.Tcap = std::max(ss.Tcap, (3 * ss.Gcap + 63) / 64 * 64);
+      PPASR_REQUIRE((size_t)ss.Gcap * 192 <= (size_t)ss.Tcap * 64 && ss.Gcap * 2 % 16 == 0 && 3 * ss.Gcap >= cfg.max_len - 1,
+                    "internal error: grouped cache capacity");
+    }
+    ss.gdirty = 0;
     const size_t n = (size_t)L * B * H * ss.Tcap * 64;
     PPASR_CUDA_CHECK(cudaMalloc(&ss.kk, n * 2));
     PPASR_CUDA_CHECK(cudaMalloc(&ss.vt, n * 2));
@@ -1191,18 +1202,22 @@ int ppasr_b200_stream_reset(ppasr_b200_ctx* c, int32_t B) {
   // empty conv cache == the reference's zero left padding of the first chunk (convolution.py:109-110)
   PPASR_CUDA_CHECK(cudaMemset(ss.cnn, 0, (size_t)L * B * lorder * D * 2));
   if (cfg.model_type == 3) {
-    // grouped blocks append into zeroed caches: the missing frames of a partially filled last group must read as zero
-    PPASR_REQUIRE(ss.Tcap >= 768, "efficient_conformer streaming needs max_len >= 768");
-    // only the grouped blocks read beyond what was written (their K [B*H*256, 192] / V^T [B*H*192, 256] views are the
-    // first B*H*49152 elements of the block's slice); the plain blocks are bounded by the tensor-map extents
-    const size_t slice = (size_t)B * H * ss.Tcap * 64, gview = (size_t)B * H * 256 * 192;
-    for (int l = 0; l < L; ++l) {
+    // grouped blocks append into zeroed caches: the missing frames of a partially filled last group must read as zero.
+    // Only the grouped blocks read beyond what was written (the plain blocks are bounded by the tensor-map extents), and
+    // only groups [0, gdirty) of each (b, h) have been written since the caches were last zero, so only those are cleared:
+    // the leading gdirty of every Gcap-group K row block and of every V^T row
+    const size_t slice = (size_t)B * H * ss.Tcap * 64;
+    for (int l = 0; l < L && ss.gdirty > 0; ++l) {
       if (!((c->eff_group_mask >> l) & 1)) continue;
-      PPASR_CUDA_CHECK(cudaMemset(ss.kk + (size_t)l * slice, 0, gview * 2));
-      PPASR_CUDA_CHECK(cudaMemset(ss.vt + (size_t)l * slice, 0, gview * 2));
+      PPASR_CUDA_CHECK(cudaMemset2D(ss.kk + (size_t)l * slice, (size_t)ss.Gcap * 192 * 2, 0, (size_t)ss.gdirty * 192 * 2,
+                                    (size_t)B * H));
+      PPASR_CUDA_CHECK(cudaMemset2D(ss.vt + (size_t)l * slice, (size_t)ss.Gcap * 2, 0, (size_t)ss.gdirty * 2, (size_t)B * H * 192));
     }
-    if (!ss.pgc) PPASR_CUDA_CHECK(cudaMalloc(&ss.pgc, (size_t)4 * 256 * 768 * 2));
-    PPASR_CUDA_CHECK(cudaMemset(ss.pgc, 0, (size_t)4 * 256 * 768 * 2));
+    ss.gdirty = 0;
+    if (!ss.pgc) {  // rows past a chunk's keys are masked; zero them once so they hold finite values
+      PPASR_CUDA_CHECK(cudaMalloc(&ss.pgc, (size_t)4 * ss.Gcap * 768 * 2));
+      PPASR_CUDA_CHECK(cudaMemset(ss.pgc, 0, (size_t)4 * ss.Gcap * 768 * 2));
+    }
   }
   ss.kstart = ss.kend = ss.offset = 0;
   return PPASR_OK;
@@ -1263,11 +1278,7 @@ int ppasr_b200_encode_chunk(ppasr_b200_ctx* c, const float* feats, int32_t feats
                                            "as PPASRPredictor passes, predict.py:304-306)");
     PPASR_REQUIRE(c->eff_stride_idx < 0 || ss.kend % 2 == 0,
                   "efficient_conformer chunk streaming needs even chunk sizes (all but the last chunk of a stream)");
-    if (c->eff_group_mask != 0 && (kend_new + 2) / 3 > EFF_GCAP) {
-      set_last_error("efficient_conformer stream longer than 768 encoder frames (30.7 s): the grouped attention keeps at most "
-                     "256 key groups; call reset_stream");
-      return PPASR_ERR_STATE;
-    }
+    ss.gdirty = std::max(ss.gdirty, (kend_new + 2) / 3);  // groups this chunk's grouped QKV epilogues write into
   }
   // per-layer cache maps with extent = keys valid after this chunk (TMA zero-fills beyond)
   std::string err;
@@ -1281,9 +1292,9 @@ int ppasr_b200_encode_chunk(ppasr_b200_ctx* c, const float* feats, int32_t feats
     const int kv = (kend_new + rate - 1) / rate;  // keys valid after this chunk, at the block's rate
     bool ok;
     if ((c->eff_group_mask >> l) & 1) {
-      ok = gi < 4 && make_tmap_2d(&ss.tm_k[l], ss.kk + lk, 192, (uint64_t)B * H * EFF_GCAP, 192 * 2, 64, &err) &&
-           make_tmap_2d(&ss.tm_vt[l], ss.vt + lk, (uint64_t)((kv + 2) / 3), (uint64_t)B * H * 192, EFF_GCAP * 2, 192, &err) &&
-           make_tmap_2d(&ss.tm_pgc[gi], ss.pgc + (size_t)gi * EFF_GCAP * 768, 768, EFF_GCAP, 768 * 2, 64, &err);
+      ok = gi < 4 && make_tmap_2d(&ss.tm_k[l], ss.kk + lk, 192, (uint64_t)B * H * ss.Gcap, 192 * 2, 64, &err) &&
+           make_tmap_2d(&ss.tm_vt[l], ss.vt + lk, (uint64_t)((kv + 2) / 3), (uint64_t)B * H * 192, (uint64_t)ss.Gcap * 2, 192, &err) &&
+           make_tmap_2d(&ss.tm_pgc[gi], ss.pgc + (size_t)gi * ss.Gcap * 768, 768, ss.Gcap, 768 * 2, 64, &err);
       if (gi >= 4) err = "more than 4 grouped blocks are not supported";
       ++gi;
     } else {
@@ -1679,6 +1690,28 @@ int ppasr_b200_op_attention(const void* q2, const void* kk, const void* vt, int3
   ap.B = B, ap.H = H, ap.T1 = T1, ap.T2 = T2, ap.q_rows_per_bh = T1, ap.k_rows_per_bh = T2, ap.k_row0 = 0;
   ap.pos_row0 = pos_row0, ap.pos_col0 = pos_col0, ap.D = H * 64, ap.klens = klens, ap.out = (__nv_bfloat16*)out;
   PPASR_CUDA_CHECK(launch_rel_attention(tq, tk, tp, tv, ap, reinterpret_cast<cudaStream_t>(stream)));
+  return PPASR_OK;
+}
+
+int ppasr_b200_op_grouped_attention(const void* q2g, const void* kk, int32_t k_pitch, const void* vt, int32_t vt_pitch,
+                                    const void* pos, void* out, int32_t B, int32_t H, int32_t T, int32_t Tgk,
+                                    const int32_t* klens, void* stream) {
+  PPASR_REQUIRE(q2g && kk && vt && pos && out, "null pointer");
+  PPASR_REQUIRE(B > 0 && H == 4 && T > 0 && Tgk > 0 && k_pitch >= Tgk && vt_pitch >= Tgk, "bad shape (H must be 4)");
+  PPASR_REQUIRE(vt_pitch % 8 == 0, "vt_pitch must be a multiple of 8");
+  const int Tg = (T + 2) / 3;
+  std::string err;
+  CUtensorMap tq, tk, tp, tv;
+  if (!make_tmap_2d(&tq, q2g, 384, (uint64_t)B * H * Tg, 384 * 2, 128, &err) ||
+      !make_tmap_2d(&tk, kk, 192, (uint64_t)B * H * k_pitch, 192 * 2, 64, &err) ||
+      !make_tmap_2d(&tp, pos, 768, Tgk, 768 * 2, 64, &err) ||
+      !make_tmap_2d(&tv, vt, Tgk, (uint64_t)B * H * 192, (uint64_t)vt_pitch * 2, 192, &err)) {
+    set_last_error(err);
+    return PPASR_ERR_CUDA;
+  }
+  GroupedAttnParams gp{B, H, T, Tg, klens, (__nv_bfloat16*)out};
+  gp.Tgk = Tgk, gp.k_pitch = k_pitch;
+  PPASR_CUDA_CHECK(launch_grouped_attention(tq, tk, tp, tv, gp, reinterpret_cast<cudaStream_t>(stream)));
   return PPASR_OK;
 }
 

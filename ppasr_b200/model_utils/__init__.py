@@ -139,8 +139,8 @@ class SqueezeformerModel(_HotPathModel):
 class EfficientConformerModel(_HotPathModel):
     """efficient_conformer/model.py:16-63,147-183. get_encoder_out_chunk (forward_chunk, encoder.py:266-394) keeps its
     append-only grouped / half-rate caches on the device (run_encoder in csrc/runtime.cu); like the Squeezeformer the caller gets
-    opaque continuation tokens instead of the reference's cache tensors. Streams are limited to 768 encoder frames (30.7 s)
-    between reset_stream() calls and need required_cache_size < 0 (what PPASRPredictor passes, predict.py:304-306)."""
+    opaque continuation tokens instead of the reference's cache tensors. Streams run up to max_len encoder frames between
+    reset_stream() calls and need required_cache_size < 0 (what PPASRPredictor passes, predict.py:304-306)."""
     use_model = "efficient_conformer"
 
 
