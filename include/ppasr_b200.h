@@ -222,6 +222,14 @@ int ppasr_b200_op_fused_ffn(const void* y_bf16, const void* w1_bf16, const void*
 int ppasr_b200_op_attention(const void* q2, const void* kk, const void* vt, int32_t T2p, const void* pos,
                             int32_t pos_rows, int32_t pos_ld, int32_t pos_row0, int32_t pos_col0, void* out,
                             int32_t B, int32_t H, int32_t T1, int32_t T2, const int32_t* klens, void* stream);
+/* QKV projection + rel-pos attention of one offline block (D = 256, H = 4): y [B*T,256] bf16 (the LayerNorm output),
+ * wqkv [768,256] bf16 (K-major rows: q, k, v; row = h*64 + d inside each), bqkv fp32 [768], pos_u / pos_v fp32 [256],
+ * pos [pos_rows, pos_ld] bf16 with key 0 at row pos_row0 and the block's columns from pos_col0 -> out bf16 [B*T,256];
+ * klens nullable int32 [B]. fused != 0 runs qkv_rel_attention_kernel (1 <= T <= 256, otherwise an error), fused = 0 the
+ * QKV GEMM + rel_attention_kernel pair on scratch operands; the two give the same bits. */
+int ppasr_b200_op_qkv_attention(const void* y, const void* wqkv, const float* bqkv, const float* pos_u, const float* pos_v,
+                                const void* pos, int32_t pos_rows, int32_t pos_ld, int32_t pos_row0, int32_t pos_col0,
+                                const int32_t* klens, int32_t B, int32_t T, void* out, int32_t fused, void* stream);
 /* grouped rel-pos attention of the Efficient Conformer (group size 3, 4 heads x 192) on the operand layouts the grouped QKV
  * epilogue writes: q2g [B,H,ceil(T/3),384] = [q+u | q+v], kk [B,H,k_pitch,192], vt [B,H,192,vt_pitch] (vt_pitch % 8 == 0),
  * pos [Tgk,768] (all bf16) -> out bf16 [B*T,256]. Tgk key groups (<= k_pitch, vt_pitch; any count), klens nullable int32 [B]

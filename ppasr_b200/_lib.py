@@ -88,6 +88,7 @@ PROTOTYPES = {
     "ppasr_b200_op_softmax": (c_int, [P, I, P, I, I, P]),
     "ppasr_b200_op_fused_ffn": (c_int, [P, P, P, P, P, P, P, P, P, P, P, I, I, c_float, P]),
     "ppasr_b200_op_attention": (c_int, [P, P, P, I, P, I, I, I, I, P, I, I, I, I, P, P]),
+    "ppasr_b200_op_qkv_attention": (c_int, [P, P, P, P, P, P, I, I, I, I, P, I, I, P, I, P]),
     "ppasr_b200_op_grouped_attention": (c_int, [P, P, I, P, I, P, P, I, I, I, I, P, P]),
     "ppasr_b200_debug_copy_x": (c_int, [P, P, P]),
     "ppasr_b200_debug_copy_phase": (c_int, [P, P, P, P]),

@@ -155,6 +155,23 @@ struct AttnParams {
 cudaError_t launch_rel_attention(const CUtensorMap& tm_q, const CUtensorMap& tm_k, const CUtensorMap& tm_p,
                                  const CUtensorMap& tm_vt, const AttnParams& p, cudaStream_t st);
 
+// QKV projection + relative-position attention in one kernel (attention.cu, offline blocks): one CTA per (head, utterance)
+// projects y [B*T, D] with the head's rows of the packed wqkv and attends over the utterance's T keys. tm_y: the y map of the
+// QKV GEMM (box 128 rows); tm_w: wqkv [3D, D] with a 64-row box; tm_p: the positional table (box 128 rows).
+// Only D = 256, H = 4 and 1 <= T <= 256 (cudaErrorInvalidValue otherwise). Bit-identical to the QKV GEMM + rel_attention.
+struct QkvAttnParams {
+  int B, H, T, D;
+  int pos_row0;  // positional row of key 0
+  int pos_col0;  // first column (layer * D) of this layer's slice in the positional table
+  const float* bqkv;   // [3D]
+  const float* pos_u;  // [D] pos_bias_u
+  const float* pos_v;  // [D] pos_bias_v
+  const int* klens;    // per-utterance valid key count (nullable = all T valid)
+  __nv_bfloat16* out;  // [B*T, D]
+};
+cudaError_t launch_qkv_rel_attention(const CUtensorMap& tm_y, const CUtensorMap& tm_w, const CUtensorMap& tm_p,
+                                     const QkvAttnParams& p, cudaStream_t st);
+
 
 // Grouped rel-pos attention of the Efficient Conformer (grouped_attention.cu)
 struct GroupedAttnParams {

@@ -72,6 +72,7 @@ struct BlockW {
 };
 struct BlockMaps {  // their tensor maps (B operands)
   CUtensorMap wqkv, wo, pw1, pw2;
+  CUtensorMap wqkv_h;  // the same wqkv with a 64-row box: one head's q, k or v rows (qkv_rel_attention_kernel)
 };
 
 struct LayerW : BlockW {
@@ -448,6 +449,7 @@ int pack_attention(ppasr_b200_ctx* c, const std::string& p, int l, bool grouped,
   if (int rc = check_weights(c)) return rc;
   std::string err;
   if (!make_tmap_2d(&m.wqkv, w.wqkv, D, 3 * D, (uint64_t)D * 2, BN_NARROW, &err) ||
+      !make_tmap_2d(&m.wqkv_h, w.wqkv, D, 3 * D, (uint64_t)D * 2, 64, &err) ||
       !make_tmap_2d(&m.wo, w.wo, D, D, (uint64_t)D * 2, BN_WIDE, &err)) {
     set_last_error(err);
     return PPASR_ERR_CUDA;
@@ -885,6 +887,10 @@ int build_plan(ppasr_b200_ctx* c, int B, int T) {
   return PPASR_OK;
 }
 
+// Offline plain attention: the QKV projection runs inside the attention kernel (qkv_rel_attention_kernel) when every
+// utterance fits two 128-frame tiles; longer ones take the QKV GEMM + rel_attention_kernel pair.
+bool fused_qkv_attention(int D, int H, int T) { return D == 256 && H == 4 && T >= 1 && T <= 256; }
+
 template <int BN, int ST, class Epi>
 cudaError_t gemm(ppasr_b200_ctx* c, const CUtensorMap& a, const CUtensorMap& b, int M, int N, int K, const Epi& epi,
                  cudaStream_t st) {
@@ -1009,7 +1015,10 @@ int run_encoder(ppasr_b200_ctx* c, cudaStream_t st, bool chunk) {
     } else {
       AttnParams ap{};
       ap.B = B, ap.H = H, ap.T1 = Tc, ap.D = D, ap.pos_col0 = l * D, ap.out = p.att, ap.q_rows_per_bh = Tc;
-      if (!chunk) {
+      if (!chunk && fused_qkv_attention(D, H, Tc)) {
+        QkvAttnParams qp{B, H, Tc, D, 0, l * D, w.bqkv, w.pos_u, w.pos_v, vl, p.att};
+        { PROF(PC_ATTENTION); PPASR_CUDA_CHECK(launch_qkv_rel_attention(p.tm_y, m.wqkv_h, *tmpos, qp, st)); }
+      } else if (!chunk) {
         EpiQKV<BN_NARROW> e{p.q2, p.kk, p.vt, w.bqkv, w.pos_u, w.pos_v, Mc, Tc, H, Tc, p.Tkp, 0};
         { PROF(PC_QKV); PPASR_CUDA_CHECK((gemm<BN_NARROW, ST_NARROW>(c, p.tm_y, m.wqkv, Mc, 3 * D, D, e, st))); }
         ap.T2 = Tc, ap.k_rows_per_bh = Tc, ap.k_row0 = 0, ap.pos_row0 = 0, ap.klens = vl;
@@ -1691,6 +1700,62 @@ int ppasr_b200_op_attention(const void* q2, const void* kk, const void* vt, int3
   ap.pos_row0 = pos_row0, ap.pos_col0 = pos_col0, ap.D = H * 64, ap.klens = klens, ap.out = (__nv_bfloat16*)out;
   PPASR_CUDA_CHECK(launch_rel_attention(tq, tk, tp, tv, ap, reinterpret_cast<cudaStream_t>(stream)));
   return PPASR_OK;
+}
+
+int ppasr_b200_op_qkv_attention(const void* y, const void* wqkv, const float* bqkv, const float* pos_u, const float* pos_v,
+                                const void* pos, int32_t pos_rows, int32_t pos_ld, int32_t pos_row0, int32_t pos_col0,
+                                const int32_t* klens, int32_t B, int32_t T, void* out, int32_t fused, void* stream) {
+  PPASR_REQUIRE(y && wqkv && bqkv && pos_u && pos_v && pos && out, "null pointer");
+  PPASR_REQUIRE(B > 0 && T > 0 && pos_ld % 8 == 0, "bad shape (pos_ld must be a multiple of 8)");
+  const int D = 256, H = 4, M = B * T;
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  std::string err;
+  CUtensorMap ty, tp;
+  if (!make_tmap_2d(&ty, y, D, M, (uint64_t)D * 2, GEMM_BLOCK_M, &err) ||
+      !make_tmap_2d(&tp, pos, pos_ld, pos_rows, (uint64_t)pos_ld * 2, 128, &err)) {
+    set_last_error(err);
+    return PPASR_ERR_CUDA;
+  }
+  if (fused) {
+    CUtensorMap tw;
+    if (!make_tmap_2d(&tw, wqkv, D, 3 * D, (uint64_t)D * 2, 64, &err)) {
+      set_last_error(err);
+      return PPASR_ERR_CUDA;
+    }
+    QkvAttnParams qp{B, H, T, D, pos_row0, pos_col0, bqkv, pos_u, pos_v, klens, (__nv_bfloat16*)out};
+    PPASR_CUDA_CHECK(launch_qkv_rel_attention(ty, tw, tp, qp, st));
+    return PPASR_OK;
+  }
+  // the QKV GEMM + rel_attention_kernel pair on scratch q2 / kk / vt laid out as in the offline plan
+  const int Tkp = (T + 63) / 64 * 64;
+  __nv_bfloat16 *q2 = nullptr, *kk = nullptr, *vt = nullptr;
+  const size_t nq = (size_t)B * H * T * 128, nk = (size_t)B * H * T * 64, nv = (size_t)B * H * 64 * Tkp;
+  PPASR_CUDA_CHECK(cudaMallocAsync(&q2, (nq + nk + nv) * 2, st));
+  kk = q2 + nq, vt = kk + nk;
+  int rc = PPASR_OK;
+  CUtensorMap tw, tq, tk, tv;
+  if (!make_tmap_2d(&tw, wqkv, D, 3 * D, (uint64_t)D * 2, BN_NARROW, &err) ||
+      !make_tmap_2d(&tq, q2, 128, (uint64_t)B * H * T, 256, 128, &err) ||
+      !make_tmap_2d(&tk, kk, 64, (uint64_t)B * H * T, 128, 128, &err) ||
+      !make_tmap_2d(&tv, vt, T, (uint64_t)B * H * 64, (uint64_t)Tkp * 2, 64, &err)) {
+    set_last_error(err);
+    rc = PPASR_ERR_CUDA;
+  } else {
+    cudaError_t e = cudaMemsetAsync(vt, 0, nv * 2, st);
+    EpiQKV<BN_NARROW> epi{q2, kk, vt, bqkv, pos_u, pos_v, M, T, H, T, Tkp, 0};
+    if (e == cudaSuccess)
+      e = launch_gemm<BN_NARROW, ST_NARROW, false>(ty, tw, make_shape(M, 3 * D, D, BN_NARROW), epi, device_sm_count(), st);
+    AttnParams ap{};
+    ap.B = B, ap.H = H, ap.T1 = T, ap.T2 = T, ap.q_rows_per_bh = T, ap.k_rows_per_bh = T, ap.k_row0 = 0;
+    ap.pos_row0 = pos_row0, ap.pos_col0 = pos_col0, ap.D = D, ap.klens = klens, ap.out = (__nv_bfloat16*)out;
+    if (e == cudaSuccess) e = launch_rel_attention(tq, tk, tp, tv, ap, st);
+    if (e != cudaSuccess) {
+      set_last_error(std::string("CUDA error: ") + cudaGetErrorString(e));
+      rc = PPASR_ERR_CUDA;
+    }
+  }
+  cudaFreeAsync(q2, st);
+  return rc;
 }
 
 int ppasr_b200_op_grouped_attention(const void* q2g, const void* kk, int32_t k_pitch, const void* vt, int32_t vt_pitch,
